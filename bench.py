@@ -1,6 +1,6 @@
 """bench.py -- the driver's measurement contract for the TF-recomm hot path (matrix-factorization train step).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: batch assembly -> forward + d cost/d logits -> id dedup
 (radix sort + ordered segment sums) -> TF-semantics sparse Adam over the WHOLE tables.  README model (squared
@@ -22,6 +22,12 @@ timed region.  `roofline` = the dominant kernel (adam_stream_multi_kernel, the w
 CUDA events around its launches.  `cpu_baseline` / `--impl reference` = the CPU restatement of the TF path
 (oracle/tfr_oracle.c, OpenMP over all host cores) on a bounded sample -- the reference's own code cannot run here
 (TensorFlow absent, ops.py does not import; DESIGN.md).
+
+--steps K sets the timed steps of `value` and of `e2e`.  `e2e`'s timed region includes the fill of its feed pipeline (the
+first three batches are handed over inside it), a share of the time that grows as K shrinks: compare e2e numbers taken
+at the same K.  --dump-outputs DIR writes what the last timed step of `value`
+computed as DIR/<name>.npy (float32, about 5 MB): see last_step_outputs.  Columns, initial tables and index stream are
+all seeded, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import ctypes as C
@@ -166,10 +172,37 @@ def time_stream_steps(eng, steps, torch):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     torch.cuda.synchronize()
     ev0.record()
-    eng.run_stream_steps(steps, use_graph=True)
+    bufs = eng.run_stream_steps(steps, use_graph=True)
     ev1.record()
     torch.cuda.synchronize()
-    return ev0.elapsed_time(ev1) / 1e3
+    return ev0.elapsed_time(ev1) / 1e3, bufs
+
+
+DUMP_ROWS = 4096
+
+
+def dump_rows(n):
+    """The table rows --dump-outputs writes of a table of n rows: a fixed sample, ascending."""
+    return np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_ROWS), replace=False))
+
+
+def last_step_outputs(eng, bufs, torch):
+    """What the last timed step computed, as host arrays: the predictions run_stream_steps hands back (logits, infer:
+    from the PRE-update tables) and the tables that step left behind, which alone show its update -- of users and items
+    the rows dump_rows picks, since the ML-25M tables alone are 116 MB."""
+    out = {k: bufs[k].cpu().numpy() for k in ("logits", "infer")}
+    out["mu"] = eng.t["mu"].cpu().numpy()
+    for side, n in (("user", eng.U), ("item", eng.I)):
+        idx = torch.from_numpy(dump_rows(n)).to(eng.device)
+        for tab in (side + "_bias", side + "_feat"):
+            out[tab] = eng.t[tab][idx].cpu().numpy()
+    return out
+
+
+def write_outputs(outputs, out_dir):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 def _adam_tables(eng, ws, _lib):
@@ -244,7 +277,7 @@ def _n_partials(d, B):
     return max(1, min(1024, (B + rows_per_cta - 1) // rows_per_cta))
 
 
-def run_workload(name, args, torch, with_e2e=True, with_roofline=True, sample_clocks=True):
+def run_workload(name, args, torch, with_e2e=True, with_roofline=True, sample_clocks=True, dump=False):
     from tf_recomm_b200.engine import SvdEngine
     w = WORKLOADS[name]
     B = w["B"]
@@ -263,7 +296,9 @@ def run_workload(name, args, torch, with_e2e=True, with_roofline=True, sample_cl
     if sampler:
         sampler.start()
         time.sleep(0.3)
-    secs = time_stream_steps(eng, args.steps, torch)
+    secs, last = time_stream_steps(eng, args.steps, torch)
+    # taken before anything below steps the engine again (the clock sampler's run-on lasts a wall-clock time)
+    outputs = last_step_outputs(eng, last, torch) if dump else None
     if sampler and secs < 1.0:
         # keep the same work running long enough for the 100 ms clock sampler to see it under load
         eng.set_batch_cursor(0)
@@ -278,19 +313,20 @@ def run_workload(name, args, torch, with_e2e=True, with_roofline=True, sample_cl
     bytes_step = algorithmic_bytes_step(w["U"], w["I"], w["d"], B)
     peak, peak_src = measured_peaks()
     res = dict(value=value, ms_per_step=ms_step, bytes_step=bytes_step, hbm_gbs_step=bytes_step / (ms_step / 1e3) / 1e9,
-               peak=peak, peak_src=peak_src, clocks=clocks, w=w, steps_per_epoch=n_train // B)
+               peak=peak, peak_src=peak_src, clocks=clocks, w=w, steps_per_epoch=n_train // B, outputs=outputs)
     if with_e2e:
+        AHEAD, WARM = 3, 15
         rng = np.random.default_rng(3)
-        batches = []
-        for _ in range(min(max(args.steps, 100), 200) + 15):   # (>= 100 timed steps: the pipeline's fill is part of the number)
+        drawn = []
+        for _ in range(WARM + min(args.steps, 200)):   # at most 200 distinct timed batches (1.5 MB of host columns each)
             rows = rng.integers(0, n_train, B)
-            batches.append((cols[0][rows].astype(np.float64), cols[1][rows].astype(np.float64),
-                            cols[2][rows].astype(np.float64)))   # float64 columns: what ShuffleIterator yields
+            drawn.append((cols[0][rows].astype(np.float64), cols[1][rows].astype(np.float64),
+                          cols[2][rows].astype(np.float64)))   # float64 columns: what ShuffleIterator yields
+        timed = [drawn[WARM + j % (len(drawn) - WARM)] for j in range(args.steps)]
         # the driver's loop (svd_train_val.py): batches t+1 .. t+3 have been handed over when step t is asked for and
         # returns its predictions (host) -- the later ones are being packed by the feed worker thread while t+1 is fetched
         # and its ids sorted under step t's table pass.  Every step's H2D (12 B / rating) and D2H (4 or 8 B / rating) are inside
-        # the timed region.
-        AHEAD, WARM = 3, 15
+        # the timed region, and so is the pipeline's fill: at small --steps it weighs on the number.
 
         def feed_loop(bs):
             for j in range(min(AHEAD, len(bs))):
@@ -301,13 +337,13 @@ def run_workload(name, args, torch, with_e2e=True, with_roofline=True, sample_cl
                 eng.train_step_host(*bs[j])
         # every step graph captured up front, then a warm-up in the same pattern (staging sets, pinned buffers, worker)
         eng.prepare_feed_graphs(B)
-        feed_loop(batches[:WARM])
+        feed_loop(drawn[:WARM])
         torch.cuda.synchronize()
         t0 = time.perf_counter()   # (the priming hand-overs are inside: every timed step's H2D is counted)
-        feed_loop(batches[WARM:])
+        feed_loop(timed)
         torch.cuda.synchronize()
         dt = time.perf_counter() - t0
-        n = len(batches) - WARM
+        n = len(timed)
         res["e2e"] = {"value": B * n / dt, "unit": "ratings/s", "h2d_bytes_per_step": eng.h2d_bytes(B),
                       "d2h_bytes_per_step": eng.d2h_bytes(B), "ms_per_step": dt / n * 1e3, "steps": n,
                       "path": "SvdEngine.train_step_host + prefetch_host three batches ahead (what Session.run([train_op, logits, "
@@ -339,19 +375,24 @@ def emit(line):
 
 def main():
     global JSON_OUT
+    sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree (which may be read-only), bytecode included
     JSON_OUT = _claim_stdout()
     sys.modules.setdefault("bench", sys.modules[__name__])  # bench_sharded / tools `import bench`: this very module
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=None)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps of value and e2e (default 200)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", type=str, default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", type=str, default=None)
     ap.add_argument("--no-also", action="store_true", help="skip the secondary ML-1M measurement")
     ap.add_argument("--cpu-steps", type=int, default=None, help="steps of the bounded CPU baseline sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (one GPU, --impl ours)")
     args = ap.parse_args()
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
+    if args.dump_outputs and (args.gpus > 1 or world > 1 or args.impl != "ours"):
+        ap.error("--dump-outputs needs a one-GPU run of --impl ours")
     if args.gpus > 1 or world > 1:
         import bench_sharded as sharded_bench
         return sharded_bench.main(args)
@@ -371,7 +412,9 @@ def main():
     import tf_recomm_b200  # noqa: F401
     assert torch.cuda.is_available(), "bench.py needs a CUDA device; there is no CPU fallback (use --impl reference)"
     torch.cuda.set_device(0)
-    r = run_workload(name, args, torch)
+    r = run_workload(name, args, torch, dump=bool(args.dump_outputs))
+    if args.dump_outputs:
+        write_outputs(r["outputs"], args.dump_outputs)
     cores = os.cpu_count()
     cpu_steps = args.cpu_steps or (6 if w["d"] >= 64 else 60)
     tot, n = cpu_reference_run(w, cpu_steps, 2)

@@ -35,8 +35,8 @@ def test_driver_session_and_stream_modes_agree(tmp_path):
     graphs on device-resident columns with the SAME index stream (np.random.seed(13575) + ShuffleIterator draws):
     the reported train / val errors must coincide, and the RMSE must fall."""
     common = ["--synthetic", "ml1m", "--ratings", "60000", "--epochs", "4", "--batch", "1000", "--dim", "15"]
-    a = _errors(_run(common + ["--mode", "session", "--checkpoint", str(tmp_path / "a.ckpt")]))
-    b = _errors(_run(common + ["--mode", "stream", "--checkpoint", str(tmp_path / "b.ckpt")]))
+    a = _errors(_run(common + ["--mode", "session", "--checkpoint", str(tmp_path / "a.ckpt"), "--logdir", str(tmp_path / "la")]))
+    b = _errors(_run(common + ["--mode", "stream", "--checkpoint", str(tmp_path / "b.ckpt"), "--logdir", str(tmp_path / "lb")]))
     assert len(a) >= 4 and len(a) == len(b)
     for (ea, ta, va), (eb, tb, vb) in zip(a, b):
         assert ea == eb
@@ -75,11 +75,12 @@ def test_checkpoint_restore_continues_bit_identically(tmp_path):
         assert np.array_equal(ta[n], tb[n]), n
 
 
-def test_driver_fork_variant_reports_acc_auc_nll():
+def test_driver_fork_variant_reports_acc_auc_nll(tmp_path):
     """The code as written (ops.py:44,85-89,125,145: |q| in the dot, sigmoid cross-entropy, bias L2, SGD) through the
     reference's DISCRETE branch: accuracy / AUC / mean NLL per epoch (svd_train_val.py:94-98,138-143,156)."""
     text = _run(["--synthetic", "ml1m", "--ratings", "40000", "--epochs", "3", "--batch", "500", "--dim", "20",
-                 "--variant", "fork", "--lr", "0.005", "--reg", "0.01", "--checkpoint", os.devnull])
+                 "--variant", "fork", "--lr", "0.005", "--reg", "0.01", "--checkpoint", os.devnull,
+                 "--logdir", str(tmp_path / "log")])
     rows = re.findall(r"^\s*(\d+) TRAIN\(size=\d+/\d+, macc=([0-9.]+), mauc=([0-9.]+), mnll=([0-9.]+)\) "
                       r"TEST\(size=\d+, macc=([0-9.]+), auc=([0-9.]+), mnll=([0-9.]+)\)", text, flags=re.M)
     assert len(rows) >= 3, text[-400:]
@@ -106,7 +107,7 @@ def test_driver_reads_the_reference_csv_layout(tmp_path, monkeypatch):
         yaml.safe_dump(dict(USER_NUM=U, ITEM_NUM=I, NB_CLASSES=5, BATCH_SIZE=100), f)
     monkeypatch.chdir(tmp_path)
     rows = _errors(_run(["--dataset", "tiny", "--epochs", "5", "--batch", "100", "--dim", "8", "--lr", "0.01",
-                         "--checkpoint", str(tmp_path / "fm.ckpt")]))
+                         "--checkpoint", str(tmp_path / "fm.ckpt"), "--logdir", str(tmp_path / "log")]))
     assert len(rows) >= 5 and rows[-1][2] < rows[0][2]
     z = np.load(str(tmp_path / "fm.ckpt"))
     assert z["user_feat"].shape == (U, 8) and z["item_feat"].shape == (I, 8)
