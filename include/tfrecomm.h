@@ -394,6 +394,19 @@ int tfr_allpairs_consume(const float* user_feat, const float* item_feat, const f
                          int64_t item_stride, int32_t k, int32_t n_cand, double* topk_val, int32_t* topk_idx,
                          int32_t* n_uncertified, const int64_t* obs_indptr, const int32_t* obs_item, const float* obs_rate,
                          double* row_se, void* workspace, int64_t workspace_bytes, void* stream);
+/* The same top-k ranking over the items each user has NOT already rated: excl_indptr int64 [n_users + 1] / excl_item int32
+ * list, per user, the item ids that must never be returned (ascending inside a user, duplicates allowed; excl_indptr = null:
+ * nothing excluded, the result of tfr_allpairs_consume).  The tensor-core sweep skips them when it keeps candidates and the
+ * certificate is over the rankable items: a user ranks min(k, rankable_u) items, rankable_u = n_items - (distinct excluded
+ * ids of u), the ranks past that are (-inf, -1) (a user with every item excluded: all (-inf, -1), certified).  Any dim <=
+ * 512: a dim the tcgen05 sweep cannot take (dim % 32 != 0 or dim > 128) sends EVERY row through the exact float64 path
+ * (*n_uncertified = n_users), O(n_users * n_items * (dim + k)) on CUDA cores -- meant for ML-1M-sized tables.
+ * workspace: tfr_allpairs_topk_workspace_bytes. */
+int tfr_allpairs_rank_excluding(const float* user_feat, const float* item_feat, const float* user_bias,
+                                const float* item_bias, const float* mu, int64_t n_users, int64_t n_items, int32_t dim,
+                                int64_t user_stride, int64_t item_stride, int32_t k, int32_t n_cand,
+                                const int64_t* excl_indptr, const int32_t* excl_item, double* topk_val, int32_t* topk_idx,
+                                int32_t* n_uncertified, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ---- host side of the feed_dict boundary: the columns a reference iterator yields (dataio.py:114-117: float64 views
  * of one [B, ncols] matrix, ids included) packed into a pinned staging buffer in the device's types -- int32 ids
@@ -487,6 +500,18 @@ int tfr_host_wait_flag(const void* flag_host, uint32_t at_least, int64_t timeout
 int64_t tfr_binary_metrics_workspace_bytes(int64_t n);
 int tfr_binary_metrics(const float* logits, const float* labels, int64_t n, void* workspace, int64_t workspace_bytes,
                        double* out4, void* stream);
+
+/* ---- top-k ranking metrics on the device --------------------------------------------------------------------------------
+ * topk_idx [n_rows, k]: any ranking (tfr_allpairs_rank_excluding, tfr_topk_rows; -1 = no item, never a hit); relevant set
+ * as CSR: rel_indptr int64 [n_rows + 1], rel_item int32 strictly ascending inside a row.  Per row u with R_u its relevant
+ * items and h_r = [topk_idx[u, r] in R_u]:  HR = [sum h_r >= 1], precision = sum h_r / k, recall = sum h_r / |R_u|,
+ * NDCG = sum_r h_r / log2(r + 2) over sum_{r < min(k, |R_u|)} 1 / log2(r + 2), in float64.  Rows with |R_u| = 0 are not
+ * evaluated.  sums (device, 5 doubles) = (sum HR, sum precision, sum recall, sum NDCG, rows evaluated); row_metrics
+ * (device, [n_rows, 4] = HR, precision, recall, NDCG; NaN for rows not evaluated) only when not null.  Fixed-order
+ * reduction, no floating-point atomics: the same bits every run. */
+int64_t tfr_ranking_metrics_workspace_bytes(int64_t n_rows, int32_t k);
+int tfr_ranking_metrics(const int32_t* topk_idx, int64_t n_rows, int32_t k, const int64_t* rel_indptr, const int32_t* rel_item,
+                        double* row_metrics, double* sums, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ---- KTM design matrix on the device: replaces fm.py:61-93 df_to_sparse (scipy coo / hstack / tocsr on the host) ---------
  * One block per active agent, hstacked in the order given: agents_host[g] in 0..7 = users, items, skills, attempts, wins,

@@ -16,6 +16,10 @@ Two ways to run the step loop:
   --mode session   (default) the reference's loop verbatim: next(iter_train) -> sess.run(feed_dict) per step.
   --mode stream    the same batches, but the training columns live in HBM and the whole epoch's index stream is
                    drawn up front (same RandomState consumption); each step is one replay of a captured CUDA graph.
+
+--topk K adds, after every report, the top-K recommendation quality on the validation split: each user is ranked over
+the items they did not rate in training, and hit rate / precision / recall / NDCG at K are measured against their
+validation items (rated >= --topk-min-rating; on the DISCRETE branch, an outcome of 1).
 """
 import argparse
 import os
@@ -77,6 +81,11 @@ def svd(train, test, args, log=print):
         if args.mode == "stream":
             engine.set_train_data(train["user"], train["item"], train["outcome"])
             engine.set_se_ring(nb_batches)
+        topk = int(getattr(args, "topk", 0) or 0)
+        if topk:
+            # the training pairs are never recommended: their CSR is built once, not per report
+            topk_exclude = engine.pair_csr(train["user"], train["item"])
+            topk_min_rating = 1.0 if discrete else float(args.topk_min_rating)
         start = time.time()
         total_steps = args.epochs * nb_batches
         i = 0
@@ -174,6 +183,14 @@ def svd(train, test, args, log=print):
                 rec = dict(epoch=epoch, train_rmse=train_rmse, test_rmse=test_rmse, elapsed=end - start)
                 log("{:3d} TRAIN(size={:d}/{:d}, rmse={:f}) TEST(size={:d}, rmse={:f}) {:f}(s)".format(
                     epoch, last_batch, len(train["user"]), train_rmse, len(test["user"]), test_rmse, end - start))
+            if topk:
+                t_topk = time.time()
+                rm = engine.ranking_metrics(topk, test["user"], test["item"], rates=test["outcome"],
+                                            min_rating=topk_min_rating, exclude=topk_exclude)
+                rec["topk"] = rm
+                log("TOPK(k={:d}, users={:d}, hr={:f}, precision={:f}, recall={:f}, ndcg={:f})".format(
+                    topk, rm["n_users"], rm["hr"], rm["precision"], rm["recall"], rm["ndcg"]))
+                end += time.time() - t_topk   # the next report's elapsed time is the training's alone
             history.append(rec)
             if writer is not None:
                 # svd_train_val.py:189-192: train_rmse / test_rmse under these two tags (NaN on the DISCRETE branch, where
@@ -183,6 +200,10 @@ def svd(train, test, args, log=print):
                 if discrete:
                     for tag in ("train_macc", "train_mauc", "train_mnll", "test_macc", "test_auc", "test_mnll"):
                         writer.add_summary(summary.make_scalar_summary(tag, rec[tag]), report_at)
+                if topk:
+                    for tag, key in (("hr_at_k", "hr"), ("precision_at_k", "precision"), ("recall_at_k", "recall"),
+                                     ("ndcg_at_k", "ndcg")):
+                        writer.add_summary(summary.make_scalar_summary(tag, rec["topk"][key]), report_at)
                 writer.flush()
             start = end
         if writer is not None:
@@ -240,6 +261,11 @@ def main(argv=None):
                     help="TensorBoard event files (svd_train_val.py:57); empty string = none")
     ap.add_argument("--host-metrics", dest="host_metrics", action="store_true",
                     help="DISCRETE branch: ACC / AUC / NLL with the reference's host code instead of on the device")
+    ap.add_argument("--topk", type=int, default=0,
+                    help="after every report, hit rate / precision / recall / NDCG at this k on the validation split, "
+                         "training items excluded from the ranking (0 = off)")
+    ap.add_argument("--topk-min-rating", dest="topk_min_rating", type=float, default=4.0,
+                    help="README variant: the validation ratings that count as relevant for --topk")
     args = ap.parse_args(argv)
     np.random.seed(config.SEED)  # svd_train_val.py:15
     train, val = load(args)

@@ -13,6 +13,11 @@
 // never exists.
 //
 // CUDA-core path (any dim): exact fp32, same outputs; also the reference for the tf32 tolerance in the tests.
+//
+// Ranking of UNSEEN items (tfr_allpairs_rank_excluding): the top-k consumer skips each user's excluded items (CSR walk in
+// the epilogue, like the observed-pairs walk) and the certificate counts only rankable items.  For a dim the tcgen05
+// sweep cannot take (dim % 32 != 0 or dim > 128, up to 512) there is no sweep: every row goes through the exact float64
+// fallback, O(n_users * n_items * (dim + k)) -- fine at the ML-1M shape, not a path for ML-25M.
 #include <cuda.h>
 #include <string.h>
 
@@ -120,6 +125,9 @@ __device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, float* v) {
 //   * OBS: the squared error on the OBSERVED pairs, als3.py:110-120,139-143 (predict = M[user_ids, work_ids], then
 //     compute_rmse): the pairs come as CSR by user with ascending item ids; every row's thread walks its list as the
 //     tiles go by and accumulates (score - rating)^2 in float64.
+//   * EXCL (with TOPK, without OBS): items the user must not be recommended (the ones already rated), CSR by user with
+//     ascending item ids, duplicates allowed; the row's lane walks its list like the OBS walk and a column equal to the
+//     next excluded id is never appended to the candidate buffer.  Everything else of TOPK is unchanged.
 constexpr int AP_THREADS = 320, AP_EPI_WARPS = 8;
 enum { BAR_A = 0, BAR_FULL_B = 1, BAR_EMPTY_B = 3, BAR_TMEM_FULL = 5, BAR_TMEM_EMPTY = 7, AP_NBARS = 9 };
 constexpr int AP_MAX_CAND = 128;
@@ -137,6 +145,8 @@ struct ApConsumers {
   const int32_t* obs_item;   // OBS: [nnz] ascending inside a user's range
   const float* obs_rate;     // OBS: [nnz]
   double* row_se;            // OBS: [n_users] sum over the user's observed pairs of (score - rating)^2
+  const int64_t* excl_indptr; // EXCL: [n_users + 1]
+  const int32_t* excl_item;   // EXCL: [nnz] ascending inside a user's range
 };
 
 // order of the ranking: higher score first, lower item index on ties
@@ -235,7 +245,7 @@ __device__ __noinline__ ApListState ap_compact_warp(float* __restrict__ cval, in
   return out;
 }
 
-template <int KCHUNKS, bool TOPK, bool OBS>
+template <int KCHUNKS, bool TOPK, bool OBS, bool EXCL>
 __global__ void __launch_bounds__(AP_THREADS, 1)
     allpairs_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                        const float* __restrict__ ub, const float* __restrict__ ib, const float* __restrict__ mu,
@@ -342,6 +352,20 @@ __global__ void __launch_bounds__(AP_THREADS, 1)
     int onext = 0x7fffffff, onext2 = 0x7fffffff;   // the next pair's item id, and the one after it (fetched ahead: a
     float orate = 0.0f, orate2 = 0.0f;             // hit then never waits for a load it has just issued)
     double se = 0.0;
+    // EXCL: this row's excluded items [xp, xend), the next one's id and the one after it (fetched ahead, as for OBS)
+    int64_t xp = 0, xend = 0;
+    int xnext = 0x7fffffff, xnext2 = 0x7fffffff;
+    if (EXCL && row_ok) {
+      xp = cs.excl_indptr[row];
+      xend = cs.excl_indptr[row + 1];
+      if (xp < xend) xnext = cs.excl_item[xp];
+      if (xp + 1 < xend) xnext2 = cs.excl_item[xp + 1];
+    }
+    auto excl_advance = [&]() {
+      ++xp;
+      xnext = xnext2;
+      xnext2 = xp + 1 < xend ? cs.excl_item[xp + 1] : 0x7fffffff;
+    };
     if (OBS && row_ok) {
       op = cs.obs_indptr[row];
       oend = cs.obs_indptr[row + 1];
@@ -371,6 +395,9 @@ __global__ void __launch_bounds__(AP_THREADS, 1)
       if (OBS) {
         while (onext < n0) obs_advance();  // pairs of the columns the other half owns, or of earlier tiles
       }
+      if (EXCL) {
+        while (xnext < n0) excl_advance();
+      }
       mbar_wait(&bars[BAR_TMEM_FULL + acc], (t >> 1) & 1);
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 #pragma unroll
@@ -390,9 +417,16 @@ __global__ void __launch_bounds__(AP_THREADS, 1)
             const bool ok = row_ok && col < n_items;
             if (scores && ok) scores[(size_t)row * n_items + col] = s;
             if (ok && s > best[q]) { best[q] = s; besti[q] = col; }
+            bool excluded = false;
+            if (EXCL) {
+              if (col == xnext) {
+                excluded = true;
+                do excl_advance(); while (xnext == col);   // duplicates of an id
+              }
+            }
             if (TOPK) {
               // hot path: the row's own lane appends (two stores); compaction is checked once per 32-column chunk
-              if (ok && s > thr) {
+              if (ok && s > thr && !excluded) {
                 __stcg(my_val + lcnt, s);
                 __stcg(my_idx + lcnt, col);
                 ++lcnt;
@@ -472,13 +506,18 @@ __global__ void __launch_bounds__(AP_THREADS, 1)
 // descending, lowest item index on ties); they are the exact top-k of the WHOLE row if the k-th exact score is > T + E_u.
 // Rows for which that cannot be shown (near-ties deeper than the spare candidates) are appended to `uncert` and redone
 // exactly over all items by allpairs_exact_rows_kernel.  One warp per row.
+// With an exclusion list (EXCL sweep) the argument is the same over the row's RANKABLE items: an excluded item is never a
+// candidate, and every other item that is not one scored at most T.  The row ranks min(k, rankable_u) items, rankable_u =
+// n_items - (distinct excluded ids of u); the ranks past that are (-inf, -1), and a row whose items are all excluded is
+// all (-inf, -1) and certified.
 constexpr int RS_WARPS = 2;
 __global__ void __launch_bounds__(32 * RS_WARPS) allpairs_rescore_kernel(
     const float* __restrict__ U, const float* __restrict__ V, const float* __restrict__ ub, const float* __restrict__ ib,
     const float* __restrict__ mu, int n_users, int n_items, int dim, int64_t us, int64_t is,
     const float* __restrict__ cand_val, const int32_t* __restrict__ cand_idx, const int32_t* __restrict__ cand_cnt,
     const float* __restrict__ cand_thr, int K, int k, const float* __restrict__ vmax2, double* __restrict__ out_val,
-    int32_t* __restrict__ out_idx, int32_t* __restrict__ uncert, int32_t* __restrict__ n_uncert) {
+    int32_t* __restrict__ out_idx, int32_t* __restrict__ uncert, int32_t* __restrict__ n_uncert,
+    const int64_t* __restrict__ excl_indptr, const int32_t* __restrict__ excl_item) {
   __shared__ double s_sc[RS_WARPS][8 * AP_MAX_CAND];
   __shared__ int s_ix[RS_WARPS][8 * AP_MAX_CAND];
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -551,8 +590,15 @@ __global__ void __launch_bounds__(32 * RS_WARPS) allpairs_rescore_kernel(
     }
     last_v = bv; last_i = bi; kth = bv; ++got;
   }
+  int rankable = n_items;
+  if (excl_indptr && got < k) {   // (warp-uniform) only a short row needs its number of rankable items
+    const int64_t x0 = excl_indptr[row], x1 = excl_indptr[row + 1];
+    int distinct = 0;
+    for (int64_t p = x0 + lane; p < x1; p += 32) distinct += (p == x0 || excl_item[p] != excl_item[p - 1]) ? 1 : 0;
+    rankable -= warp_sum_i(distinct);
+  }
   if (lane == 0) {
-    const int kk = k < n_items ? k : n_items;
+    const int kk = k < rankable ? k : rankable;
     bool certified = T == -INFINITY;   // nothing was ever dropped: every rankable item is a candidate
     if (!certified && got >= kk) {
       const double E = 0.001953125 * sqrt(un2) * sqrt((double)vmax2[0]);   // 2^-9 * ||u|| * max ||v||
@@ -578,13 +624,17 @@ __global__ void allpairs_vmax2_kernel(const float* __restrict__ V, int n_items, 
 
 // The uncertified rows, redone exactly over ALL items: a persistent CTA per row computes the row's float64 scores into
 // its scratch line, then picks the k best by k rounds of a block-wide arg-max (the total order of ap_better).
+// Excluded items (excl_indptr != null) are marked NaN in the line, which the arg-max never picks: they are skipped, and
+// the ranks past the row's rankable items are (-inf, -1).
 __global__ void __launch_bounds__(1024) allpairs_exact_rows_kernel(const float* __restrict__ U, const float* __restrict__ V,
                                                                   const float* __restrict__ ub, const float* __restrict__ ib,
                                                                   const float* __restrict__ mu, int n_items, int dim,
                                                                   int64_t us, int64_t is, const int32_t* __restrict__ uncert,
                                                                   const int32_t* __restrict__ n_uncert, int k,
                                                                   double* __restrict__ scratch, double* __restrict__ out_val,
-                                                                  int32_t* __restrict__ out_idx) {
+                                                                  int32_t* __restrict__ out_idx,
+                                                                  const int64_t* __restrict__ excl_indptr,
+                                                                  const int32_t* __restrict__ excl_item) {
   __shared__ float s_u[512];
   __shared__ double s_v[32];
   __shared__ int s_i[32];
@@ -605,6 +655,10 @@ __global__ void __launch_bounds__(1024) allpairs_exact_rows_kernel(const float* 
       line[it] = ((acc + bu) + (double)ib[it]) + m;
     }
     __syncthreads();
+    if (excl_indptr) {
+      for (int64_t p = excl_indptr[row] + threadIdx.x; p < excl_indptr[row + 1]; p += blockDim.x) line[excl_item[p]] = nan("");
+      __syncthreads();
+    }
     double last_v = INFINITY;
     int last_i = -1;
     for (int r = 0; r < k; ++r) {
@@ -651,6 +705,12 @@ __global__ void __launch_bounds__(1024) allpairs_exact_rows_kernel(const float* 
       }
     }
   }
+}
+
+// every row to the exact path (dims the tcgen05 sweep cannot take): uncert = 0 .. n_users - 1, *n_uncert = n_users
+__global__ void allpairs_all_rows_kernel(int n_users, int32_t* __restrict__ uncert, int32_t* __restrict__ n_uncert) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n_users; i += gridDim.x * blockDim.x) uncert[i] = i;
+  if (blockIdx.x == 0 && threadIdx.x == 0) *n_uncert = n_users;
 }
 
 // ---- CUDA-core path: exact fp32, any dim --------------------------------------------------------------------
@@ -858,19 +918,21 @@ static int launch_allpairs_tc(const float* user_feat, const float* item_feat, co
   const int kch = dim / 32;
   const size_t smem = (size_t)3 * kch * AP_CHUNK_BYTES + 1024 + 128 + (2 * 256 + 512) * 4 + 256 * 8 + 64;
   const unsigned grid = (unsigned)((n_users + AP_BM - 1) / AP_BM);
-  const bool topk = cs.cand_val != nullptr, obs = cs.obs_indptr != nullptr;
-#define TFR_AP_LAUNCH(KC_, TK_, OB_)                                                                                   \
+  const bool topk = cs.cand_val != nullptr, obs = cs.obs_indptr != nullptr, excl = cs.excl_indptr != nullptr;
+  TFR_CHECK_ARG(!excl || (topk && !obs));   // the exclusion walk exists only in the top-k sweep
+#define TFR_AP_LAUNCH(KC_, TK_, OB_, EX_)                                                                              \
   {                                                                                                                    \
-    TFR_CUDA(cudaFuncSetAttribute(allpairs_tc_kernel<KC_, TK_, OB_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    allpairs_tc_kernel<KC_, TK_, OB_><<<grid, AP_THREADS, smem, st>>>(ma, mb, user_bias, item_bias, mu, (int)n_users,   \
-                                                                      (int)n_items, cs);                              \
+    TFR_CUDA(cudaFuncSetAttribute(allpairs_tc_kernel<KC_, TK_, OB_, EX_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    allpairs_tc_kernel<KC_, TK_, OB_, EX_><<<grid, AP_THREADS, smem, st>>>(ma, mb, user_bias, item_bias, mu, (int)n_users, \
+                                                                           (int)n_items, cs);                         \
   }
 #define TFR_AP_CASE(KC_)                                          \
   if (kch == KC_) {                                               \
-    if (topk && obs) TFR_AP_LAUNCH(KC_, true, true)               \
-    else if (topk) TFR_AP_LAUNCH(KC_, true, false)                \
-    else if (obs) TFR_AP_LAUNCH(KC_, false, true)                 \
-    else TFR_AP_LAUNCH(KC_, false, false)                         \
+    if (excl) TFR_AP_LAUNCH(KC_, true, false, true)               \
+    else if (topk && obs) TFR_AP_LAUNCH(KC_, true, true, false)   \
+    else if (topk) TFR_AP_LAUNCH(KC_, true, false, false)         \
+    else if (obs) TFR_AP_LAUNCH(KC_, false, true, false)          \
+    else TFR_AP_LAUNCH(KC_, false, false, false)                  \
   }
   TFR_AP_CASE(1) TFR_AP_CASE(2) TFR_AP_CASE(3) TFR_AP_CASE(4)
 #undef TFR_AP_CASE
@@ -888,13 +950,18 @@ extern "C" int64_t tfr_allpairs_topk_workspace_bytes(int64_t n_users, int64_t n_
 }
 
 // Per-user top-k ranking over ALL items (forward.py:47-61 for every user at once) and / or the squared error on the
-// observed pairs (als3.py:110-120,139-143), consumed in the epilogue of the tcgen05 GEMM.
-extern "C" int tfr_allpairs_consume(const float* user_feat, const float* item_feat, const float* user_bias,
-                                    const float* item_bias, const float* mu, int64_t n_users, int64_t n_items, int32_t dim,
-                                    int64_t user_stride, int64_t item_stride, int32_t k, int32_t n_cand, double* topk_val,
-                                    int32_t* topk_idx, int32_t* n_uncertified, const int64_t* obs_indptr,
-                                    const int32_t* obs_item, const float* obs_rate, double* row_se, void* workspace,
-                                    int64_t workspace_bytes, void* stream) {
+// observed pairs (als3.py:110-120,139-143), consumed in the epilogue of the tcgen05 GEMM.  One launcher for both entry
+// points: tfr_allpairs_consume (no exclusion, tcgen05 dims only) and tfr_allpairs_rank_excluding (top-k only, optional
+// exclusion list, any dim <= 512).  any_dim: a dim the tcgen05 sweep cannot take (dim % 32 != 0 or dim > 128) sends EVERY
+// row through allpairs_exact_rows_kernel, O(n_users * n_items * (dim + k)) on CUDA cores -- fine at the ML-1M shape, not
+// meant for ML-25M.
+static int allpairs_consume_impl(const float* user_feat, const float* item_feat, const float* user_bias,
+                                 const float* item_bias, const float* mu, int64_t n_users, int64_t n_items, int32_t dim,
+                                 int64_t user_stride, int64_t item_stride, int32_t k, int32_t n_cand, double* topk_val,
+                                 int32_t* topk_idx, int32_t* n_uncertified, const int64_t* obs_indptr,
+                                 const int32_t* obs_item, const float* obs_rate, double* row_se,
+                                 const int64_t* excl_indptr, const int32_t* excl_item, bool any_dim, void* workspace,
+                                 int64_t workspace_bytes, void* stream) {
   if (user_stride == 0) user_stride = dim;
   if (item_stride == 0) item_stride = dim;
   TFR_CHECK_ARG(user_stride >= dim && item_stride >= dim);
@@ -904,6 +971,7 @@ extern "C" int tfr_allpairs_consume(const float* user_feat, const float* item_fe
   TFR_CHECK_ARG(topk || obs);
   TFR_CHECK_ARG(!topk || (topk_val && topk_idx && n_uncertified && n_cand >= k && n_cand <= AP_MAX_CAND && dim <= 512));
   TFR_CHECK_ARG(!obs || (obs_item && obs_rate && row_se));
+  TFR_CHECK_ARG(!excl_indptr || (topk && !obs && excl_item));
   if (n_users == 0 || n_items == 0) return TFR_OK;
   TFR_CHECK_ARG(user_feat && item_feat && user_bias && item_bias && mu);
   cudaStream_t st = (cudaStream_t)stream;
@@ -923,13 +991,25 @@ extern "C" int tfr_allpairs_consume(const float* user_feat, const float* item_fe
     cs.cand_idx = reinterpret_cast<int32_t*>(w); w += align_up(8 * n_users * (int64_t)n_cand * 4, 256);
     cs.cand_cnt = reinterpret_cast<int32_t*>(w); w += align_up(2 * n_users * 4, 256);
     cs.cand_thr = reinterpret_cast<float*>(w); w += align_up(2 * n_users * 4, 256);
-    uncert = reinterpret_cast<int32_t*>(w); w += align_up(2 * n_users * 4, 256);
+    uncert = reinterpret_cast<int32_t*>(w); w += align_up(2 * n_users * 4, 256);   // >= n_users rows: all of them fit
     scratch = reinterpret_cast<double*>(w);
     cs.K = n_cand;
     TFR_CUDA(cudaMemsetAsync(vmax2, 0, 256, st));
     TFR_CUDA(cudaMemsetAsync(n_uncertified, 0, sizeof(int32_t), st));
   }
   if (obs) { cs.obs_indptr = obs_indptr; cs.obs_item = obs_item; cs.obs_rate = obs_rate; cs.row_se = row_se; }
+  cs.excl_indptr = excl_indptr; cs.excl_item = excl_item;
+  if (any_dim && (dim % 32 != 0 || dim > 128)) {   // (top-k only: checked above) every row through the exact path
+    allpairs_all_rows_kernel<<<(unsigned)((n_users + 255) / 256 < 1024 ? (n_users + 255) / 256 : 1024), 256, 0, st>>>(
+        (int)n_users, uncert, n_uncertified);
+    TFR_LAUNCH_CHECK();
+    allpairs_exact_rows_kernel<<<(unsigned)ap_exact_ctas(), 1024, 0, st>>>(user_feat, item_feat, user_bias, item_bias, mu,
+                                                                         (int)n_items, dim, user_stride, item_stride, uncert,
+                                                                         n_uncertified, k, scratch, topk_val, topk_idx,
+                                                                         excl_indptr, excl_item);
+    TFR_LAUNCH_CHECK();
+    return TFR_OK;
+  }
   const int stages = tune(TUNE_AP_STAGES);
   int rc = TFR_OK;
   if (!topk || (stages & 1))
@@ -941,15 +1021,40 @@ extern "C" int tfr_allpairs_consume(const float* user_feat, const float* item_fe
     TFR_LAUNCH_CHECK();
     allpairs_rescore_kernel<<<(unsigned)((n_users + RS_WARPS - 1) / RS_WARPS), 32 * RS_WARPS, 0, st>>>(
         user_feat, item_feat, user_bias, item_bias, mu, (int)n_users, (int)n_items, dim, user_stride, item_stride,
-        cs.cand_val, cs.cand_idx, cs.cand_cnt, cs.cand_thr, n_cand, k, vmax2, topk_val, topk_idx, uncert, n_uncertified);
+        cs.cand_val, cs.cand_idx, cs.cand_cnt, cs.cand_thr, n_cand, k, vmax2, topk_val, topk_idx, uncert, n_uncertified,
+        excl_indptr, excl_item);
     TFR_LAUNCH_CHECK();
     if (stages & 4)
     allpairs_exact_rows_kernel<<<(unsigned)ap_exact_ctas(), 1024, 0, st>>>(user_feat, item_feat, user_bias, item_bias, mu,
                                                                          (int)n_items, dim, user_stride, item_stride, uncert,
-                                                                         n_uncertified, k, scratch, topk_val, topk_idx);
+                                                                         n_uncertified, k, scratch, topk_val, topk_idx,
+                                                                         excl_indptr, excl_item);
     TFR_LAUNCH_CHECK();
   }
   return TFR_OK;
+}
+
+extern "C" int tfr_allpairs_consume(const float* user_feat, const float* item_feat, const float* user_bias,
+                                    const float* item_bias, const float* mu, int64_t n_users, int64_t n_items, int32_t dim,
+                                    int64_t user_stride, int64_t item_stride, int32_t k, int32_t n_cand, double* topk_val,
+                                    int32_t* topk_idx, int32_t* n_uncertified, const int64_t* obs_indptr,
+                                    const int32_t* obs_item, const float* obs_rate, double* row_se, void* workspace,
+                                    int64_t workspace_bytes, void* stream) {
+  return allpairs_consume_impl(user_feat, item_feat, user_bias, item_bias, mu, n_users, n_items, dim, user_stride,
+                               item_stride, k, n_cand, topk_val, topk_idx, n_uncertified, obs_indptr, obs_item, obs_rate,
+                               row_se, nullptr, nullptr, false, workspace, workspace_bytes, stream);
+}
+
+extern "C" int tfr_allpairs_rank_excluding(const float* user_feat, const float* item_feat, const float* user_bias,
+                                           const float* item_bias, const float* mu, int64_t n_users, int64_t n_items,
+                                           int32_t dim, int64_t user_stride, int64_t item_stride, int32_t k, int32_t n_cand,
+                                           const int64_t* excl_indptr, const int32_t* excl_item, double* topk_val,
+                                           int32_t* topk_idx, int32_t* n_uncertified, void* workspace,
+                                           int64_t workspace_bytes, void* stream) {
+  TFR_CHECK_ARG(k > 0);
+  return allpairs_consume_impl(user_feat, item_feat, user_bias, item_bias, mu, n_users, n_items, dim, user_stride,
+                               item_stride, k, n_cand, topk_val, topk_idx, n_uncertified, nullptr, nullptr, nullptr, nullptr,
+                               excl_indptr, excl_item, true, workspace, workspace_bytes, stream);
 }
 
 extern "C" int tfr_allpairs(const float* user_feat, const float* item_feat, const float* user_bias,

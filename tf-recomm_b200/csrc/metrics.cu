@@ -6,6 +6,7 @@
 //   * the KTM sparse design matrix of fm.py:61-93 (df_to_sparse: one block per active agent, hstacked) built as CSR
 //     directly in HBM: count -> scan -> fill.
 // Both need a prefix sum: a three-phase (block sums, scan of the sums, apply) exclusive scan, deterministic.
+//   * top-k ranking metrics (hit rate, precision, recall, NDCG at k) of a ranking against a held-out relevant set.
 #include <string.h>
 
 #include "common.cuh"
@@ -191,6 +192,87 @@ __global__ void __launch_bounds__(1024) metrics_finish_kernel(const int64_t* __r
   }
 }
 
+// ================================ ranking metrics at k ==================================================================
+// One warp per ranked row u (grid-stride over the rows), relevant set R_u as CSR (strictly ascending item ids); a ranked
+// id is a hit when a binary search finds it in R_u (-1 never does).  Per row, with h_r the hit flag of rank r:
+//   HR = [sum h_r >= 1], precision = sum h_r / k, recall = sum h_r / |R_u|,
+//   NDCG = (sum_r h_r / log2(r + 2)) / (sum_{r < min(k, |R_u|)} 1 / log2(r + 2))          (float64)
+// Rows with |R_u| = 0 are not evaluated.  Each block folds its warps' sums in warp order into part[block][5]; one block
+// folds the partials in a fixed order (ranking_metrics_finish_kernel): no floating-point atomics, the same bits every run.
+constexpr int RM_WARPS = 8, RM_MAX_BLOCKS = 1024;
+__global__ void __launch_bounds__(32 * RM_WARPS) ranking_metrics_rows_kernel(const int32_t* __restrict__ topk_idx, int64_t n_rows,
+                                                                            int k, const int64_t* __restrict__ rel_indptr,
+                                                                            const int32_t* __restrict__ rel_item,
+                                                                            double* __restrict__ row_metrics,
+                                                                            double* __restrict__ part) {
+  __shared__ double s_acc[RM_WARPS][5];
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  double acc[5] = {0.0, 0.0, 0.0, 0.0, 0.0};   // (HR, precision, recall, NDCG, evaluated rows): lane 0's copy counts
+  for (int64_t u = (int64_t)blockIdx.x * RM_WARPS + w; u < n_rows; u += (int64_t)gridDim.x * RM_WARPS) {
+    const int64_t r0 = rel_indptr[u], r1 = rel_indptr[u + 1];
+    const int64_t n_rel = r1 - r0;
+    if (n_rel == 0) {
+      if (row_metrics && lane < 4) row_metrics[u * 4 + lane] = nan("");   // not evaluated
+      continue;
+    }
+    int hits = 0;
+    double dcg = 0.0, idcg = 0.0;
+    for (int r = lane; r < k; r += 32) {
+      const int32_t it = topk_idx[u * k + r];
+      const double disc = 1.0 / log2((double)(r + 2));
+      if (r < n_rel) idcg += disc;
+      if (it < 0) continue;
+      int64_t lo = r0, hi = r1;   // first position with rel_item >= it
+      while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (rel_item[mid] < it) lo = mid + 1; else hi = mid;
+      }
+      if (lo < r1 && rel_item[lo] == it) { ++hits; dcg += disc; }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      hits += __shfl_xor_sync(0xffffffffu, hits, o);
+      dcg += __shfl_xor_sync(0xffffffffu, dcg, o);
+      idcg += __shfl_xor_sync(0xffffffffu, idcg, o);
+    }
+    const double hr = hits > 0 ? 1.0 : 0.0, prec = (double)hits / (double)k, rec = (double)hits / (double)n_rel,
+                 ndcg = dcg / idcg;
+    if (row_metrics && lane < 4) row_metrics[u * 4 + lane] = lane == 0 ? hr : lane == 1 ? prec : lane == 2 ? rec : ndcg;
+    acc[0] += hr; acc[1] += prec; acc[2] += rec; acc[3] += ndcg; acc[4] += 1.0;
+  }
+  if (lane == 0) {
+#pragma unroll
+    for (int j = 0; j < 5; ++j) s_acc[w][j] = acc[j];
+  }
+  __syncthreads();
+  if (threadIdx.x < 5) {
+    double t = 0.0;
+    for (int ww = 0; ww < RM_WARPS; ++ww) t += s_acc[ww][threadIdx.x];
+    part[blockIdx.x * 5 + threadIdx.x] = t;
+  }
+}
+
+__global__ void __launch_bounds__(256) ranking_metrics_finish_kernel(const double* __restrict__ part, int n_part,
+                                                                     double* __restrict__ sums) {
+  __shared__ double s_sum[5][256];
+  for (int j = 0; j < 5; ++j) {
+    double t = 0.0;
+    for (int b = threadIdx.x; b < n_part; b += 256) t += part[b * 5 + j];
+    s_sum[j][threadIdx.x] = t;
+  }
+  __syncthreads();
+  if (threadIdx.x < 5) {
+    double t = 0.0;
+    for (int i = 0; i < 256; ++i) t += s_sum[threadIdx.x][i];
+    sums[threadIdx.x] = t;
+  }
+}
+
+static int ranking_metrics_blocks(int64_t n_rows) {
+  const int64_t b = (n_rows + RM_WARPS - 1) / RM_WARPS;
+  return (int)(b < 1 ? 1 : (b < RM_MAX_BLOCKS ? b : RM_MAX_BLOCKS));
+}
+
 // ================================ KTM design matrix (fm.py:61-93) ==========================================================
 struct KtmArgs {
   const int32_t *user, *item;          // [n]
@@ -317,6 +399,34 @@ extern "C" int tfr_binary_metrics(const float* logits, const float* labels, int6
   metrics_runs_kernel<<<gb, 256, 0, st>>>(endf, end_ex, pos_ex, posf, n, run_pos, run_cnt);
   TFR_LAUNCH_CHECK();
   metrics_finish_kernel<<<1, 1024, 0, st>>>(run_pos, run_cnt, end_ex, n, part, n_part, out4);
+  TFR_LAUNCH_CHECK();
+  return TFR_OK;
+}
+
+extern "C" int64_t tfr_ranking_metrics_workspace_bytes(int64_t n_rows, int32_t k) {
+  if (n_rows < 0 || k <= 0) return TFR_ERR_INVALID;
+  return 256 + align_up((int64_t)ranking_metrics_blocks(n_rows) * 5 * 8, 256);
+}
+
+extern "C" int tfr_ranking_metrics(const int32_t* topk_idx, int64_t n_rows, int32_t k, const int64_t* rel_indptr,
+                                   const int32_t* rel_item, double* row_metrics, double* sums, void* workspace,
+                                   int64_t workspace_bytes, void* stream) {
+  TFR_CHECK_ARG(n_rows >= 0 && k > 0 && sums);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (n_rows == 0) {
+    TFR_CUDA(cudaMemsetAsync(sums, 0, 5 * sizeof(double), st));
+    return TFR_OK;
+  }
+  TFR_CHECK_ARG(topk_idx && rel_indptr && rel_item && workspace);
+  if (workspace_bytes < tfr_ranking_metrics_workspace_bytes(n_rows, k)) {
+    set_error("ranking-metrics workspace too small");
+    return TFR_ERR_WORKSPACE;
+  }
+  double* part = reinterpret_cast<double*>(align_up((int64_t)(uintptr_t)workspace, 256));
+  const int nb = ranking_metrics_blocks(n_rows);
+  ranking_metrics_rows_kernel<<<nb, 32 * RM_WARPS, 0, st>>>(topk_idx, n_rows, k, rel_indptr, rel_item, row_metrics, part);
+  TFR_LAUNCH_CHECK();
+  ranking_metrics_finish_kernel<<<1, 256, 0, st>>>(part, nb, sums);
   TFR_LAUNCH_CHECK();
   return TFR_OK;
 }

@@ -9,6 +9,7 @@ import contextlib
 import ctypes as C
 import os
 import time
+from typing import NamedTuple
 
 import numpy as np
 import torch
@@ -20,6 +21,12 @@ from ._lib import (ABS_ITEM, FORK_FLAGS, LOSS_SIGMOID_CE, OPT_SGD, README_FLAGS,
 TABLE_NAMES = ("mu", "user_bias", "item_bias", "user_feat", "item_feat")
 _SLOT_FIELDS = {"mu": ("m_mu", "v_mu"), "user_bias": ("m_ub", "v_ub"), "item_bias": ("m_ib", "v_ib"),
                 "user_feat": ("m_uf", "v_uf"), "item_feat": ("m_if", "v_if")}
+
+
+class PairCSR(NamedTuple):
+    """(user, item) pairs as CSR by user on the device: indptr int64 [U + 1], items int32 ascending inside a user."""
+    indptr: torch.Tensor
+    items: torch.Tensor
 
 
 def _require_cuda():
@@ -252,10 +259,7 @@ class SvdEngine:
         return self.binary_metrics(st["d_out"][:B], st["d_feed"][2 * B:].view(torch.float32))
 
     # ---- all-pairs consumers fused into the GEMM epilogue ------------------------------------------------------------
-    def rank_all_users(self, k=50, n_cand=None):
-        """forward.py:47-61 for EVERY user in one sweep of the tcgen05 GEMM: -> (items [U, k] int32, scores [U, k]
-        float64, n_uncertified).  Identical to ranking the float64 score matrix of als3.py:112 (score descending, lowest
-        item id on ties): tensor-core candidates, float64 rescore, certificate, exact fallback (tfr_allpairs_consume)."""
+    def _topk_setup(self, k, n_cand):
         k = int(min(k, self.I))
         if n_cand is None:
             n_cand = min(128, max(k + 14, 8))
@@ -265,25 +269,124 @@ class SvdEngine:
         n_unc = torch.zeros(1, dtype=torch.int32, device=dev)
         nbytes = check(self.L.tfr_allpairs_topk_workspace_bytes(self.U, self.I, k, n_cand))
         ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        with torch.cuda.device(dev):
-            check(self.L.tfr_allpairs_consume(self.t["user_feat"].data_ptr(), self.t["item_feat"].data_ptr(),
-                                              self.t["user_bias"].data_ptr(), self.t["item_bias"].data_ptr(),
-                                              self.t["mu"].data_ptr(), self.U, self.I, self.d, self.feat_stride,
-                                              self.feat_stride, k, n_cand, val.data_ptr(), idx.data_ptr(), n_unc.data_ptr(),
-                                              None, None, None, None, ws.data_ptr(), nbytes, self._stream()))
+        return k, n_cand, idx, val, n_unc, ws, nbytes
+
+    def rank_all_users(self, k=50, n_cand=None, exclude=None):
+        """forward.py:47-61 for EVERY user in one sweep of the tcgen05 GEMM: -> (items [U, k] int32, scores [U, k]
+        float64, n_uncertified).  Identical to ranking the float64 score matrix of als3.py:112 (score descending, lowest
+        item id on ties): tensor-core candidates, float64 rescore, certificate, exact fallback (tfr_allpairs_consume).
+
+        exclude: items each user must not be recommended (usually the training pairs): a (users, items) pair of id arrays
+        (host or device) or a PairCSR from pair_csr().  The ranking is then over each user's remaining items
+        (tfr_allpairs_rank_excluding); a user with fewer than k of them gets (-inf, -1) past the last one.  With exclude,
+        any dim <= 512 is accepted (dims the tensor cores cannot take rank every row exactly on CUDA cores), and an
+        engine whose model scores u.|v| (ABS_ITEM, the fork variant) is ranked by that score."""
+        if exclude is None:
+            k, n_cand, idx, val, n_unc, ws, nbytes = self._topk_setup(k, n_cand)
+            with torch.cuda.device(self.device):
+                check(self.L.tfr_allpairs_consume(self.t["user_feat"].data_ptr(), self.t["item_feat"].data_ptr(),
+                                                  self.t["user_bias"].data_ptr(), self.t["item_bias"].data_ptr(),
+                                                  self.t["mu"].data_ptr(), self.U, self.I, self.d, self.feat_stride,
+                                                  self.feat_stride, k, n_cand, val.data_ptr(), idx.data_ptr(),
+                                                  n_unc.data_ptr(), None, None, None, None, ws.data_ptr(), nbytes,
+                                                  self._stream()))
+            return idx, val, int(n_unc.item())
+        csr = exclude if isinstance(exclude, PairCSR) else self.pair_csr(*exclude)
+        return self._rank_excluding(k, n_cand, csr)
+
+    def _rank_excluding(self, k, n_cand, csr):
+        """tfr_allpairs_rank_excluding; csr = None: nothing excluded."""
+        k, n_cand, idx, val, n_unc, ws, nbytes = self._topk_setup(k, n_cand)
+        item_feat, item_stride = self.t["item_feat"], self.feat_stride
+        if self.flags & ABS_ITEM:   # the model's score is u.|v| (ops.py:44): rank on a copy of |item_feat|
+            item_feat, item_stride = torch.abs(item_feat).contiguous(), 0
+        with torch.cuda.device(self.device):
+            check(self.L.tfr_allpairs_rank_excluding(
+                self.t["user_feat"].data_ptr(), item_feat.data_ptr(), self.t["user_bias"].data_ptr(),
+                self.t["item_bias"].data_ptr(), self.t["mu"].data_ptr(), self.U, self.I, self.d, self.feat_stride,
+                item_stride, k, n_cand, csr.indptr.data_ptr() if csr is not None else None,
+                csr.items.data_ptr() if csr is not None else None, val.data_ptr(), idx.data_ptr(), n_unc.data_ptr(),
+                ws.data_ptr(), nbytes, self._stream()))
         return idx, val, int(n_unc.item())
+
+    def _csr_by_user(self, users, items, rates=None, dedup=False):
+        """(user, item[, rate]) pairs -> CSR by user, item ids ascending inside a user: (indptr int64 [U + 1], items int32,
+        rates float32 | None).  dedup: every distinct pair once (rates are then not carried); otherwise every pair as
+        given, duplicates included."""
+        self._check_ids(users, items)
+        dev = self.device
+        u, i = self._dev_i32(users).to(torch.int64), self._dev_i32(items).to(torch.int64)
+        rt = None
+        if dedup:
+            key = torch.unique(u * self.I + i)   # sorted
+            u, it = key // self.I, (key % self.I).to(torch.int32).contiguous()
+        else:
+            r = self._dev_f32(rates) if rates is not None else None
+            order = torch.argsort(u * self.I + i, stable=True)
+            it = i[order].to(torch.int32).contiguous()
+            rt = r[order].contiguous() if r is not None else None
+        indptr = torch.zeros(self.U + 1, dtype=torch.int64, device=dev)
+        indptr[1:] = torch.cumsum(torch.bincount(u, minlength=self.U), 0)
+        return indptr, it, rt
+
+    def pair_csr(self, users, items):
+        """The distinct (user, item) pairs as a PairCSR: build an exclusion set once, pass it to rank_all_users /
+        ranking_metrics as often as needed."""
+        indptr, it, _ = self._csr_by_user(users, items, dedup=True)
+        return PairCSR(indptr, it)
+
+    def ranking_metrics(self, k, users, items, rates=None, min_rating=None, exclude=None, n_cand=None):
+        """Top-k recommendation quality on held-out pairs: every user is ranked over the items not in `exclude` (usually
+        the training pairs; (users, items) or a PairCSR), and the ranking is scored against the user's relevant items =
+        the distinct held-out pairs (users, items) -- with rates >= min_rating when both are given -- minus any pair in
+        `exclude` (an excluded item can never be recommended).  Users without relevant items are not evaluated.
+        -> dict(hr, precision, recall, ndcg, n_users, n_uncertified): means over the evaluated users (hit rate, precision,
+        recall and NDCG at k, tfr_ranking_metrics on the device), n_users = how many were evaluated."""
+        excl = None
+        if exclude is not None:
+            excl = exclude if isinstance(exclude, PairCSR) else self.pair_csr(*exclude)
+        self._check_ids(users, items)
+        if rates is not None and min_rating is not None:
+            keep = self._dev_f32(rates) >= float(min_rating)
+            users, items = self._dev_i32(users)[keep], self._dev_i32(items)[keep]
+        dev = self.device
+        key = torch.unique(self._dev_i32(users).to(torch.int64) * self.I + self._dev_i32(items).to(torch.int64))
+        if excl is not None and excl.items.numel() > 0:
+            ex_user = torch.repeat_interleave(torch.arange(self.U, device=dev), excl.indptr[1:] - excl.indptr[:-1])
+            ex_key = ex_user * self.I + excl.items.to(torch.int64)   # sorted: CSR order
+            pos = torch.searchsorted(ex_key, key).clamp_(max=ex_key.numel() - 1)
+            key = key[ex_key[pos] != key]
+        rel_indptr = torch.zeros(self.U + 1, dtype=torch.int64, device=dev)
+        rel_indptr[1:] = torch.cumsum(torch.bincount(key // self.I, minlength=self.U), 0)
+        rel_item = (key % self.I).to(torch.int32).contiguous()
+        idx, _, n_unc = self._rank_excluding(k, n_cand, excl)
+        s = self.ranking_sums(idx, PairCSR(rel_indptr, rel_item)).cpu().numpy()
+        n = int(round(s[4]))
+        mean = (lambda x: float(x) / n) if n else (lambda x: float("nan"))
+        return dict(hr=mean(s[0]), precision=mean(s[1]), recall=mean(s[2]), ndcg=mean(s[3]), n_users=n,
+                    n_uncertified=n_unc)
+
+    def ranking_sums(self, topk_idx, relevant, row_metrics=None):
+        """tfr_ranking_metrics of a ranking topk_idx [n, k] (int32, device) against relevant, a PairCSR over the same n
+        rows -> (sum HR, sum precision, sum recall, sum NDCG, rows evaluated), float64 [5] on the device; row_metrics: a
+        float64 [n, 4] device tensor to receive the per-row values (NaN where not evaluated)."""
+        n, k = topk_idx.shape
+        dev = self.device
+        sums = torch.empty(5, dtype=torch.float64, device=dev)
+        nbytes = check(self.L.tfr_ranking_metrics_workspace_bytes(n, k))
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        with torch.cuda.device(dev):
+            check(self.L.tfr_ranking_metrics(topk_idx.data_ptr(), n, k, relevant.indptr.data_ptr(),
+                                             relevant.items.data_ptr(),
+                                             row_metrics.data_ptr() if row_metrics is not None else None, sums.data_ptr(),
+                                             ws.data_ptr(), nbytes, self._stream()))
+        return sums
 
     def observed_rmse(self, users, items, rates):
         """als3.py:110-120,139-143: RMSE of M[user_ids, work_ids] against the ratings, with M = U.V^T + biases consumed
         tile by tile in the GEMM epilogue (never materialised).  -> (rmse, row_se [U] float64)."""
-        self._check_ids(users, items)
         dev = self.device
-        u, i, r = self._dev_i32(users).to(torch.int64), self._dev_i32(items).to(torch.int64), self._dev_f32(rates)
-        order = torch.argsort(u * self.I + i, stable=True)     # CSR by user, item ids ascending inside a user
-        indptr = torch.zeros(self.U + 1, dtype=torch.int64, device=dev)
-        indptr[1:] = torch.cumsum(torch.bincount(u, minlength=self.U), 0)
-        it = i[order].to(torch.int32).contiguous()
-        rt = r[order].contiguous()
+        indptr, it, rt = self._csr_by_user(users, items, rates)
         row_se = torch.empty(self.U, dtype=torch.float64, device=dev)
         with torch.cuda.device(dev):
             check(self.L.tfr_allpairs_consume(self.t["user_feat"].data_ptr(), self.t["item_feat"].data_ptr(),
@@ -291,7 +394,7 @@ class SvdEngine:
                                               self.t["mu"].data_ptr(), self.U, self.I, self.d, self.feat_stride,
                                               self.feat_stride, 0, 0, None, None, None, indptr.data_ptr(), it.data_ptr(),
                                               rt.data_ptr(), row_se.data_ptr(), None, 0, self._stream()))
-        n = max(int(u.numel()), 1)
+        n = max(int(it.numel()), 1)
         return float(torch.sqrt(row_se.sum() / n)), row_se
 
     # ---- ranking: forward.py:47-61 get_ranking (every item scored for one user, sorted, first 50 kept) --------------
