@@ -408,6 +408,28 @@ int tfr_allpairs_rank_excluding(const float* user_feat, const float* item_feat, 
                                 const int64_t* excl_indptr, const int32_t* excl_item, double* topk_val, int32_t* topk_idx,
                                 int32_t* n_uncertified, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* ---- top-k ranking for a batch of QUERY users: forward.py:47-61 get_ranking for the users asked about -------------------
+ * Row q of topk_val (float64) / topk_idx [n_queries, k] is the ranking of user query_users[q], identical in ids and bits to
+ * that user's row of tfr_allpairs_rank_excluding with the same tables, k and exclusion list:
+ *  - score = ((acc + (double)b_u) + (double)b_i) + (double)mu, acc = sum over d = 0 .. dim-1, in that order from 0.0, of
+ *    (double)u[d] * (double)v[d]; flags & TFR_ABS_ITEM: v = |v| (the fork model's u.|v|; no other flag changes the score);
+ *  - score descending, lowest item id on ties; excluded items are never returned; a user with fewer than k rankable items
+ *    gets (-inf, -1) past the last one.
+ * excl_indptr int64 [n_users + 1] / excl_item: the exclusion CSR indexed by USER ID (not by query; ascending inside a user,
+ * duplicates allowed), e.g. the training pairs built once; null = nothing excluded.  query_users (device) may repeat and
+ * come in any order; an id outside [0, n_users) gives a row of (-inf, -1) and is never read through.  n_queries = 0 is a
+ * no-op.  1 <= dim <= 512, 1 <= k <= 1024, n_items < 2^31, else TFR_ERR_INVALID before any CUDA call.
+ * Float64 on CUDA cores: O(n_queries * n_items * dim), no tensor-core candidates.  The item axis is split into chunks
+ * (knob RANK_CHUNK, items per chunk) that are scored and selected in parallel, then merged per query: any chunking gives the
+ * same result.  workspace: tfr_rank_users_workspace_bytes (a function of its arguments only; needs no device). */
+int64_t tfr_rank_users_workspace_bytes(int64_t n_queries, int64_t n_items, int32_t k);
+int tfr_rank_users(const float* user_feat, const float* item_feat, const float* user_bias, const float* item_bias,
+                   const float* mu, int64_t n_users, int64_t n_items, int32_t dim,
+                   int64_t user_stride, int64_t item_stride /* floats between rows; 0 = dim */, int32_t flags,
+                   const int32_t* query_users, int64_t n_queries, int32_t k, const int64_t* excl_indptr,
+                   const int32_t* excl_item, double* topk_val, int32_t* topk_idx, void* workspace, int64_t workspace_bytes,
+                   void* stream);
+
 /* ---- host side of the feed_dict boundary: the columns a reference iterator yields (dataio.py:114-117: float64 views
  * of one [B, ncols] matrix, ids included) packed into a pinned staging buffer in the device's types -- int32 ids
  * (value cast, like TF feeding an int32 placeholder, A.7) followed by float32 rates: [users B | items B | rates B].

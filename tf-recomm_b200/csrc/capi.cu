@@ -48,6 +48,7 @@ const TuneEntry kTune[TUNE_COUNT] = {
     // step) and a loss at the ML-1M shape (the early-resident dependents delay the side stream's id sort: 53 vs 37 us)
     {"PDL", 0},
     {"SORT_SPLIT", 0},
+    {"RANK_CHUNK", 4096}, {"RANK_STAGES", 7},
 };
 std::mutex g_tune_mu;
 int g_tune_val[TUNE_COUNT];

@@ -29,6 +29,8 @@ enum TuneKey {
   TUNE_TL_EVERY_CTA,      // debug timeline: the pass's exit stamp from every CTA instead of a sample
   TUNE_PDL,               // 1: programmatic dependent launch along the step's critical path (see pdl_wait)
   TUNE_SORT_SPLIT,        // 1: every id sort in its one-launch-per-phase form (default: only inside the feed graph)
+  TUNE_RANK_CHUNK,        // tfr_rank_users: items per selection chunk (a multiple of 1024, 1024 .. 16384)
+  TUNE_RANK_STAGES,       // debug: which kernels of tfr_rank_users run (1 score | 2 select | 4 merge)
   TUNE_COUNT
 };
 int tune(TuneKey k);

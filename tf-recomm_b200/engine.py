@@ -309,6 +309,37 @@ class SvdEngine:
                 ws.data_ptr(), nbytes, self._stream()))
         return idx, val, int(n_unc.item())
 
+    def rank_users(self, users, k=50, exclude=None):
+        """forward.py:47-61 for the users asked about: -> (items [n, k] int32, scores [n, k] float64) on the device, row q
+        the ranking of users[q] (ids may repeat, any order; host or device), k = min(k, I).  Bit for bit the user's row of
+        rank_all_users(k, exclude=exclude), at a cost that scales with n instead of U (tfr_rank_users: float64 on CUDA
+        cores).  exclude: (users, items) pairs or a PairCSR from pair_csr(), indexed by user id; build it once for repeated
+        calls.  The fork model (ABS_ITEM) is ranked by u.|v| + biases."""
+        self._check_ids(users, [])
+        csr = None
+        if exclude is not None:
+            csr = exclude if isinstance(exclude, PairCSR) else self.pair_csr(*exclude)
+        q = self._dev_i32(np.atleast_1d(np.asarray(users)) if not isinstance(users, torch.Tensor) else users.reshape(-1))
+        n, k = int(q.numel()), int(min(k, self.I))
+        dev = self.device
+        idx = torch.empty(n, k, dtype=torch.int32, device=dev)
+        val = torch.empty(n, k, dtype=torch.float64, device=dev)
+        if n == 0:
+            return idx, val
+        nbytes = check(self.L.tfr_rank_users_workspace_bytes(n, self.I, k))
+        key = ("rank_users_ws", n, k)   # serving calls of one shape reuse their workspace
+        ws = self._stage.get(key)
+        if ws is None:
+            ws = self._stage[key] = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        with torch.cuda.device(dev):
+            check(self.L.tfr_rank_users(
+                self.t["user_feat"].data_ptr(), self.t["item_feat"].data_ptr(), self.t["user_bias"].data_ptr(),
+                self.t["item_bias"].data_ptr(), self.t["mu"].data_ptr(), self.U, self.I, self.d, self.feat_stride,
+                self.feat_stride, self.flags & ABS_ITEM, q.data_ptr(), n, k,
+                csr.indptr.data_ptr() if csr is not None else None, csr.items.data_ptr() if csr is not None else None,
+                val.data_ptr(), idx.data_ptr(), ws.data_ptr(), nbytes, self._stream()))
+        return idx, val
+
     def _csr_by_user(self, users, items, rates=None, dedup=False):
         """(user, item[, rate]) pairs -> CSR by user, item ids ascending inside a user: (indptr int64 [U + 1], items int32,
         rates float32 | None).  dedup: every distinct pair once (rates are then not carried); otherwise every pair as
@@ -925,6 +956,15 @@ class SvdEngine:
         arrays["__shape__"] = np.array([self.U, self.I, self.d, self.flags], np.int64)
         with open(path, "wb") as f:
             np.savez(f, **arrays)
+
+    @classmethod
+    def from_checkpoint(cls, path, device=None):
+        """An engine of the shape and model flags recorded in a checkpoint written by save(), restored from it."""
+        with np.load(path) as z:
+            U, I, d, flags = (int(x) for x in z["__shape__"])
+        eng = cls(U, I, d, 1e-3, 0.0, flags=flags, device=device)
+        eng.restore(path)
+        return eng
 
     def restore(self, path):
         z = np.load(path)
