@@ -430,6 +430,27 @@ int tfr_rank_users(const float* user_feat, const float* item_feat, const float* 
                    const int32_t* excl_item, double* topk_val, int32_t* topk_idx, void* workspace, int64_t workspace_bytes,
                    void* stream);
 
+/* ---- fold-in of users that were not trained: exact least-squares user rows against the fixed item side -----------------
+ * With item_feat, item_bias and mu fixed, the training loss (ops.py:81-89,124-126: squared error + reg * L2 on the gathered
+ * rows, biases too with TFR_REG_BIAS) restricted to one user is a ridge regression in theta = [p_u ; b_u].  Its per-occurrence
+ * gradients summed over the user's n ratings vanish exactly at the solution of
+ *   (sum_j x_j x_j^T + reg * n * D) theta = sum_j (r_j - mu - b_{i_j}) x_j,   x_j = [v~_{i_j} ; 1],
+ *   D = diag(1, ..., 1, REG_BIAS ? 1 : 0),   v~ = |v| with TFR_ABS_ITEM (ops.py:44), else v,
+ * duplicates counted as in training.  Row r's ratings are items / rates [indptr[r] .. indptr[r + 1]) (indptr int64 [n + 1]);
+ * out_feat [n, dim] / out_bias [n] receive theta rounded to fp32.  Float64 throughout, one CTA per row: Gram and right-hand
+ * side summed in the row's CSR order from 0.0 (no atomics: a row's bits depend on its own ratings only, whatever the batch),
+ * reg * n added to the diagonal, Cholesky + forward / back substitution in shared memory.  info [n] (int32): 0 = ok; j + 1 =
+ * pivot j was not > 0 (reachable only with reg = 0); -1 = an item id outside [0, n_items), never read through; a row with
+ * info != 0 is written as NaN.  A row without ratings gets p = 0, b = 0, info 0 (the model then scores it by mu + b_i).
+ * reg is used as (double)reg.  Asynchronous, no workspace, capturable in a CUDA graph; n = 0 is a no-op.  TFR_ERR_INVALID
+ * before any CUDA call for dim outside [1, 128], flags & TFR_LOSS_SIGMOID_CE (the fork's loss makes the problem
+ * nonlinear), reg negative, NaN or infinite, and null pointers when n > 0.  The output goes straight into tfr_rank_users
+ * as an n-row user table. */
+int tfr_fold_in_users(const float* item_feat, const float* item_bias, const float* mu, int64_t n_items, int32_t dim,
+                      int64_t item_stride /* floats between rows; 0 = dim */, int32_t flags, float reg,
+                      const int64_t* indptr, const int32_t* items, const float* rates, int64_t n, float* out_feat,
+                      float* out_bias, int32_t* info, void* stream);
+
 /* ---- host side of the feed_dict boundary: the columns a reference iterator yields (dataio.py:114-117: float64 views
  * of one [B, ncols] matrix, ids included) packed into a pinned staging buffer in the device's types -- int32 ids
  * (value cast, like TF feeding an int32 placeholder, A.7) followed by float32 rates: [users B | items B | rates B].

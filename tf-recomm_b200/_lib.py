@@ -157,6 +157,7 @@ _PROTOS = {
                                               i64, vp]),
     "tfr_rank_users_workspace_bytes": (i64, [i64, i64, i32]),
     "tfr_rank_users": (C.c_int, [vp, vp, vp, vp, vp, i64, i64, i32, i64, i64, i32, vp, i64, i32, vp, vp, vp, vp, vp, i64, vp]),
+    "tfr_fold_in_users": (C.c_int, [vp, vp, vp, i64, i32, i64, i32, f32, vp, vp, vp, i64, vp, vp, vp, vp]),
     "tfr_ranking_metrics_workspace_bytes": (i64, [i64, i32]),
     "tfr_ranking_metrics": (C.c_int, [vp, i64, i32, vp, vp, vp, vp, vp, i64, vp]),
     "tfr_host_pack_feed": (C.c_int, [vp, i32, i64, vp, i32, i64, vp, i32, i64, i64, vp]),

@@ -29,6 +29,16 @@ class PairCSR(NamedTuple):
     items: torch.Tensor
 
 
+class FoldedUsers(NamedTuple):
+    """Users folded into a trained model (SvdEngine.fold_in), on the device: feat [n, d] / bias [n] fp32, the row's
+    least-squares user row; ratings: the fold-in ratings as a PairCSR over the n rows (duplicates kept); info [n] int32,
+    0 = ok, j + 1 = pivot j was not > 0, -1 = an item id out of range (rows with info != 0 are NaN)."""
+    feat: torch.Tensor
+    bias: torch.Tensor
+    ratings: PairCSR
+    info: torch.Tensor
+
+
 def _require_cuda():
     if not torch.cuda.is_available():
         raise TfrError("tf-recomm_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback for this path")
@@ -170,10 +180,10 @@ class SvdEngine:
         check(self.L.tfr_svd_step_carve(ws.data_ptr(), ws.numel(), B, self.d, C.byref(out)))
         return out
 
-    def _check_ids(self, users, items):
+    def _check_ids(self, users, items, n_users=None):
         """ids outside the tables are an error where they enter (TF's CPU embedding_lookup raises
-        InvalidArgumentError): nothing out of range ever reaches a gather."""
-        for name, a, n in (("user", users, self.U), ("item", items, self.I)):
+        InvalidArgumentError): nothing out of range ever reaches a gather.  n_users: rows of the user side (default U)."""
+        for name, a, n in (("user", users, self.U if n_users is None else n_users), ("item", items, self.I)):
             if isinstance(a, torch.Tensor):
                 if a.numel() == 0:
                     continue
@@ -320,6 +330,11 @@ class SvdEngine:
         if exclude is not None:
             csr = exclude if isinstance(exclude, PairCSR) else self.pair_csr(*exclude)
         q = self._dev_i32(np.atleast_1d(np.asarray(users)) if not isinstance(users, torch.Tensor) else users.reshape(-1))
+        return self._rank_rows(self.t["user_feat"], self.t["user_bias"], self.U, self.feat_stride, q, k, csr)
+
+    def _rank_rows(self, user_feat, user_bias, n_users, user_stride, q, k, csr):
+        """tfr_rank_users of the query rows q (device int32) of the user table (user_feat, user_bias) against this
+        engine's item side; csr: exclusion CSR indexed by the table's rows, or None."""
         n, k = int(q.numel()), int(min(k, self.I))
         dev = self.device
         idx = torch.empty(n, k, dtype=torch.int32, device=dev)
@@ -333,18 +348,60 @@ class SvdEngine:
             ws = self._stage[key] = torch.empty(nbytes, dtype=torch.uint8, device=dev)
         with torch.cuda.device(dev):
             check(self.L.tfr_rank_users(
-                self.t["user_feat"].data_ptr(), self.t["item_feat"].data_ptr(), self.t["user_bias"].data_ptr(),
-                self.t["item_bias"].data_ptr(), self.t["mu"].data_ptr(), self.U, self.I, self.d, self.feat_stride,
+                user_feat.data_ptr(), self.t["item_feat"].data_ptr(), user_bias.data_ptr(),
+                self.t["item_bias"].data_ptr(), self.t["mu"].data_ptr(), n_users, self.I, self.d, user_stride,
                 self.feat_stride, self.flags & ABS_ITEM, q.data_ptr(), n, k,
                 csr.indptr.data_ptr() if csr is not None else None, csr.items.data_ptr() if csr is not None else None,
                 val.data_ptr(), idx.data_ptr(), ws.data_ptr(), nbytes, self._stream()))
         return idx, val
 
-    def _csr_by_user(self, users, items, rates=None, dedup=False):
+    # ---- fold-in: user rows for users the model was not trained on ------------------------------------------------------
+    def fold_in(self, rows, items, rates, n=None, reg=None):
+        """Least-squares user rows for new users (or new ratings of known ones) against the trained item side: for each
+        row label r in [0, n) the (p_u, b_u) that minimises the training loss (ops.py:81-89,124-126, squared error +
+        reg * L2) over the ratings (rows == r) with item_feat, item_bias and mu fixed -- tfr_fold_in_users, float64 normal
+        equations solved by Cholesky on the device.  rows / items / rates: host or device arrays of one rating each
+        (duplicates count, as in training); n defaults to max(rows) + 1; reg defaults to the engine's reg.  A row without
+        ratings gets p = 0, b = 0.  -> FoldedUsers (rank it with rank_folded).  The fork's sigmoid-CE loss is not a
+        least-squares problem and is refused."""
+        if self.flags & LOSS_SIGMOID_CE:
+            raise TfrError("fold_in solves the squared-error objective; the sigmoid cross-entropy model is not supported")
+        reg = self.hyper["reg"] if reg is None else float(reg)
+        if not reg >= 0.0:
+            raise TfrError("fold_in: reg must be >= 0, got %r" % reg)
+        sizes = [a.numel() if isinstance(a, torch.Tensor) else np.asarray(a).size for a in (rows, items, rates)]
+        if len(set(sizes)) != 1:
+            raise TfrError("fold_in: rows, items and rates differ in length: %s" % sizes)
+        if n is None:
+            n = int((rows if isinstance(rows, torch.Tensor) else np.asarray(rows)).max()) + 1 if sizes[0] else 0
+        n = int(n)
+        indptr, it, rt = self._csr_by_user(rows, items, rates, n_rows=n)
+        dev = self.device
+        feat = torch.empty(n, self.d, dtype=torch.float32, device=dev)
+        bias = torch.empty(n, dtype=torch.float32, device=dev)
+        info = torch.empty(n, dtype=torch.int32, device=dev)
+        with torch.cuda.device(dev):
+            check(self.L.tfr_fold_in_users(
+                self.t["item_feat"].data_ptr(), self.t["item_bias"].data_ptr(), self.t["mu"].data_ptr(), self.I, self.d,
+                self.feat_stride, self.flags, reg, indptr.data_ptr(), it.data_ptr(), rt.data_ptr(), n, feat.data_ptr(),
+                bias.data_ptr(), info.data_ptr(), self._stream()))
+        return FoldedUsers(feat, bias, PairCSR(indptr, it), info)
+
+    def rank_folded(self, folded, k=50, exclude_rated=True):
+        """Top-k of folded users (fold_in): -> (items [n, k] int32, scores [n, k] float64) on the device, row r the ranking
+        of folded row r, scored as rank_users scores a trained user (tfr_rank_users on the folded rows as an n-row user
+        table; u.|v| for the fork model).  exclude_rated: never recommend the items the row was folded in from.  A row
+        that could not be folded (info != 0, NaN) ranks nothing: (-inf, -1)."""
+        n = int(folded.feat.shape[0])
+        q = torch.arange(n, dtype=torch.int32, device=self.device)
+        return self._rank_rows(folded.feat, folded.bias, n, 0, q, k, folded.ratings if exclude_rated else None)
+
+    def _csr_by_user(self, users, items, rates=None, dedup=False, n_rows=None):
         """(user, item[, rate]) pairs -> CSR by user, item ids ascending inside a user: (indptr int64 [U + 1], items int32,
         rates float32 | None).  dedup: every distinct pair once (rates are then not carried); otherwise every pair as
-        given, duplicates included."""
-        self._check_ids(users, items)
+        given, duplicates included, in a stable order.  n_rows: rows of the CSR (user ids in [0, n_rows)), default U."""
+        self._check_ids(users, items, n_rows)
+        n_rows = self.U if n_rows is None else n_rows
         dev = self.device
         u, i = self._dev_i32(users).to(torch.int64), self._dev_i32(items).to(torch.int64)
         rt = None
@@ -356,8 +413,8 @@ class SvdEngine:
             order = torch.argsort(u * self.I + i, stable=True)
             it = i[order].to(torch.int32).contiguous()
             rt = r[order].contiguous() if r is not None else None
-        indptr = torch.zeros(self.U + 1, dtype=torch.int64, device=dev)
-        indptr[1:] = torch.cumsum(torch.bincount(u, minlength=self.U), 0)
+        indptr = torch.zeros(n_rows + 1, dtype=torch.int64, device=dev)
+        indptr[1:] = torch.cumsum(torch.bincount(u, minlength=n_rows), 0)
         return indptr, it, rt
 
     def pair_csr(self, users, items):
