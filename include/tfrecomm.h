@@ -59,7 +59,14 @@ int tfr_device_sm_count(void);
  * tfr_tune_set gave it, else the environment variable TFR_<NAME> at first use, else its default.  Names (csrc/capi.cu):
  * SMEM_CARVEOUT, SEG_TILE, SEG_MAX_UNITS, PASS_RING (1 = interleaved tables take the TMA-bulk ring pass, 0 = the
  * LDG/STG pass), RING_STAGES, RING_STAGE_KB, RING_THREADS, RING_L2_HINT, STREAM_THREADS, STREAM_CTAS_PER_SM, ...
- * Knobs change launch geometry only, never results. */
+ * What a knob may change:
+ *  - bit for bit the same results: SMEM_CARVEOUT, TILES_CARVEOUT, STREAM_LD, STREAM_ST, STREAM_CTAS_PER_SM,
+ *    STREAM_UNROLL, STREAM_THREADS, STREAM_DYNAMIC, TL_EVERY_CTA, PDL, SORT_SPLIT, PASS_RING, RING_STAGES,
+ *    RING_STAGE_KB, RING_THREADS, RING_L2_HINT, RING_CTAS_PER_SM, RING_SLOT_MODE 0..2, RANK_CHUNK;
+ *  - the fp32 rounding of the training step, within the oracle's 1e-5 bar: SEG_TILE (where runs of equal ids are
+ *    regrouped into partial sums; its default depends on the batch size, the dim and the device's SM count) and
+ *    SEG_MAX_UNITS (lanes per row, hence the order of the fused forward's dot products, and the default tile);
+ *  - results, on purpose (debug and measurement only): STREAM_COPY_ONLY, RING_SLOT_MODE 3, AP_STAGES, RANK_STAGES. */
 int tfr_tune_set(const char* name, int32_t value);
 int tfr_tune_get(const char* name, int32_t* value);
 

@@ -690,6 +690,7 @@ def test_ring_pass_bit_identical(shape, ring_cfg):
     B = 700
     batches = [make_batch(rng, U, I, B) for _ in range(3)]
     out = []
+    saved = {k: _lib.tune_get(k) for k in ["PASS_RING", *ring_cfg]}
     try:
         for ring in (0, 1):
             _lib.tune_set("PASS_RING", ring)
@@ -701,8 +702,7 @@ def test_ring_pass_bit_identical(shape, ring_cfg):
             torch.cuda.synchronize()
             out.append((eng.get_tables(), eng.opt_scalars()))
     finally:
-        _lib.tune_set("PASS_RING", 0)
-        for k, v in dict(RING_STAGES=4, RING_STAGE_KB=24, RING_THREADS=320, RING_L2_HINT=2).items():
+        for k, v in saved.items():
             _lib.tune_set(k, v)
     (ta, sa), (tb, sb) = out
     for n in ta:

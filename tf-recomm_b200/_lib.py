@@ -200,7 +200,10 @@ def check(rc):
 
 
 def tune_set(name, value):
-    """Process-wide tuning knob (tfr_tune_set): launch geometry only, never results."""
+    """Process-wide tuning knob (tfr_tune_set).  Most knobs change launch geometry only and keep results bit for bit;
+    SEG_TILE and SEG_MAX_UNITS change the fp32 rounding of the training step (within the oracle's 1e-5 bar);
+    STREAM_COPY_ONLY, RING_SLOT_MODE=3, AP_STAGES and RANK_STAGES are debug knobs that change results on purpose
+    (include/tfrecomm.h lists them all)."""
     check(load().tfr_tune_set(name.encode(), int(value)))
 
 

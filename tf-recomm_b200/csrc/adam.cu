@@ -380,9 +380,12 @@ static int launch_stream_chunks(const StreamTab* chunks, int n_chunks, const tfr
   // CTAs of 512 threads take the whole register file, and the id sort of the NEXT batch (8K registers per CTA,
   // forked under this pass) could then only start when the pass drains -- which puts it on the critical path.
   // (3 x 256 also leaves room but measures 7 % slower: TFR_STREAM_* to experiment.)
-  const int cfg_ctas = tune(TUNE_STREAM_CTAS_PER_SM), cfg_unroll = tune(TUNE_STREAM_UNROLL);
+  const int cfg_ctas = tune(TUNE_STREAM_CTAS_PER_SM);
+  int cfg_unroll = tune(TUNE_STREAM_UNROLL);
+  if (cfg_unroll < 1) cfg_unroll = 2;
   int cfg_threads = tune(TUNE_STREAM_THREADS);
   if (cfg_threads < 32 || cfg_threads > 512) cfg_threads = 448;
+  cfg_threads &= ~31;  // whole warps: the dynamic variant's warp-wide shuffle needs every lane
   int64_t grid = ((int64_t)units + cfg_threads * cfg_unroll - 1) / (cfg_threads * cfg_unroll);
   const int64_t cap = (int64_t)sm_count() * cfg_ctas;
   if (cfg_ctas > 0 && grid > cap) grid = cap;

@@ -647,13 +647,30 @@ using namespace tfr;
 namespace tfr {
 // Lane-group geometry of the tiles kernel: few lanes per row, several units (of VEC floats) per lane -- a warp then
 // walks 32/L tiles at once and everything that is per entry rather than per float (shuffles, branches, addresses) is
-// paid once per warp instruction for 32/L entries.  UNITS is 1, 2 or 4 (rounded up; surplus units are masked).
+// paid once per warp instruction for 32/L entries.  UNITS is 1, 2, 4, 8 or 16 (rounded up; surplus units are masked);
+// 8 and 16 only occur for rows of 129..511 floats with dim % 4 != 0 (32 lanes of one float each).
 struct SegGeom {
   int vec, lanes, units;
 };
-static SegGeom seg_geom(int dim) {
-  int forced = tune(TUNE_SEG_MAX_UNITS);  // experiments: force 1, 2 or 4 units per lane
-  if (forced != 1 && forced != 2 && forced != 4) forced = 0;
+// Every (VEC, L, UNITS) the tiles kernel is instantiated for: launch_segsum dispatches over this list, and for every dim
+// of 1..512 seg_geom returns a member of it, whatever SEG_MAX_UNITS is (tests/test_geometry.py mirrors both).
+#define TFR_SEG_CASES(X)                                                                                            \
+  /* default geometry (<= 4 units per lane): L = 1 for rows of up to 4 units, then UNITS = 4 */                     \
+  X(4, 1, 1) X(4, 1, 2) X(4, 1, 4) X(4, 2, 4) X(4, 4, 4) X(4, 8, 4) X(4, 16, 4) X(4, 32, 4)                         \
+  X(1, 1, 1) X(1, 1, 2) X(1, 1, 4) X(1, 2, 4) X(1, 4, 4) X(1, 8, 4) X(1, 16, 4) X(1, 32, 4)                         \
+  /* one unit per lane (rows of fewer than 32 units), two units (rows of 33..64 floats, dim % 4 != 0) */            \
+  X(4, 2, 1) X(4, 4, 1) X(4, 8, 1) X(4, 16, 1) X(4, 32, 1)                                                          \
+  X(1, 2, 1) X(1, 4, 1) X(1, 8, 1) X(1, 16, 1) X(1, 32, 1)                                                          \
+  X(1, 32, 2) X(4, 16, 2) X(1, 8, 2)                                                                                \
+  /* rows of 129..511 floats, dim % 4 != 0 */                                                                       \
+  X(1, 32, 8) X(1, 32, 16)
+static bool seg_case_exists(const SegGeom& g) {
+#define TFR_SEG_HAS(V, LL, UU) if (g.vec == V && g.lanes == LL && g.units == UU) return true;
+  TFR_SEG_CASES(TFR_SEG_HAS)
+#undef TFR_SEG_HAS
+  return false;
+}
+static SegGeom seg_geom_max_units(int dim, int forced) {
   SegGeom g;
   g.vec = (dim % 4 == 0) ? 4 : 1;
   const int n_units = dim / g.vec;
@@ -665,7 +682,16 @@ static SegGeom seg_geom(int dim) {
   while (l * max_units < n_units && l < 32) l <<= 1;
   g.lanes = l;
   const int u = (n_units + l - 1) / l;
-  g.units = u <= 1 ? 1 : (u <= 2 ? 2 : (u <= 4 ? 4 : u));
+  g.units = u <= 1 ? 1 : u <= 2 ? 2 : u <= 4 ? 4 : u <= 8 ? 8 : u <= 16 ? 16 : u;
+  return g;
+}
+static SegGeom seg_geom(int dim) {
+  int forced = tune(TUNE_SEG_MAX_UNITS);  // experiments: force 1, 2 or 4 units per lane
+  if (forced != 1 && forced != 2 && forced != 4) forced = 0;
+  const SegGeom g = seg_geom_max_units(dim, forced);
+  // a forced unit count that has no instantiation for this dim falls back to the default geometry HERE, so that the
+  // tile size, the fused forward's partial count (segsum_grid_x) and the launch all see the same geometry
+  if (forced && !seg_case_exists(g)) return seg_geom_max_units(dim, 0);
   return g;
 }
 // Tile size: a lane group walks its tile entry by entry (a chain of dependent instructions), so the kernel's time is
@@ -754,18 +780,11 @@ static int launch_segsum(const SegSide& su, const SegSide& si, int n_sides, cons
                            fw ? (int)grid.x : 0));                                                                  \
     return TFR_OK;                                                                                                 \
   }
-  // default geometry (<= 4 units per lane): L = 1 for rows of up to 4 units, then UNITS = 4
-  TFR_SEG_CASE(4, 1, 1) TFR_SEG_CASE(4, 1, 2) TFR_SEG_CASE(4, 1, 4) TFR_SEG_CASE(4, 2, 4) TFR_SEG_CASE(4, 4, 4)
-  TFR_SEG_CASE(4, 8, 4) TFR_SEG_CASE(4, 16, 4) TFR_SEG_CASE(4, 32, 4)
-  TFR_SEG_CASE(1, 1, 1) TFR_SEG_CASE(1, 1, 2) TFR_SEG_CASE(1, 1, 4) TFR_SEG_CASE(1, 2, 4) TFR_SEG_CASE(1, 4, 4)
-  TFR_SEG_CASE(1, 8, 4) TFR_SEG_CASE(1, 16, 4) TFR_SEG_CASE(1, 32, 4)
-  // one unit per lane (rows of fewer than 32 units), two units (rows of 33..64 floats, dim % 4 != 0)
-  TFR_SEG_CASE(4, 2, 1) TFR_SEG_CASE(4, 4, 1) TFR_SEG_CASE(4, 8, 1) TFR_SEG_CASE(4, 16, 1) TFR_SEG_CASE(4, 32, 1)
-  TFR_SEG_CASE(1, 2, 1) TFR_SEG_CASE(1, 4, 1) TFR_SEG_CASE(1, 8, 1) TFR_SEG_CASE(1, 16, 1) TFR_SEG_CASE(1, 32, 1)
-  TFR_SEG_CASE(1, 32, 2) TFR_SEG_CASE(4, 16, 2) TFR_SEG_CASE(1, 8, 2)
+  TFR_SEG_CASES(TFR_SEG_CASE)
 #undef TFR_SEG_CASE
 #undef TFR_SEG_LAUNCH
-  set_error("unsupported dim %d (vec %d lanes %d units %d): at most 512 floats per row", dim, g.vec, g.lanes, units);
+  set_error("unsupported dim %d (vec %d lanes %d units %d): the segment sums take rows of 1 to 512 floats", dim, g.vec,
+            g.lanes, units);
   return TFR_ERR_INVALID;
 }
 
