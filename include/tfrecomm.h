@@ -387,7 +387,9 @@ int tfr_allpairs(const float* user_feat, const float* item_feat, const float* us
  *    (n_cand <= 128; 64 for k = 50 is plenty); the candidates are then rescored in float64 -- the reference's own
  *    precision, als3.py:112 is numpy float64 -- ranked (score descending, lowest item index on ties) and CERTIFIED: the
  *    first k are the exact top-k of the whole row if the k-th exact score exceeds the worst candidate's tensor-core score
- *    by more than the tf32 error bound 2^-9 * ||u|| * max||v||.  Rows that cannot be certified (near-ties) are redone over
+ *    by more than a bound on the tensor-core score's error, (2^-9 + dim * 2^-22) * ||u|| * max||v|| + 2^-22 * (||u|| *
+ *    max||v|| + |b_u| + max|fl(b_i + mu)|) (tf32 operands, fp32 accumulation and bias additions).  n_cand below 11 keeps
+ *    11 candidates (the workspace query accounts for them).  Rows that cannot be certified (near-ties) are redone over
  *    all items in float64 on CUDA cores.  Result: topk_val (float64) / topk_idx [n_users, k], identical to ranking the
  *    float64 score matrix; *n_uncertified = how many rows took the exact path.  Missing ranks (k > n_items): (-inf, -1).
  *  obs_indptr != null: the squared error on the OBSERVED pairs, als3.py:110-120,139-143 (predict = M[user_ids, work_ids],

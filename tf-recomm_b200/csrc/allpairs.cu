@@ -498,8 +498,22 @@ __global__ void __launch_bounds__(AP_THREADS, 1)
 }
 
 // ---- exact rescore of the tensor-core candidates, with a certificate --------------------------------------------------
-// The tensor cores rank with tf32 operands (fp32 words whose low 13 mantissa bits are ignored): a score is off by at most
-//   E_u = 2.01 * 2^-10 * ||u||_2 * max_i ||v_i||_2  (+ fp32 accumulation / bias roundings, covered by the 2^-9 used).
+// The sweep ranks s = fl(fl(D + b_u) + fl(b_i + mu)) (fp32, round to nearest), D the tensor cores' fp32 dot product of
+// tf32 operands.  Its distance from the exact score u.v + b_u + b_i + mu is at most
+//   E_u = (2^-9 + dim * 2^-22) * ||u|| * V  +  2^-22 * (||u|| * V + |b_u| + B),   V = max_i ||v_i||, B = max_i |fl(b_i + mu)|:
+//   * tf32: the MMA reads 10 of an operand's 23 mantissa bits, |x' - x| < 2^-10 |x| whether it truncates or rounds, so
+//     |u'v' - uv| < (2^-9 + 2^-20) |uv|;
+//   * accumulation: dim/8 k-steps each add 8 exact products to the fp32 accumulator.  Even a step that aligns its 9
+//     addends to the largest and truncates each of them and its result to 24 bits loses < 10 ulps (2^-23 relative) of
+//     values <= sum |u'v'|: over the sweep < dim/8 * 20 * 2^-24 = 0.625 * dim * 2^-22 of sum |u'v'|.  With the 2^-20 of
+//     the products (dim >= 32) the dot product is within (2^-9 + dim * 2^-22) * sum_k |u_k v_k|, and sum_k |u_k v_k| <=
+//     ||u|| * V;
+//   * the three additions round to nearest, each by <= 2^-24 of its result: fl(b_i + mu) is <= B, fl(D + b_u) and s are
+//     <= |D| + |b_u| (+ B), so together <= 2^-23 (1 + 2^-23) (|D| + |b_u| + B): 2^-22 leaves a factor of 2.  This term is
+//     what is left when ||u|| * V vanishes (a zero user row, an all-zero item table) and the biases do not.
+// V and B come from allpairs_vmax2_kernel (V^2 rounded up).  Measured on a B200 (1000 W power limit) with
+// tests/test_topk_certificate.py's inputs: |s - exact| <= 0.47 E_u, and on random operands the dot product's error is
+// <= 0.27 * 2^-9 * sum_k |u_k v_k|; kind::tf32 truncates (its scores equal a truncating model's bit for bit).
 // Every item that is NOT in a row's two buffers scored at most T = max of the buffers' thresholds on the tensor cores,
 // hence at most T + E_u exactly (a buffer that never had to drop anything has threshold -inf).  The candidates are
 // rescored in float64 -- the reference's own precision: als3.py:112 is numpy float64 -- and the k best picked (score
@@ -515,8 +529,8 @@ __global__ void __launch_bounds__(32 * RS_WARPS) allpairs_rescore_kernel(
     const float* __restrict__ U, const float* __restrict__ V, const float* __restrict__ ub, const float* __restrict__ ib,
     const float* __restrict__ mu, int n_users, int n_items, int dim, int64_t us, int64_t is,
     const float* __restrict__ cand_val, const int32_t* __restrict__ cand_idx, const int32_t* __restrict__ cand_cnt,
-    const float* __restrict__ cand_thr, int K, int k, const float* __restrict__ vmax2, double* __restrict__ out_val,
-    int32_t* __restrict__ out_idx, int32_t* __restrict__ uncert, int32_t* __restrict__ n_uncert,
+    const float* __restrict__ cand_thr, int K, int k, const float* __restrict__ vmax2 /* [V^2, B] */,
+    double* __restrict__ out_val, int32_t* __restrict__ out_idx, int32_t* __restrict__ uncert, int32_t* __restrict__ n_uncert,
     const int64_t* __restrict__ excl_indptr, const int32_t* __restrict__ excl_item) {
   __shared__ double s_sc[RS_WARPS][8 * AP_MAX_CAND];
   __shared__ int s_ix[RS_WARPS][8 * AP_MAX_CAND];
@@ -601,15 +615,18 @@ __global__ void __launch_bounds__(32 * RS_WARPS) allpairs_rescore_kernel(
     const int kk = k < rankable ? k : rankable;
     bool certified = T == -INFINITY;   // nothing was ever dropped: every rankable item is a candidate
     if (!certified && got >= kk) {
-      const double E = 0.001953125 * sqrt(un2) * sqrt((double)vmax2[0]);   // 2^-9 * ||u|| * max ||v||
+      const double uv = sqrt(un2) * sqrt((double)vmax2[0]);
+      const double E = (0x1p-9 + dim * 0x1p-22) * uv + 0x1p-22 * (uv + fabs((double)ub[row]) + (double)vmax2[1]);
       certified = kth > (double)T + E;
     }
     if (!certified) uncert[atomicAdd(n_uncert, 1)] = row;
   }
 }
 
-// max over the item rows of ||v||^2 (float, atomicMax on the bit pattern of a non-negative float); out zeroed by the caller
-__global__ void allpairs_vmax2_kernel(const float* __restrict__ V, int n_items, int dim, int64_t is, float* __restrict__ out) {
+// out[0] = max over the item rows of ||v||^2, out[1] = max |fl(b_i + mu)| (the sweep's add_rn), both by atomicMax on the
+// bit pattern of a non-negative float; out zeroed by the caller
+__global__ void allpairs_vmax2_kernel(const float* __restrict__ V, const float* __restrict__ ib, const float* __restrict__ mu,
+                                      int n_items, int dim, int64_t is, float* __restrict__ out) {
   const int lane = threadIdx.x & 31;
   const int it = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (it >= n_items) return;
@@ -619,7 +636,10 @@ __global__ void allpairs_vmax2_kernel(const float* __restrict__ V, int n_items, 
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) n2 += __shfl_xor_sync(0xffffffffu, n2, o);
   n2 = n2 * 1.0001f;  // the float sum may round down
-  if (lane == 0) atomicMax(reinterpret_cast<int*>(out), __float_as_int(n2));
+  if (lane == 0) {
+    atomicMax(reinterpret_cast<int*>(out), __float_as_int(n2));
+    atomicMax(reinterpret_cast<int*>(out) + 1, __float_as_int(fabsf(add_rn(ib[it], *mu))));
+  }
 }
 
 // The uncertified rows, redone exactly over ALL items: a persistent CTA per row computes the row's float64 scores into
@@ -943,8 +963,14 @@ static int launch_allpairs_tc(const float* user_feat, const float* item_feat, co
 
 static int ap_exact_ctas() { return 2 * sm_count(); }
 
+// Candidates the sweep keeps per row-half.  A buffer of C = 4K entries must take the K kept after a compaction plus the up
+// to 32 appends of the next column chunk (the sweep compacts a buffer with more than C - 32 entries after each chunk):
+// 4K >= K + 32, so a smaller n_cand keeps 11.  More candidates than asked only make the certificate easier to meet.
+static int ap_buffer_k(int n_cand) { return n_cand > 11 ? n_cand : 11; }
+
 extern "C" int64_t tfr_allpairs_topk_workspace_bytes(int64_t n_users, int64_t n_items, int32_t k, int32_t n_cand) {
   if (n_users < 0 || n_items < 0 || k <= 0 || n_cand < k || n_cand > AP_MAX_CAND) return TFR_ERR_INVALID;
+  n_cand = ap_buffer_k(n_cand);
   return 256 + 2 * align_up(8 * n_users * (int64_t)n_cand * 4, 256) + 3 * align_up(2 * n_users * 4, 256) +
          align_up((int64_t)ap_exact_ctas() * n_items * 8, 256) + 256;
 }
@@ -985,6 +1011,7 @@ static int allpairs_consume_impl(const float* user_feat, const float* item_feat,
       set_error("all-pairs top-k workspace too small");
       return TFR_ERR_WORKSPACE;
     }
+    n_cand = ap_buffer_k(n_cand);
     char* w = reinterpret_cast<char*>(align_up((int64_t)(uintptr_t)workspace, 256));
     vmax2 = reinterpret_cast<float*>(w); w += 256;
     cs.cand_val = reinterpret_cast<float*>(w); w += align_up(8 * n_users * (int64_t)n_cand * 4, 256);
@@ -1017,7 +1044,8 @@ static int allpairs_consume_impl(const float* user_feat, const float* item_feat,
                             cs, st);
   if (rc) return rc;
   if (topk && (stages & 2)) {
-    allpairs_vmax2_kernel<<<(unsigned)((n_items * 32 + 255) / 256), 256, 0, st>>>(item_feat, (int)n_items, dim, item_stride, vmax2);
+    allpairs_vmax2_kernel<<<(unsigned)((n_items * 32 + 255) / 256), 256, 0, st>>>(item_feat, item_bias, mu, (int)n_items, dim,
+                                                                               item_stride, vmax2);
     TFR_LAUNCH_CHECK();
     allpairs_rescore_kernel<<<(unsigned)((n_users + RS_WARPS - 1) / RS_WARPS), 32 * RS_WARPS, 0, st>>>(
         user_feat, item_feat, user_bias, item_bias, mu, (int)n_users, (int)n_items, dim, user_stride, item_stride,
