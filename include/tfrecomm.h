@@ -66,6 +66,8 @@ int tfr_device_sm_count(void);
  *  - the fp32 rounding of the training step, within the oracle's 1e-5 bar: SEG_TILE (where runs of equal ids are
  *    regrouped into partial sums; its default depends on the batch size, the dim and the device's SM count) and
  *    SEG_MAX_UNITS (lanes per row, hence the order of the fused forward's dot products, and the default tile);
+ *  - the float64 summation order of the ALS half-sweep's heavy rows, which keeps parity with the exact solution, not bits:
+ *    ALS_CHUNK (ratings per Gram chunk; read once, by tfr_als_chunk, when a plan is built);
  *  - results, on purpose (debug and measurement only): STREAM_COPY_ONLY, RING_SLOT_MODE 3, AP_STAGES, RANK_STAGES. */
 int tfr_tune_set(const char* name, int32_t value);
 int tfr_tune_get(const char* name, int32_t* value);
@@ -459,6 +461,52 @@ int tfr_fold_in_users(const float* item_feat, const float* item_bias, const floa
                       int64_t item_stride /* floats between rows; 0 = dim */, int32_t flags, float reg,
                       const int64_t* indptr, const int32_t* items, const float* rates, int64_t n, float* out_feat,
                       float* out_bias, int32_t* info, void* stream);
+
+/* ---- alternating least squares: exact user and item half-sweeps on the device --------------------------------------------
+ * The objective is the training loss of the squared-error model, summed over every training occurrence (duplicates count):
+ *   L = sum_(u,i,r) [ 1/2 (r - mu - b_u - b_i - p_u.q_i)^2 + 1/2 reg (|p_u|^2 + |q_i|^2) (+ 1/2 reg (b_u^2 + b_i^2) with
+ *       TFR_REG_BIAS) ]
+ * A sweep is three exact block minimisations of L, each of which can only lower it in exact arithmetic:
+ *   1. users: tfr_als_half_sweep with the item side fixed (fixed = item_feat / item_bias, CSR by user of the item ids);
+ *   2. items: tfr_als_half_sweep with the user side fixed (fixed = the fp32 user rows of step 1, CSR by item of the user ids);
+ *   3. mu <- mu + sum e / N: tfr_svd_objective with mu_out = mu.
+ * tfr_als_half_sweep: every row r of the solved side listed in light_rows or heavy_rows gets the (feat, bias) that solves
+ * fold-in's system (tfr_fold_in_users) over its ratings partner / rates [indptr[r] .. indptr[r + 1]) against the fixed side,
+ * in float64, rounded to fp32 and written to out_feat + r * out_stride / out_bias[r] (the m / v rows of an interleaved
+ * table are never touched).  The plan (built once per training set by the caller):
+ *   - light_rows [n_light]: rows with <= chunk ratings, solved one CTA per row with fold-in's code (same bits as
+ *     tfr_fold_in_users of the same CSR);
+ *   - heavy_rows [n_heavy], heavy_ptr int64 [n_heavy + 1], chunk_heavy [n_chunks]: rows with > chunk ratings; heavy row h owns
+ *     chunks [heavy_ptr[h], heavy_ptr[h + 1]) of `chunk` consecutive ratings (the last one shorter), chunk_heavy[c] = h.
+ *     One CTA per chunk writes its float64 Gram + right-hand side to the workspace (tfr_als_workspace_bytes(n_chunks, dim):
+ *     (D (D + 1) / 2 + D) * 8 bytes per chunk, D = dim + 1), one CTA per heavy row sums them in chunk order and solves.
+ *     chunk is the plan's: tfr_als_chunk() (knob ALS_CHUNK, clamped to [32, 2^20] and rounded up to a multiple of 32) at
+ *     the time the plan was built.
+ * A row without ratings gets zeros.  A row whose pivot is not > 0 (unreachable with reg > 0) or that names a partner id
+ * outside [0, n_fixed) keeps its previous values and adds 1 to *n_failed (device int32, never reset here).  Asynchronous,
+ * no host synchronisation, capturable in a CUDA graph; n_light = n_heavy = 0 is a no-op.  TFR_ERR_INVALID before any CUDA
+ * call for dim outside [1, 128], flags & (TFR_LOSS_SIGMOID_CE | TFR_ABS_ITEM) (not least squares / not quadratic in q_i),
+ * var_mask != TFR_VAR_ALL, reg <= 0, NaN or infinite (with reg > 0 every system is SPD) and null pointers.
+ * tfr_svd_objective: over the CSR by user of the training ratings (user_items / user_rates, in range) and the item CSR's
+ * indptr (for the item rows' occurrence counts), e = r - mu - b_u - b_i - p_u.q~_i per occurrence in float64 from the fp32
+ * tables (q~ = |q| with TFR_ABS_ITEM); out6 (device, 6 doubles, optional) = (L, sum e^2, sum e, sum n_row |row|^2,
+ * sum n_row b_row^2, N); mu_out (optional) = fl32(mu + sum e / N) when N > 0 (step 3).  Fixed-order reduction, no
+ * floating-point atomics: the same bits every run.  workspace: tfr_svd_objective_workspace_bytes. */
+int32_t tfr_als_chunk(void);
+int64_t tfr_als_workspace_bytes(int64_t n_chunks, int32_t dim);
+int tfr_als_half_sweep(const float* fixed_feat, const float* fixed_bias, const float* mu, int64_t n_fixed, int32_t dim,
+                       int64_t fixed_stride /* floats between rows; 0 = dim */, int32_t flags, int32_t var_mask, float reg,
+                       const int64_t* indptr, const int32_t* partner, const float* rates, const int32_t* light_rows,
+                       int64_t n_light, const int32_t* heavy_rows, const int64_t* heavy_ptr, int64_t n_heavy,
+                       const int32_t* chunk_heavy, int64_t n_chunks, int32_t chunk, float* out_feat,
+                       int64_t out_stride /* 0 = dim */, float* out_bias, int32_t* n_failed, void* workspace,
+                       int64_t workspace_bytes, void* stream);
+int64_t tfr_svd_objective_workspace_bytes(int64_t n_users, int64_t n_items);
+int tfr_svd_objective(const float* user_feat, const float* user_bias, const float* item_feat, const float* item_bias,
+                      const float* mu, int64_t n_users, int64_t n_items, int32_t dim, int64_t user_stride,
+                      int64_t item_stride /* 0 = dim */, int32_t flags, float reg, const int64_t* user_indptr,
+                      const int32_t* user_items, const float* user_rates, const int64_t* item_indptr, double* out6,
+                      float* mu_out, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ---- host side of the feed_dict boundary: the columns a reference iterator yields (dataio.py:114-117: float64 views
  * of one [B, ncols] matrix, ids included) packed into a pinned staging buffer in the device's types -- int32 ids

@@ -17,6 +17,10 @@ Two ways to run the step loop:
   --mode stream    the same batches, but the training columns live in HBM and the whole epoch's index stream is
                    drawn up front (same RandomState consumption); each step is one replay of a captured CUDA graph.
 
+--solver als trains by alternating least squares instead (SvdEngine.als_sweep): every epoch is one sweep that solves each
+user row, then each item row, exactly in float64 against the other side, then updates mu; TRAIN is the RMSE over the whole
+training set after the sweep.  --batch, --lr and --mode do not apply to it.
+
 --topk K adds, after every report, the top-K recommendation quality on the validation split: each user is ranked over
 the items they did not rate in training, and hit rate / precision / recall / NDCG at K are measured against their
 validation items (rated >= --topk-min-rating; on the DISCRETE branch, an outcome of 1).
@@ -215,6 +219,78 @@ def svd(train, test, args, log=print):
     return history
 
 
+def svd_als(train, test, args, log=print):
+    """--solver als: the same model, initialisation, report lines, --topk, summaries and checkpoint as svd(), trained by one
+    ALS sweep per epoch.  TRAIN(size=N/N) is the RMSE over every training rating (tfr_svd_objective), TEST the forward's."""
+    user_batch = ops.placeholder(ops.int32, shape=[None], name="id_user")
+    item_batch = ops.placeholder(ops.int32, shape=[None], name="id_item")
+    rate_batch = ops.placeholder(ops.float32, shape=[None])
+    wins_batch = ops.placeholder(ops.float32, shape=[None], name="nb_wins")
+    fails_batch = ops.placeholder(ops.float32, shape=[None], name="nb_fails")
+    ops.reset_default_graph()
+    infer, logits, regularizer, _, _, _, _ = ops.inference_svd(
+        user_batch, item_batch, wins_batch, fails_batch, user_num=args.user_num, item_num=args.item_num, dim=args.dim,
+        device=config.DEVICE, variant=args.variant)
+    ops.train.get_or_create_global_step()
+    ops.optimization(infer, logits, regularizer, rate_batch, learning_rate=args.lr, reg=args.reg, device=config.DEVICE)
+    init_op = ops.group(ops.global_variables_initializer(), ops.local_variables_initializer())
+    saver = ops.train.Saver()
+    history = []
+    n_train, n_test = len(train["user"]), len(test["user"])
+    with ops.Session() as sess:
+        sess.run(init_op)
+        engine = ops.session.current_model().engine
+        writer = summary.FileWriter(args.logdir) if getattr(args, "logdir", None) else None
+        data = engine.als_data(train["user"], train["item"], train["outcome"])
+        topk = int(getattr(args, "topk", 0) or 0)
+        if topk:
+            topk_exclude = engine.pair_csr(train["user"], train["item"])
+        log("{} {} {} {}".format("epoch", "train_error", "val_error", "elapsed_time"))
+        start = time.time()
+        for epoch in range(args.epochs):
+            failed = engine.als_sweep(data, reg=args.reg)
+            train_rmse = engine.training_objective(data, reg=args.reg)["rmse"]
+            n_failed = int(failed.item())
+            if n_failed:
+                log("ALS: %d rows kept their previous values (a pivot was not > 0)" % n_failed)
+            test_se = []
+            for test_users, test_items, test_rates, test_wins, test_fails in dataio.OneEpochIterator(
+                    [test[c] for c in ("user", "item", "outcome", "wins", "fails")], batch_size=-1):
+                _, test_infer = sess.run([logits, infer], feed_dict={
+                    user_batch: test_users, item_batch: test_items, wins_batch: test_wins, fails_batch: test_fails})
+                test_se.append(np.power(test_rates - test_infer, 2))
+            end = time.time()
+            test_rmse = float(np.sqrt(np.mean(test_se)))
+            rec = dict(epoch=epoch, train_rmse=train_rmse, test_rmse=test_rmse, elapsed=end - start)
+            log("{:3d} TRAIN(size={:d}/{:d}, rmse={:f}) TEST(size={:d}, rmse={:f}) {:f}(s)".format(
+                epoch, n_train, n_train, train_rmse, n_test, test_rmse, end - start))
+            if topk:
+                t_topk = time.time()
+                rm = engine.ranking_metrics(topk, test["user"], test["item"], rates=test["outcome"],
+                                            min_rating=float(args.topk_min_rating), exclude=topk_exclude)
+                rec["topk"] = rm
+                log("TOPK(k={:d}, users={:d}, hr={:f}, precision={:f}, recall={:f}, ndcg={:f})".format(
+                    topk, rm["n_users"], rm["hr"], rm["precision"], rm["recall"], rm["ndcg"]))
+                end += time.time() - t_topk
+            history.append(rec)
+            if writer is not None:
+                writer.add_summary(summary.make_scalar_summary("training_error", train_rmse), epoch)
+                writer.add_summary(summary.make_scalar_summary("test_error", test_rmse), epoch)
+                if topk:
+                    for tag, key in (("hr_at_k", "hr"), ("precision_at_k", "precision"), ("recall_at_k", "recall"),
+                                     ("ndcg_at_k", "ndcg")):
+                        writer.add_summary(summary.make_scalar_summary(tag, rec["topk"][key]), epoch)
+                writer.flush()
+            start = end
+        if writer is not None:
+            writer.close()
+        if args.checkpoint:
+            path = os.path.join(config.BASE_DIR, args.checkpoint)
+            log(path)
+            saver.save(sess, path)
+    return history
+
+
 def load(args):
     if args.dataset:
         df_train, df_val, df_test = dataio.get_data(args.dataset)
@@ -248,14 +324,18 @@ def main(argv=None):
     ap.add_argument("--synthetic", type=str, default="ml1m", choices=sorted(synthetic.SHAPES))
     ap.add_argument("--ratings", type=int, default=None, help="override the number of synthetic ratings")
     ap.add_argument("--variant", type=str, default=config.MODEL_VARIANT, choices=["readme", "fork"])
-    ap.add_argument("--epochs", type=int, default=config.EPOCH_MAX)
-    ap.add_argument("--batch", type=int, default=config.BATCH_SIZE)
+    ap.add_argument("--solver", type=str, default="adam", choices=["adam", "als"],
+                    help="adam: the reference's optimizer steps (default); als: exact alternating least squares sweeps "
+                         "on the device, README variant only, dim <= 128")
+    ap.add_argument("--epochs", type=int, default=config.EPOCH_MAX, help="epochs (with --solver als: sweeps)")
+    ap.add_argument("--batch", type=int, default=config.BATCH_SIZE, help="batch size (not used by --solver als)")
     ap.add_argument("--dim", type=int, default=config.DIM)
-    ap.add_argument("--lr", type=float, default=config.LEARNING_RATE)
+    ap.add_argument("--lr", type=float, default=config.LEARNING_RATE, help="learning rate (not used by --solver als)")
     ap.add_argument("--reg", type=float, default=config.LAMBDA_REG)
     ap.add_argument("--user-num", dest="user_num", type=int, default=None)
     ap.add_argument("--item-num", dest="item_num", type=int, default=None)
-    ap.add_argument("--mode", type=str, default="session", choices=["session", "stream"])
+    ap.add_argument("--mode", type=str, default="session", choices=["session", "stream"],
+                    help="step loop of --solver adam (not used by --solver als)")
     ap.add_argument("--checkpoint", type=str, default="fm.ckpt")
     ap.add_argument("--logdir", type=str, default="/tmp/svd/log",
                     help="TensorBoard event files (svd_train_val.py:57); empty string = none")
@@ -267,9 +347,12 @@ def main(argv=None):
     ap.add_argument("--topk-min-rating", dest="topk_min_rating", type=float, default=4.0,
                     help="README variant: the validation ratings that count as relevant for --topk")
     args = ap.parse_args(argv)
+    if args.solver == "als" and args.variant == "fork":
+        ap.error("--solver als solves the squared-error README model; --variant fork (sigmoid cross-entropy, |q_i|) "
+                 "is not supported")
     np.random.seed(config.SEED)  # svd_train_val.py:15
     train, val = load(args)
-    svd(train, val, args)
+    (svd_als if args.solver == "als" else svd)(train, val, args)
     print("Done!")
 
 

@@ -158,6 +158,13 @@ _PROTOS = {
     "tfr_rank_users_workspace_bytes": (i64, [i64, i64, i32]),
     "tfr_rank_users": (C.c_int, [vp, vp, vp, vp, vp, i64, i64, i32, i64, i64, i32, vp, i64, i32, vp, vp, vp, vp, vp, i64, vp]),
     "tfr_fold_in_users": (C.c_int, [vp, vp, vp, i64, i32, i64, i32, f32, vp, vp, vp, i64, vp, vp, vp, vp]),
+    "tfr_als_chunk": (i32, []),
+    "tfr_als_workspace_bytes": (i64, [i64, i32]),
+    "tfr_als_half_sweep": (C.c_int, [vp, vp, vp, i64, i32, i64, i32, i32, f32, vp, vp, vp, vp, i64, vp, vp, i64, vp, i64, i32,
+                                     vp, i64, vp, vp, vp, i64, vp]),
+    "tfr_svd_objective_workspace_bytes": (i64, [i64, i64]),
+    "tfr_svd_objective": (C.c_int, [vp, vp, vp, vp, vp, i64, i64, i32, i64, i64, i32, f32, vp, vp, vp, vp, vp, vp, vp, i64,
+                                    vp]),
     "tfr_ranking_metrics_workspace_bytes": (i64, [i64, i32]),
     "tfr_ranking_metrics": (C.c_int, [vp, i64, i32, vp, vp, vp, vp, vp, i64, vp]),
     "tfr_host_pack_feed": (C.c_int, [vp, i32, i64, vp, i32, i64, vp, i32, i64, i64, vp]),
@@ -201,7 +208,8 @@ def check(rc):
 
 def tune_set(name, value):
     """Process-wide tuning knob (tfr_tune_set).  Most knobs change launch geometry only and keep results bit for bit;
-    SEG_TILE and SEG_MAX_UNITS change the fp32 rounding of the training step (within the oracle's 1e-5 bar);
+    SEG_TILE and SEG_MAX_UNITS change the fp32 rounding of the training step (within the oracle's 1e-5 bar); ALS_CHUNK
+    changes the float64 summation order of the ALS half-sweep's heavy rows (parity with the exact solution, not bits);
     STREAM_COPY_ONLY, RING_SLOT_MODE=3, AP_STAGES and RANK_STAGES are debug knobs that change results on purpose
     (include/tfrecomm.h lists them all)."""
     check(load().tfr_tune_set(name.encode(), int(value)))

@@ -49,6 +49,10 @@ const TuneEntry kTune[TUNE_COUNT] = {
     {"PDL", 0},
     {"SORT_SPLIT", 0},
     {"RANK_CHUNK", 4096}, {"RANK_STAGES", 7},
+    // ALS item half-sweep at the ML-25M shape, d = 128 (NVIDIA B200, 1000 W, profiles/r06_als_ml25m.json): 112.3 / 111.1 /
+    // 111.1 / 112.6 / 121.4 ms at 1024 / 2048 / 4096 / 8192 / 16384 ratings per chunk; 4096 ties the fastest with a 224 MB
+    // workspace (2048: 491 MB)
+    {"ALS_CHUNK", 4096},
 };
 std::mutex g_tune_mu;
 int g_tune_val[TUNE_COUNT];

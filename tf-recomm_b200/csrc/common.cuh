@@ -31,6 +31,7 @@ enum TuneKey {
   TUNE_SORT_SPLIT,        // 1: every id sort in its one-launch-per-phase form (default: only inside the feed graph)
   TUNE_RANK_CHUNK,        // tfr_rank_users: items per selection chunk (a multiple of 1024, 1024 .. 16384)
   TUNE_RANK_STAGES,       // debug: which kernels of tfr_rank_users run (1 score | 2 select | 4 merge)
+  TUNE_ALS_CHUNK,         // ALS half-sweeps: ratings per Gram chunk of a heavy row (tfr_als_chunk: a multiple of 32)
   TUNE_COUNT
 };
 int tune(TuneKey k);

@@ -39,6 +39,39 @@ class FoldedUsers(NamedTuple):
     info: torch.Tensor
 
 
+class RatingCSR(NamedTuple):
+    """Ratings as CSR on the device: indptr int64 [rows + 1], partner int32 (the other side's id, ascending inside a row,
+    duplicates kept in a stable order), rates float32."""
+    indptr: torch.Tensor
+    partner: torch.Tensor
+    rates: torch.Tensor
+
+
+class AlsPlan(NamedTuple):
+    """The rows of one side of an ALS half-sweep (tfr_als_half_sweep), on the device: light int32 (rows with <= chunk
+    ratings, one CTA each), heavy int32 (rows with more), heavy_ptr int64 [n_heavy + 1] (heavy row h owns chunks
+    heavy_ptr[h] .. heavy_ptr[h + 1]), chunk_heavy int32 [n_chunks] (the heavy row of each chunk)."""
+    light: torch.Tensor
+    heavy: torch.Tensor
+    heavy_ptr: torch.Tensor
+    chunk_heavy: torch.Tensor
+
+
+class AlsData(NamedTuple):
+    """A training set prepared for SvdEngine.als_sweep / training_objective (SvdEngine.als_data), built once on the device:
+    by_user / by_item the ratings as CSR by user and by item; user_plan / item_plan the row lists of each half-sweep; chunk
+    the ALS_CHUNK the plans were built with; workspace, failed (int32 [1]: rows of the last sweep that kept their previous
+    values) and objective (float64 [6]) the buffers the calls use, so that a sweep allocates nothing."""
+    by_user: RatingCSR
+    by_item: RatingCSR
+    user_plan: AlsPlan
+    item_plan: AlsPlan
+    chunk: int
+    workspace: torch.Tensor
+    failed: torch.Tensor
+    objective: torch.Tensor
+
+
 def _require_cuda():
     if not torch.cuda.is_available():
         raise TfrError("tf-recomm_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback for this path")
@@ -395,6 +428,108 @@ class SvdEngine:
         n = int(folded.feat.shape[0])
         q = torch.arange(n, dtype=torch.int32, device=self.device)
         return self._rank_rows(folded.feat, folded.bias, n, 0, q, k, folded.ratings if exclude_rated else None)
+
+    # ---- alternating least squares: exact half-sweeps of the training loss (tfr_als_half_sweep) ---------------------------
+    def _als_refuse(self, reg=None):
+        """TfrError unless the engine's model (and reg, when given) can take an ALS sweep; tfr_als_half_sweep refuses the
+        same."""
+        if self.flags & LOSS_SIGMOID_CE:
+            raise TfrError("ALS solves the squared-error objective; the sigmoid cross-entropy model is not supported")
+        if self.flags & ABS_ITEM:
+            raise TfrError("ALS needs a model quadratic in item_feat; ABS_ITEM scores by |q_i| and is not supported")
+        if self.var_mask != VAR_ALL:
+            raise TfrError("ALS solves every variable; var_mask %#x is not supported" % self.var_mask)
+        if self.d > 128:
+            raise TfrError("ALS supports dim <= 128, got %d" % self.d)
+        if reg is not None and not (reg > 0.0 and np.isfinite(reg)):
+            raise TfrError("ALS needs reg > 0 and finite (every system is then SPD), got %r" % reg)
+
+    def _als_plan(self, indptr, chunk):
+        cnt = indptr[1:] - indptr[:-1]
+        heavy_m = cnt > chunk
+        light = torch.nonzero(~heavy_m).flatten().to(torch.int32)
+        heavy = torch.nonzero(heavy_m).flatten()
+        n_chunk = (cnt[heavy] + chunk - 1) // chunk
+        heavy_ptr = torch.zeros(heavy.numel() + 1, dtype=torch.int64, device=self.device)
+        heavy_ptr[1:] = torch.cumsum(n_chunk, 0)
+        chunk_heavy = torch.repeat_interleave(torch.arange(heavy.numel(), dtype=torch.int32, device=self.device), n_chunk)
+        return AlsPlan(light, heavy.to(torch.int32), heavy_ptr, chunk_heavy)
+
+    def als_data(self, users, items, rates):
+        """A training set (one rating per entry, duplicates count; host or device arrays) prepared for als_sweep and
+        training_objective: both CSRs and the plan of each half-sweep, built once on the device.  The heavy-row threshold is
+        the ALS_CHUNK knob (tfr_als_chunk) as it is now; the plan keeps it."""
+        self._als_refuse()
+        sizes = [a.numel() if isinstance(a, torch.Tensor) else np.asarray(a).size for a in (users, items, rates)]
+        if len(set(sizes)) != 1:
+            raise TfrError("als_data: users, items and rates differ in length: %s" % sizes)
+        self._check_ids(users, items)
+        u, i = self._dev_i32(users).to(torch.int64), self._dev_i32(items).to(torch.int64)
+        r = self._dev_f32(rates)
+        by = {}
+        for name, rows, cols, n_rows, n_cols in (("user", u, i, self.U, self.I), ("item", i, u, self.I, self.U)):
+            order = torch.argsort(rows * n_cols + cols, stable=True)
+            indptr = torch.zeros(n_rows + 1, dtype=torch.int64, device=self.device)
+            indptr[1:] = torch.cumsum(torch.bincount(rows, minlength=n_rows), 0)
+            by[name] = RatingCSR(indptr, cols[order].to(torch.int32).contiguous(), r[order].contiguous())
+        chunk = int(self.L.tfr_als_chunk())
+        up, ip = self._als_plan(by["user"].indptr, chunk), self._als_plan(by["item"].indptr, chunk)
+        nbytes = max(check(self.L.tfr_als_workspace_bytes(p.chunk_heavy.numel(), self.d)) for p in (up, ip))
+        nbytes = max(nbytes, check(self.L.tfr_svd_objective_workspace_bytes(self.U, self.I)))
+        dev = self.device
+        return AlsData(by["user"], by["item"], up, ip, chunk, torch.empty(nbytes, dtype=torch.uint8, device=dev),
+                       torch.zeros(1, dtype=torch.int32, device=dev), torch.zeros(6, dtype=torch.float64, device=dev))
+
+    def _half_sweep(self, data, reg, csr, plan, fixed, solved):
+        (ff, fb, n_fixed), (of, ob) = fixed, solved
+        check(self.L.tfr_als_half_sweep(
+            ff.data_ptr(), fb.data_ptr(), self.t["mu"].data_ptr(), n_fixed, self.d, self.feat_stride, self.flags,
+            self.var_mask, reg, csr.indptr.data_ptr(), csr.partner.data_ptr(), csr.rates.data_ptr(), plan.light.data_ptr(),
+            plan.light.numel(), plan.heavy.data_ptr(), plan.heavy_ptr.data_ptr(), plan.heavy.numel(),
+            plan.chunk_heavy.data_ptr(), plan.chunk_heavy.numel(), data.chunk, of.data_ptr(), self.feat_stride,
+            ob.data_ptr(), data.failed.data_ptr(), data.workspace.data_ptr(), data.workspace.numel(), self._stream()))
+
+    def _objective(self, data, reg, mu_out):
+        T = self.t
+        check(self.L.tfr_svd_objective(
+            T["user_feat"].data_ptr(), T["user_bias"].data_ptr(), T["item_feat"].data_ptr(), T["item_bias"].data_ptr(),
+            T["mu"].data_ptr(), self.U, self.I, self.d, self.feat_stride, self.feat_stride, self.flags, reg,
+            data.by_user.indptr.data_ptr(), data.by_user.partner.data_ptr(), data.by_user.rates.data_ptr(),
+            data.by_item.indptr.data_ptr(), data.objective.data_ptr(), mu_out, data.workspace.data_ptr(),
+            data.workspace.numel(), self._stream()))
+
+    def als_sweep(self, data, reg=None):
+        """One sweep of alternating least squares over the training set `data` (als_data), on the current stream, with no
+        host synchronisation (it can be captured in a CUDA graph): every user row (p_u, b_u) solved exactly against the
+        item side, then every item row against the new user rows, then mu <- mu + mean residual -- three exact block
+        minimisations of the training loss (include/tfrecomm.h, tfr_als_half_sweep).  reg defaults to the engine's.  The
+        Adam slots, the slot maps and the optimizer scalars (global_step included) are left as they were, so Adam training
+        can continue from the result.  -> data.failed, a device int32 [1]: rows of this sweep that kept their previous
+        values because a pivot was not > 0 (0 unless something is badly wrong)."""
+        reg = self.hyper["reg"] if reg is None else float(reg)
+        self._als_refuse(reg)
+        T = self.t
+        with torch.cuda.device(self.device):
+            data.failed.zero_()
+            self._half_sweep(data, reg, data.by_user, data.user_plan, (T["item_feat"], T["item_bias"], self.I),
+                             (T["user_feat"], T["user_bias"]))
+            self._half_sweep(data, reg, data.by_item, data.item_plan, (T["user_feat"], T["user_bias"], self.U),
+                             (T["item_feat"], T["item_bias"]))
+            self._objective(data, reg, T["mu"].data_ptr())
+        return data.failed
+
+    def training_objective(self, data, reg=None):
+        """The training loss of the current tables over `data` (als_data), in float64 on the device:
+        -> dict(loss, rmse, n), loss = sum of 1/2 e^2 + 1/2 reg |p_u|^2 + 1/2 reg |q_i|^2 (+ the bias terms with REG_BIAS)
+        over every occurrence, rmse = sqrt(mean e^2), n = number of occurrences."""
+        reg = self.hyper["reg"] if reg is None else float(reg)
+        if self.flags & LOSS_SIGMOID_CE:
+            raise TfrError("training_objective is the squared-error loss; the sigmoid cross-entropy model is not supported")
+        with torch.cuda.device(self.device):
+            self._objective(data, reg, None)
+        o = data.objective.cpu().numpy()
+        n = int(round(o[5]))
+        return dict(loss=float(o[0]), rmse=float(np.sqrt(o[1] / n)) if n else float("nan"), n=n)
 
     def _csr_by_user(self, users, items, rates=None, dedup=False, n_rows=None):
         """(user, item[, rate]) pairs -> CSR by user, item ids ascending inside a user: (indptr int64 [U + 1], items int32,
