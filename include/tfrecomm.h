@@ -343,7 +343,8 @@ int tfr_svd_train_step_gathered(const tfr_svd_tables* t, tfr_opt_scalars* opt, c
 
 /* ---- FM forward: replaces forward.py:21-22 `fma` ---------------------------------------------
  * yhat[r] = w0 + sum_i W_i x_i + 0.5 * sum_f ((sum_i V_if x_i)^2 - sum_i V_if^2 x_i^2) on CSR rows
- * (indptr int64 [n+1], indices int32, data fp32).  sums (optional) receives sum_i V_if x_i [n,dim]. */
+ * (indptr int64 [n+1], indices int32, data fp32).  sums (optional) receives sum_i V_if x_i [n,dim].
+ * dim is 1..512; any other dim is TFR_ERR_INVALID. */
 int tfr_fm_forward(int64_t n_rows, const int64_t* indptr, const int32_t* indices, const float* data,
                    const float* w0, const float* W, const float* V, int32_t dim, float* yhat, float* sums,
                    void* stream);
@@ -355,7 +356,8 @@ int tfr_fm_forward(int64_t n_rows, const int64_t* indptr, const int32_t* indices
  * (fm.py:104-110,154-155: external binary, out of scope); this is the step north_star asks for instead.
  * indptr[0] must be 0 (a batch is its own CSR matrix).  Caller-allocated scratch: rowof [nnz] (filled by the step:
  * CSR row of every non-zero), sums [n_rows, dim], err [n_rows]; workspace: tfr_svd_step_workspace_bytes(nnz, dim).
- * yhat comes from the PRE-update tables.  Rows without non-zeros are allowed (yhat = w0). */
+ * yhat comes from the PRE-update tables.  Rows without non-zeros are allowed (yhat = w0).  t->dim is 1..512; any
+ * other dim is TFR_ERR_INVALID before anything is launched. */
 typedef struct {
   int32_t n_feat, dim;
   float *w0, *W, *V;                         /* [1], [n_feat], [n_feat, dim] */

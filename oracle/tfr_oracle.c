@@ -364,26 +364,31 @@ ORC_API int orc_svd_train_step(orc_svd_state *s, const int32_t *users, const int
 ORC_API void orc_fm_forward(int64_t n_rows, const int64_t *indptr, const int32_t *indices, const float *data,
                             const float *w0, const float *W, const float *V, int32_t dim,
                             float *yhat, float *sums) {
-#pragma omp parallel for schedule(static)
-  for (int64_t r = 0; r < n_rows; ++r) {
-    float lin = 0.0f;
-    float s_f[256];
-    float q_f[256];
-    for (int f = 0; f < dim; ++f) { s_f[f] = 0.0f; q_f[f] = 0.0f; }
-    for (int64_t p = indptr[r]; p < indptr[r + 1]; ++p) {
-      const float x = data[p];
-      const float *vr = V + (size_t)indices[p] * dim;
-      lin = lin + W[indices[p]] * x;
-      for (int f = 0; f < dim; ++f) {
-        float t = vr[f] * x;
-        s_f[f] = s_f[f] + t;
-        q_f[f] = q_f[f] + t * t;
+#pragma omp parallel
+  {
+    /* one s_f / q_f pair of dim floats per thread (rows of any dim, not a fixed stack array) */
+    float *s_f = (float *)malloc((size_t)(dim > 0 ? dim : 1) * 2 * sizeof(float));
+    float *q_f = s_f + (dim > 0 ? dim : 1);
+#pragma omp for schedule(static)
+    for (int64_t r = 0; r < n_rows; ++r) {
+      float lin = 0.0f;
+      for (int f = 0; f < dim; ++f) { s_f[f] = 0.0f; q_f[f] = 0.0f; }
+      for (int64_t p = indptr[r]; p < indptr[r + 1]; ++p) {
+        const float x = data[p];
+        const float *vr = V + (size_t)indices[p] * dim;
+        lin = lin + W[indices[p]] * x;
+        for (int f = 0; f < dim; ++f) {
+          float t = vr[f] * x;
+          s_f[f] = s_f[f] + t;
+          q_f[f] = q_f[f] + t * t;
+        }
       }
+      float inter = 0.0f;
+      for (int f = 0; f < dim; ++f) inter = inter + (s_f[f] * s_f[f] - q_f[f]);
+      yhat[r] = (w0[0] + lin) + 0.5f * inter;
+      if (sums) for (int f = 0; f < dim; ++f) sums[(size_t)r * dim + f] = s_f[f];
     }
-    float inter = 0.0f;
-    for (int f = 0; f < dim; ++f) inter = inter + (s_f[f] * s_f[f] - q_f[f]);
-    yhat[r] = (w0[0] + lin) + 0.5f * inter;
-    if (sums) for (int f = 0; f < dim; ++f) sums[(size_t)r * dim + f] = s_f[f];
+    free(s_f);
   }
 }
 

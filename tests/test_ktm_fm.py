@@ -85,16 +85,24 @@ def _fm_problem(rng, F, d, n, max_nnz=5, real_valued=True, min_nnz=1):
     return indptr, indices, data
 
 
-@pytest.mark.parametrize("flags", [oracle.OPT_SGD, oracle.OPT_SGD | oracle.LOSS_SIGMOID_CE,
-                                   oracle.OPT_SGD | oracle.REG_BIAS])
+ORACLE_SGD_FLAGS = [oracle.OPT_SGD, oracle.OPT_SGD | oracle.LOSS_SIGMOID_CE, oracle.OPT_SGD | oracle.REG_BIAS]
+
+
+@pytest.mark.parametrize("flags", ORACLE_SGD_FLAGS)
 def test_fm_oracle_gradients_match_torch_autograd(flags):
     """One SGD step of the oracle == var - lr * autograd(cost), cost = data_loss + reg * sum over NON-ZERO OCCURRENCES
     of l2_loss(gathered V row) (+ gathered W with REG_BIAS): the SVD path's per-occurrence L2 (ops.py:81-89,140)."""
+    _oracle_sgd_step_vs_autograd(flags, 6)
+
+
+def _oracle_sgd_step_vs_autograd(flags, d):
+    """V's entries are drawn with variance 0.09 * 6 / d, so that the interaction term keeps one scale at every dim."""
     rng = np.random.default_rng(5)
-    F, d, n, lr, reg = 30, 6, 40, 0.01, 0.05
+    F, n, lr, reg = 30, 40, 0.01, 0.05
     indptr, indices, data = _fm_problem(rng, F, d, n)
     y = rng.integers(0, 2, n).astype(np.float32)
-    w0, W, V = np.array([0.1], np.float32), rng.normal(0, 0.3, F).astype(np.float32), rng.normal(0, 0.3, (F, d)).astype(np.float32)
+    w0, W = np.array([0.1], np.float32), rng.normal(0, 0.3, F).astype(np.float32)
+    V = rng.normal(0, 0.3 * np.sqrt(6 / d), (F, d)).astype(np.float32)
     orc = oracle.FmOracle(w0, W, V, lr, reg, flags=flags)
     yhat = orc.train_step(indptr, indices, data, y)
     tw0, tW, tV = (torch.tensor(a, dtype=torch.float64, requires_grad=True) for a in (w0, W, V))
@@ -151,12 +159,13 @@ def _assert_close(got, ref, what, rtol=RTOL, max_abs=None):
         assert np.abs(got - ref).max() <= max_abs, what
 
 
-def _fm_pair(F, d, lr, reg, flags, seed=2):
+def _fm_pair(F, d, lr, reg, flags, seed=2, eps=1e-8):
     from tf_recomm_b200.fm_engine import FmEngine
     rng = np.random.default_rng(seed)
     tabs = dict(w0=np.array([0.05], np.float32), W=rng.normal(0, 0.1, F).astype(np.float32),
                 V=rng.normal(0, 0.1, (F, d)).astype(np.float32))
-    return FmEngine(F, d, lr, reg, flags=flags, tables=tabs), oracle.FmOracle(tabs["w0"], tabs["W"], tabs["V"], lr, reg, flags=flags)
+    return (FmEngine(F, d, lr, reg, flags=flags, eps=eps, tables=tabs),
+            oracle.FmOracle(tabs["w0"], tabs["W"], tabs["V"], lr, reg, flags=flags, eps=eps))
 
 
 @pytest.mark.gpu

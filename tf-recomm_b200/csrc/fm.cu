@@ -109,14 +109,27 @@ __global__ void __launch_bounds__(256) fm_err_kernel(const tfr_opt_scalars* __re
 
 using namespace tfr;
 
+// Every (VEC, L, UNITS) fm_forward_kernel is instantiated for: (VEC, L) is row_geom's, UNITS = ceil(dim / VEC / L)
+// rounded up to 1, 2, 4, 8 or 16 (surplus units are masked), so every dim of 1..512 has a member of this list
+// (tests/test_fm_geometry.py mirrors the dispatch).  8 and 16 only occur for rows of 129..511 floats with dim % 4 != 0.
+#define TFR_FM_CASES(X)                                                                     \
+  X(4, 1, 1) X(4, 2, 1) X(4, 4, 1) X(4, 8, 1) X(4, 16, 1) X(4, 32, 1) X(4, 32, 2) X(4, 32, 4) \
+  X(1, 1, 1) X(1, 2, 1) X(1, 4, 1) X(1, 8, 1) X(1, 16, 1) X(1, 32, 1) X(1, 32, 2) X(1, 32, 4) \
+  X(1, 32, 8) X(1, 32, 16)
+
 extern "C" int tfr_fm_forward(int64_t n_rows, const int64_t* indptr, const int32_t* indices, const float* data,
                               const float* w0, const float* W, const float* V, int32_t dim, float* yhat, float* sums,
                               void* stream) {
-  TFR_CHECK_ARG(n_rows >= 0 && dim > 0);
+  TFR_CHECK_ARG(n_rows >= 0);
+  if (dim <= 0 || dim > 512) {
+    set_error("FM dim %d: the FM takes dims of 1 to 512", dim);
+    return TFR_ERR_INVALID;
+  }
   if (n_rows == 0) return TFR_OK;
   TFR_CHECK_ARG(indptr && indices && data && w0 && W && V && yhat);
   const RowGeom g = row_geom(dim);
-  const int units = (dim / g.vec + g.lanes - 1) / g.lanes;
+  const int u = (dim / g.vec + g.lanes - 1) / g.lanes;
+  const int units = u <= 1 ? 1 : u <= 2 ? 2 : u <= 4 ? 4 : u <= 8 ? 8 : 16;
   const int groups_per_cta = 256 / g.lanes;
   const unsigned grid = (unsigned)((n_rows + groups_per_cta - 1) / groups_per_cta);
   cudaStream_t st = (cudaStream_t)stream;
@@ -126,12 +139,9 @@ extern "C" int tfr_fm_forward(int64_t n_rows, const int64_t* indptr, const int32
     TFR_LAUNCH_CHECK();                                                                                        \
     return TFR_OK;                                                                                             \
   }
-  TFR_FM_CASE(4, 1, 1) TFR_FM_CASE(4, 2, 1) TFR_FM_CASE(4, 4, 1) TFR_FM_CASE(4, 8, 1) TFR_FM_CASE(4, 16, 1)
-  TFR_FM_CASE(4, 32, 1) TFR_FM_CASE(4, 32, 2) TFR_FM_CASE(4, 32, 4)
-  TFR_FM_CASE(1, 1, 1) TFR_FM_CASE(1, 2, 1) TFR_FM_CASE(1, 4, 1) TFR_FM_CASE(1, 8, 1) TFR_FM_CASE(1, 16, 1)
-  TFR_FM_CASE(1, 32, 1) TFR_FM_CASE(1, 32, 2) TFR_FM_CASE(1, 32, 4)
+  TFR_FM_CASES(TFR_FM_CASE)
 #undef TFR_FM_CASE
-  set_error("unsupported FM dim %d", dim);
+  set_error("unsupported FM dim %d (vec %d lanes %d units %d)", dim, g.vec, g.lanes, units);
   return TFR_ERR_INVALID;
 }
 
@@ -143,7 +153,11 @@ extern "C" int tfr_fm_train_step(const tfr_fm_tables* t, tfr_opt_scalars* opt, i
                                  const float* y, float* yhat, float* sums, float* err, int32_t flags, void* workspace,
                                  int64_t workspace_bytes, void* stream) {
   TFR_CHECK_ARG(t && opt && n_rows > 0 && nnz > 0 && indptr && indices && data && rowof && y && yhat && sums && err);
-  TFR_CHECK_ARG(t->n_feat > 0 && t->dim > 0 && t->w0 && t->W && t->V && t->slot);
+  TFR_CHECK_ARG(t->n_feat > 0 && t->w0 && t->W && t->V && t->slot);
+  if (t->dim <= 0 || t->dim > 512) {
+    set_error("FM dim %d: the FM takes dims of 1 to 512", t->dim);
+    return TFR_ERR_INVALID;
+  }
   const bool sgd = flags & TFR_OPT_SGD;
   TFR_CHECK_ARG(sgd || (t->m_w0 && t->v_w0 && t->m_W && t->v_W && t->m_V && t->v_V));
   tfr_svd_step_ws ws;
