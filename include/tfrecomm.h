@@ -213,7 +213,8 @@ int tfr_svd_train_step_presorted(const tfr_svd_tables* t, tfr_opt_scalars* opt, 
  * device copy drives the kernels).  side_streams (optional; n_side = 0..1): [0] runs the id sort next to the
  * forward.  Fork/join is by the two caller-owned events fork_join_events[0..1] (cudaEvent_t, created on the step's
  * device, e.g. by tfr_event_create; required when n_side > 0 -- the library keeps no events of its own), so the whole
- * step is still capturable as one graph from `stream`. */
+ * step is still capturable as one graph from `stream`.  With g_* set (row-sharded tables) the step trains with Adam
+ * only: TFR_OPT_SGD is TFR_ERR_INVALID before any CUDA call, here and in tfr_svd_train_step_presorted. */
 int tfr_svd_train_step(const tfr_svd_tables* t, tfr_opt_scalars* opt, const int32_t* users,
                        const int32_t* items, const float* rates, int64_t B, float* logits, float* infer,
                        int32_t flags, int32_t var_mask, void* workspace, int64_t workspace_bytes, void* stream,

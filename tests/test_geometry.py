@@ -210,13 +210,12 @@ def _check_outputs(logits, infer, ref_logits, ref_infer, flags, what):
         np.testing.assert_allclose(infer, ref_infer, rtol=RTOL, atol=1e-6, err_msg=what)
 
 
-def _assert_state(eng, orc, what, e_mass):
+def _assert_state(got, orc, lr, sgd, what, e_mass):
     """test_gpu_parity.assert_state_close, with the slot allowance it gives long runs (a hot row's slots are a ~400-term
     sum in tile order against the oracle's one-after-the-other order), except for the scalar mu.  Its update is one sum
     over the batch, sum_b e_b, which cancels in the fork's loss (e = sigmoid(x) - z, about +-0.5 each): mu is judged
-    against the mass of its terms, lr * sum_b |e_b| accumulated over the steps (e_mass)."""
-    got = eng.get_tables()
-    lr = eng.hyper["lr"]
+    against the mass of its terms, lr * sum_b |e_b| accumulated over the steps (e_mass).  got: the tables and Adam slots
+    as SvdEngine.get_tables() gives them (one engine's, or re-assembled shards); sgd: the model has no slots."""
     for n in TABLE_NAMES:
         ref = getattr(orc, n)
         if n == "mu":
@@ -224,7 +223,7 @@ def _assert_state(eng, orc, what, e_mass):
             assert err <= RTOL * abs(float(ref[0])) + RTOL * lr * e_mass, "%s mu: |error| %.3g" % (what, err)
         else:
             assert_fp32_close(got[n], ref, "%s %s" % (what, n), max_abs=4 * lr + 1e-6)
-        if not eng.sgd:
+        if not sgd:
             for s in ("m_", "v_"):
                 assert_fp32_close(got[s + n], orc.slots[s + n], "%s %s%s" % (what, s, n), rtol=5e-5)
 
@@ -241,7 +240,7 @@ def _run_vs_oracle(d, flags, seed, what):
         x = ref_logits.astype(np.float64)
         e = (1.0 / (1.0 + np.exp(-x)) if flags & _lib.LOSS_SIGMOID_CE else x) - rates
         e_mass += float(np.abs(e).sum())
-        _assert_state(eng, orc, "%s step %d" % (what, s), e_mass)
+        _assert_state(eng.get_tables(), orc, eng.hyper["lr"], eng.sgd, "%s step %d" % (what, s), e_mass)
     assert eng.global_step == 3 and eng.live_slots() == 0
 
 

@@ -237,6 +237,9 @@ static int run_step(const tfr_svd_tables* t, tfr_opt_scalars* opt, const int32_t
   // flags / var_mask repeat what the caller gave tfr_opt_init: the device copy drives the kernels, the
   // host copy selects which launches are issued (var_list: untrained tables get no launch at all).
   const bool sgd = flags & TFR_OPT_SGD;
+  // row-sharded mode trains with Adam only: the SGD slice update takes every run head of the sorted keys for a row,
+  // the "not mine" run (key user_num / item_num) included, one row past the local tables
+  TFR_CHECK_ARG(!(sgd && t->g_user_feat));
   TFR_CHECK_ARG(sgd || (t->m_uf && t->v_uf && t->m_if && t->v_if && t->m_ub && t->v_ub && t->m_ib && t->v_ib &&
                         t->m_mu && t->v_mu));
   tfr_svd_step_ws ws;

@@ -19,16 +19,23 @@ import torch
 import torch.distributed as dist
 
 from . import _lib, sharding
-from ._lib import README_FLAGS, VAR_ALL, OptScalars, SvdTables, check
+from ._lib import OPT_SGD, README_FLAGS, VAR_ALL, OptScalars, SvdTables, check
 from .engine import SvdEngine
 
 
 class ShardedSvdEngine:
     def __init__(self, user_num, item_num, dim, lr, reg, rank, world, flags=README_FLAGS, tables=None, device=None,
                  group=None, device_init_seed=13575):
-        """tables: full (unsharded) numpy tables to inject (tests); None -> each rank draws its shard on device."""
+        """tables: full (unsharded) numpy tables to inject (tests); None -> each rank draws its shard on device.
+        Sharded tables train with Adam only, and every rank must own at least one row of each table."""
         self.rank, self.world, self.group = int(rank), int(world), group
         self.U, self.I, self.d = int(user_num), int(item_num), int(dim)
+        if int(flags) & OPT_SGD:
+            # the SGD slice update would take the "not mine" run for a row, one past the local tables
+            raise ValueError("ShardedSvdEngine trains with Adam only: flags %#x include OPT_SGD" % int(flags))
+        if min(self.U, self.I) < self.world:
+            raise ValueError("ShardedSvdEngine needs at least one row of each table per rank: %d users, %d items, "
+                             "world %d" % (self.U, self.I, self.world))
         self.U_loc = sharding.rows_on_rank(self.U, world, rank)
         self.I_loc = sharding.rows_on_rank(self.I, world, rank)
         local = None
