@@ -511,6 +511,60 @@ int tfr_svd_objective(const float* user_feat, const float* user_bias, const floa
                       const int32_t* user_items, const float* user_rates, const int64_t* item_indptr, double* out6,
                       float* mu_out, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* ---- implicit feedback: confidence-weighted alternating least squares (iALS, Hu, Koren and Volinsky, ICDM 2008) -------
+ * Interactions are pairs (u, i) with a weight w_ui > 0.  Duplicate pairs are merged and their weights summed (the caller's
+ * job: one CSR entry per pair).  The default weight is 1 per occurrence, so w is a count.  Define:
+ *   - preference p_ui = 1 on an interaction and 0 on every other pair;
+ *   - confidence c_ui = 1 + alpha w_ui on an interaction and 1 elsewhere;
+ *   - score s_ui = x_u . y_i, with no biases and no mu.
+ * The loss, summed over all U x I pairs:
+ *   L = sum_(u,i) c_ui (p_ui - s_ui)^2 + lambda (sum_u |x_u|^2 + sum_i |y_i|^2)
+ * With Y fixed, the row of user u solves the following dim x dim system (items are symmetric):
+ *   (Y^T Y + sum_(i in R(u)) alpha w_ui y_i y_i^T + lambda I) x_u = sum_(i in R(u)) (1 + alpha w_ui) y_i
+ * A row with no interactions has x = 0 exactly.  The objective is evaluated without the U x I matrix (o the element-wise
+ * product):
+ *   L = sum_ab (X^T X o Y^T Y)_ab + sum_(u,i) in R [c_ui (1 - s_ui)^2 - s_ui^2] + lambda (tr X^T X + tr Y^T Y)
+ * The regulariser is lambda I (Hu et al.'s form), not ALS's reg * n.  A sweep is: G = tfr_gram_rows(item rows); the user
+ * half-sweep against the items; G = tfr_gram_rows(the new user rows); the item half-sweep against the users.  The sweep
+ * writes 0 into the bias of every row it solves (and the caller 0 into mu), so every ranking call of this header ranks
+ * by x . y exactly.
+ *
+ * tfr_gram_rows: gram_out (device, dim (dim + 1) / 2 doubles) = F^T F of the fp32 rows feat [n_rows] (stride floats
+ * between rows, 0 = dim) as a packed lower triangle, row-major ((a, b), b <= a, at a (a + 1) / 2 + b), in float64.  One CTA
+ * per 1024 rows writes a partial triangle to the workspace (tfr_gram_workspace_bytes(n_rows, dim)); one combine sums the
+ * partials in CTA order.  The bits do not depend on the GPU or the run; no floating-point atomics.  n_rows = 0 gives zeros.
+ * tfr_ials_half_sweep: the plan of tfr_als_half_sweep (light rows one CTA each; heavy rows in chunks of `chunk`
+ * interactions, partials in tfr_ials_workspace_bytes(n_chunks, dim) = 256 + (D (D + 1) / 2 + D) * 8 per chunk, D = dim,
+ * rounded up), over the CSR of the solved side: partner ids and weights [indptr[r] .. indptr[r + 1]).  fixed_gram is
+ * tfr_gram_rows of the fixed side.  Light rows start their float64 triangle from fixed_gram and add alpha w y y^T and
+ * (1 + alpha w) y in CSR order; heavy rows add fixed_gram, then the chunks' partials in chunk order; then lambda on the
+ * diagonal, Cholesky and substitution in shared memory.  The row is written rounded to fp32 to out_feat + r * out_stride
+ * (the m / v rows of an interleaved table are never touched) and 0 to out_bias[r] (out_bias nullable).  A pivot that is
+ * not > 0 or a partner id outside [0, n_fixed) leaves the row as it was and adds 1 to *n_failed (device int32, never reset
+ * here).  Asynchronous, no host synchronisation, capturable in a CUDA graph; n_light = n_heavy = 0 is a no-op.
+ * tfr_ials_objective: out5 (device, 5 doubles) = (L, observed part sum_R [c (1 - s)^2 - s^2], all-pairs part
+ * sum_ab (Gx o Gy)_ab, penalty lambda (tr Gx + tr Gy), number of interactions), from the user CSR (items, weights), the
+ * fp32 tables (s in float64) and the two Grams of tfr_gram_rows.  Fixed-order reduction, no floating-point atomics: the same
+ * bits every run.  workspace: tfr_ials_objective_workspace_bytes(n_users).
+ * All four calls: TFR_ERR_INVALID before any CUDA call for dim outside [1, 128], lambda <= 0, NaN or infinite, alpha < 0,
+ * NaN or infinite, a stride below dim and null pointers; TFR_ERR_WORKSPACE for a workspace below the size above. */
+int64_t tfr_gram_workspace_bytes(int64_t n_rows, int32_t dim);
+int tfr_gram_rows(const float* feat, int64_t n_rows, int32_t dim, int64_t stride /* 0 = dim */, double* gram_out,
+                  void* workspace, int64_t workspace_bytes, void* stream);
+int64_t tfr_ials_workspace_bytes(int64_t n_chunks, int32_t dim);
+int tfr_ials_half_sweep(const float* fixed_feat, int64_t n_fixed, int32_t dim, int64_t fixed_stride /* 0 = dim */,
+                        const double* fixed_gram, float alpha, float reg, const int64_t* indptr, const int32_t* partner,
+                        const float* weight, const int32_t* light_rows, int64_t n_light, const int32_t* heavy_rows,
+                        const int64_t* heavy_ptr, int64_t n_heavy, const int32_t* chunk_heavy, int64_t n_chunks,
+                        int32_t chunk, float* out_feat, int64_t out_stride /* 0 = dim */, float* out_bias /* nullable */,
+                        int32_t* n_failed, void* workspace, int64_t workspace_bytes, void* stream);
+int64_t tfr_ials_objective_workspace_bytes(int64_t n_users);
+int tfr_ials_objective(const float* user_feat, const float* item_feat, int64_t n_users, int64_t n_items, int32_t dim,
+                       int64_t user_stride, int64_t item_stride /* 0 = dim */, const double* user_gram,
+                       const double* item_gram, float alpha, float reg, const int64_t* user_indptr,
+                       const int32_t* user_items, const float* user_weight, double* out5, void* workspace,
+                       int64_t workspace_bytes, void* stream);
+
 /* ---- host side of the feed_dict boundary: the columns a reference iterator yields (dataio.py:114-117: float64 views
  * of one [B, ncols] matrix, ids included) packed into a pinned staging buffer in the device's types -- int32 ids
  * (value cast, like TF feeding an int32 placeholder, A.7) followed by float32 rates: [users B | items B | rates B].

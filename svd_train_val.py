@@ -21,6 +21,12 @@ Two ways to run the step loop:
 user row, then each item row, exactly in float64 against the other side, then updates mu; TRAIN is the RMSE over the whole
 training set after the sweep.  --batch, --lr and --mode do not apply to it.
 
+--solver ials trains the same tables from implicit feedback instead (SvdEngine.ials_sweep, Hu, Koren and Volinsky 2008):
+every training pair is an interaction of weight 1 (duplicates add), confidence 1 + --alpha * weight, every other pair a
+0 of confidence 1, --reg the lambda of lambda * I.  Every epoch is one sweep; the IMPLICIT line is the loss over all user x
+item pairs after it.  Biases and mu are 0 after a sweep, so the model ranks by p_u . q_i.  --topk is required (RMSE against
+ratings means nothing for this model); --batch, --lr and --mode do not apply.
+
 --topk K adds, after every report, the top-K recommendation quality on the validation split: each user is ranked over
 the items they did not rate in training, and hit rate / precision / recall / NDCG at K are measured against their
 validation items (rated >= --topk-min-rating; on the DISCRETE branch, an outcome of 1).
@@ -291,6 +297,65 @@ def svd_als(train, test, args, log=print):
     return history
 
 
+def svd_ials(train, test, args, log=print):
+    """--solver ials: the same model, initialisation, --topk lines, summaries and checkpoint as svd(), trained by one iALS
+    sweep per epoch from the training pairs as implicit feedback.  IMPLICIT(...) is the loss after the sweep."""
+    user_batch = ops.placeholder(ops.int32, shape=[None], name="id_user")
+    item_batch = ops.placeholder(ops.int32, shape=[None], name="id_item")
+    rate_batch = ops.placeholder(ops.float32, shape=[None])
+    wins_batch = ops.placeholder(ops.float32, shape=[None], name="nb_wins")
+    fails_batch = ops.placeholder(ops.float32, shape=[None], name="nb_fails")
+    ops.reset_default_graph()
+    infer, logits, regularizer, _, _, _, _ = ops.inference_svd(
+        user_batch, item_batch, wins_batch, fails_batch, user_num=args.user_num, item_num=args.item_num, dim=args.dim,
+        device=config.DEVICE, variant=args.variant)
+    ops.train.get_or_create_global_step()
+    ops.optimization(infer, logits, regularizer, rate_batch, learning_rate=args.lr, reg=args.reg, device=config.DEVICE)
+    init_op = ops.group(ops.global_variables_initializer(), ops.local_variables_initializer())
+    saver = ops.train.Saver()
+    history = []
+    with ops.Session() as sess:
+        sess.run(init_op)
+        engine = ops.session.current_model().engine
+        writer = summary.FileWriter(args.logdir) if getattr(args, "logdir", None) else None
+        data = engine.ials_data(train["user"], train["item"])
+        topk_exclude = engine.pair_csr(train["user"], train["item"])
+        log("{} {} {}".format("epoch", "implicit_loss", "elapsed_time"))
+        start = time.time()
+        for epoch in range(args.epochs):
+            failed = engine.ials_sweep(data, args.alpha, reg=args.reg)
+            obj = engine.implicit_objective(data, args.alpha, reg=args.reg)
+            n_failed = int(failed.item())
+            if n_failed:
+                log("iALS: %d rows kept their previous values (a pivot was not > 0)" % n_failed)
+            end = time.time()
+            rec = dict(epoch=epoch, implicit_loss=obj["loss"], elapsed=end - start)
+            log("{:3d} IMPLICIT(pairs={:d}, loss={:.10g}, observed={:.10g}, all_pairs={:.10g}, penalty={:.10g}) {:f}(s)"
+                .format(epoch, obj["n"], obj["loss"], obj["observed"], obj["all_pairs"], obj["penalty"], end - start))
+            t_topk = time.time()
+            rm = engine.ranking_metrics(args.topk, test["user"], test["item"], rates=test["outcome"],
+                                        min_rating=float(args.topk_min_rating), exclude=topk_exclude)
+            rec["topk"] = rm
+            log("TOPK(k={:d}, users={:d}, hr={:f}, precision={:f}, recall={:f}, ndcg={:f})".format(
+                args.topk, rm["n_users"], rm["hr"], rm["precision"], rm["recall"], rm["ndcg"]))
+            end += time.time() - t_topk
+            history.append(rec)
+            if writer is not None:
+                writer.add_summary(summary.make_scalar_summary("implicit_loss", obj["loss"]), epoch)
+                for tag, key in (("hr_at_k", "hr"), ("precision_at_k", "precision"), ("recall_at_k", "recall"),
+                                 ("ndcg_at_k", "ndcg")):
+                    writer.add_summary(summary.make_scalar_summary(tag, rm[key]), epoch)
+                writer.flush()
+            start = end
+        if writer is not None:
+            writer.close()
+        if args.checkpoint:
+            path = os.path.join(config.BASE_DIR, args.checkpoint)
+            log(path)
+            saver.save(sess, path)
+    return history
+
+
 def load(args):
     if args.dataset:
         df_train, df_val, df_test = dataio.get_data(args.dataset)
@@ -324,9 +389,12 @@ def main(argv=None):
     ap.add_argument("--synthetic", type=str, default="ml1m", choices=sorted(synthetic.SHAPES))
     ap.add_argument("--ratings", type=int, default=None, help="override the number of synthetic ratings")
     ap.add_argument("--variant", type=str, default=config.MODEL_VARIANT, choices=["readme", "fork"])
-    ap.add_argument("--solver", type=str, default="adam", choices=["adam", "als"],
+    ap.add_argument("--solver", type=str, default="adam", choices=["adam", "als", "ials"],
                     help="adam: the reference's optimizer steps (default); als: exact alternating least squares sweeps "
-                         "on the device, README variant only, dim <= 128")
+                         "on the device, README variant only, dim <= 128; ials: implicit-feedback ALS sweeps (the "
+                         "training pairs as interactions), README variant only, dim <= 128, needs --topk")
+    ap.add_argument("--alpha", type=float, default=1.0,
+                    help="--solver ials: confidence 1 + alpha * weight of an interaction (>= 0)")
     ap.add_argument("--epochs", type=int, default=config.EPOCH_MAX, help="epochs (with --solver als: sweeps)")
     ap.add_argument("--batch", type=int, default=config.BATCH_SIZE, help="batch size (not used by --solver als)")
     ap.add_argument("--dim", type=int, default=config.DIM)
@@ -350,9 +418,17 @@ def main(argv=None):
     if args.solver == "als" and args.variant == "fork":
         ap.error("--solver als solves the squared-error README model; --variant fork (sigmoid cross-entropy, |q_i|) "
                  "is not supported")
+    if args.solver == "ials":
+        if args.variant == "fork":
+            ap.error("--solver ials trains the README model's p_u . q_i; --variant fork (sigmoid cross-entropy, |q_i|) "
+                     "is not supported")
+        if args.topk <= 0:
+            ap.error("--solver ials needs --topk K: the model ranks items, and RMSE against ratings means nothing for it")
+        if not (args.alpha >= 0.0 and np.isfinite(args.alpha)):
+            ap.error("--alpha must be >= 0 and finite")
     np.random.seed(config.SEED)  # svd_train_val.py:15
     train, val = load(args)
-    (svd_als if args.solver == "als" else svd)(train, val, args)
+    dict(adam=svd, als=svd_als, ials=svd_ials)[args.solver](train, val, args)
     print("Done!")
 
 

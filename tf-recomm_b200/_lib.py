@@ -165,6 +165,13 @@ _PROTOS = {
     "tfr_svd_objective_workspace_bytes": (i64, [i64, i64]),
     "tfr_svd_objective": (C.c_int, [vp, vp, vp, vp, vp, i64, i64, i32, i64, i64, i32, f32, vp, vp, vp, vp, vp, vp, vp, i64,
                                     vp]),
+    "tfr_gram_workspace_bytes": (i64, [i64, i32]),
+    "tfr_gram_rows": (C.c_int, [vp, i64, i32, i64, vp, vp, i64, vp]),
+    "tfr_ials_workspace_bytes": (i64, [i64, i32]),
+    "tfr_ials_half_sweep": (C.c_int, [vp, i64, i32, i64, vp, f32, f32, vp, vp, vp, vp, i64, vp, vp, i64, vp, i64, i32, vp, i64,
+                                      vp, vp, vp, i64, vp]),
+    "tfr_ials_objective_workspace_bytes": (i64, [i64]),
+    "tfr_ials_objective": (C.c_int, [vp, vp, i64, i64, i32, i64, i64, vp, vp, f32, f32, vp, vp, vp, vp, vp, i64, vp]),
     "tfr_ranking_metrics_workspace_bytes": (i64, [i64, i32]),
     "tfr_ranking_metrics": (C.c_int, [vp, i64, i32, vp, vp, vp, vp, vp, i64, vp]),
     "tfr_host_pack_feed": (C.c_int, [vp, i32, i64, vp, i32, i64, vp, i32, i64, i64, vp]),

@@ -72,6 +72,32 @@ class AlsData(NamedTuple):
     objective: torch.Tensor
 
 
+class InteractionCSR(NamedTuple):
+    """Weighted interactions as CSR on the device: indptr int64 [rows + 1], partner int32 (the other side's id, ascending and
+    distinct inside a row), weight float32 (> 0, the merged pair's summed weight)."""
+    indptr: torch.Tensor
+    partner: torch.Tensor
+    weight: torch.Tensor
+
+
+class IalsData(NamedTuple):
+    """Implicit feedback prepared for SvdEngine.ials_sweep / implicit_objective (SvdEngine.ials_data), built once on the
+    device: by_user / by_item the merged interactions as CSR by user and by item; user_plan / item_plan the row lists of each
+    half-sweep (AlsPlan); chunk the ALS_CHUNK the plans were built with; user_gram / item_gram float64 [d (d + 1) / 2] the
+    packed Grams X^T X / Y^T Y; workspace, failed (int32 [1]: rows of the last sweep that kept their previous values) and
+    objective (float64 [5]) the buffers the calls use, so that a sweep allocates nothing."""
+    by_user: InteractionCSR
+    by_item: InteractionCSR
+    user_plan: AlsPlan
+    item_plan: AlsPlan
+    chunk: int
+    user_gram: torch.Tensor
+    item_gram: torch.Tensor
+    workspace: torch.Tensor
+    failed: torch.Tensor
+    objective: torch.Tensor
+
+
 def _require_cuda():
     if not torch.cuda.is_available():
         raise TfrError("tf-recomm_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback for this path")
@@ -530,6 +556,144 @@ class SvdEngine:
         o = data.objective.cpu().numpy()
         n = int(round(o[5]))
         return dict(loss=float(o[0]), rmse=float(np.sqrt(o[1] / n)) if n else float("nan"), n=n)
+
+    # ---- implicit feedback: confidence-weighted ALS (iALS) on the device (tfr_ials_half_sweep) --------------------------------
+    def _merge_interactions(self, rows, items, weights, n_rows, name):
+        """(row, item[, weight]) entries -> the distinct pairs sorted by (row, item): (row int64, item int64, weight float32),
+        each pair's weight the sum of its entries' weights (1 each by default), summed in float64 in the entries' order
+        (torch.segment_reduce: one sequential sum per pair, so the same entries give the same bits)."""
+        sizes = [a.numel() if isinstance(a, torch.Tensor) else np.asarray(a).size
+                 for a in ((rows, items) if weights is None else (rows, items, weights))]
+        if len(set(sizes)) != 1:
+            raise TfrError("%s: rows, items and weights differ in length: %s" % (name, sizes))
+        self._check_ids(rows, items, n_rows)
+        r, i = self._dev_i32(rows).to(torch.int64), self._dev_i32(items).to(torch.int64)
+        w = torch.ones(r.numel(), dtype=torch.float32, device=self.device) if weights is None else self._dev_f32(weights)
+        key, order = torch.sort(r * self.I + i, stable=True)
+        key, counts = torch.unique_consecutive(key, return_counts=True)
+        merged = torch.segment_reduce(w[order].double(), "sum", lengths=counts, unsafe=True).float()
+        if weights is not None and not bool(((w > 0) & torch.isfinite(w)).all() & torch.isfinite(merged).all()):
+            raise TfrError("%s: weights must be > 0 and finite, and so must their sums over duplicate pairs" % name)
+        return key // self.I, key % self.I, merged.contiguous()
+
+    def _alpha_reg(self, alpha, reg):
+        reg = self.hyper["reg"] if reg is None else float(reg)
+        self._als_refuse(reg)
+        alpha = float(alpha)
+        if not (alpha >= 0.0 and np.isfinite(alpha)):
+            raise TfrError("iALS needs alpha >= 0 and finite, got %r" % alpha)
+        return alpha, reg
+
+    def ials_data(self, users, items, weights=None):
+        """Implicit feedback (one interaction per entry, weight 1 each unless `weights` is given; host or device arrays)
+        prepared for ials_sweep and implicit_objective: duplicate pairs merged with their weights summed, both CSRs and the
+        plan of each half-sweep, built once on the device.  Weights must be > 0 and finite.  The heavy-row threshold is the
+        ALS_CHUNK knob (tfr_als_chunk) as it is now; the plan keeps it."""
+        self._als_refuse()
+        u, i, w = self._merge_interactions(users, items, weights, self.U, "ials_data")
+        dev = self.device
+        by = {}
+        for name, rows, cols, n_rows, n_cols in (("user", u, i, self.U, self.I), ("item", i, u, self.I, self.U)):
+            order = torch.argsort(rows * n_cols + cols, stable=True) if name == "item" else None
+            indptr = torch.zeros(n_rows + 1, dtype=torch.int64, device=dev)
+            indptr[1:] = torch.cumsum(torch.bincount(rows, minlength=n_rows), 0)
+            cols_s, w_s = (cols, w) if order is None else (cols[order], w[order])
+            by[name] = InteractionCSR(indptr, cols_s.to(torch.int32).contiguous(), w_s.contiguous())
+        chunk = int(self.L.tfr_als_chunk())
+        up, ip = self._als_plan(by["user"].indptr, chunk), self._als_plan(by["item"].indptr, chunk)
+        nbytes = max(check(self.L.tfr_ials_workspace_bytes(p.chunk_heavy.numel(), self.d)) for p in (up, ip))
+        nbytes = max(nbytes, check(self.L.tfr_gram_workspace_bytes(max(self.U, self.I), self.d)),
+                     check(self.L.tfr_ials_objective_workspace_bytes(self.U)))
+        n_tri = self.d * (self.d + 1) // 2
+        return IalsData(by["user"], by["item"], up, ip, chunk, torch.zeros(n_tri, dtype=torch.float64, device=dev),
+                        torch.zeros(n_tri, dtype=torch.float64, device=dev),
+                        torch.empty(nbytes, dtype=torch.uint8, device=dev), torch.zeros(1, dtype=torch.int32, device=dev),
+                        torch.zeros(5, dtype=torch.float64, device=dev))
+
+    def _gram(self, feat, n_rows, gram, ws):
+        check(self.L.tfr_gram_rows(feat.data_ptr(), n_rows, self.d, self.feat_stride, gram.data_ptr(), ws.data_ptr(),
+                                   ws.numel(), self._stream()))
+
+    def _ials_half(self, data, alpha, reg, csr, plan, fixed, solved):
+        (ff, n_fixed, gram), (of, ob) = fixed, solved
+        check(self.L.tfr_ials_half_sweep(
+            ff.data_ptr(), n_fixed, self.d, self.feat_stride, gram.data_ptr(), alpha, reg, csr.indptr.data_ptr(),
+            csr.partner.data_ptr(), csr.weight.data_ptr(), plan.light.data_ptr(), plan.light.numel(),
+            plan.heavy.data_ptr(), plan.heavy_ptr.data_ptr(), plan.heavy.numel(), plan.chunk_heavy.data_ptr(),
+            plan.chunk_heavy.numel(), data.chunk, of.data_ptr(), self.feat_stride, ob.data_ptr() if ob is not None else None,
+            data.failed.data_ptr(), data.workspace.data_ptr(), data.workspace.numel(), self._stream()))
+
+    def ials_sweep(self, data, alpha, reg=None):
+        """One sweep of implicit-feedback ALS (Hu, Koren and Volinsky 2008; include/tfrecomm.h) over `data` (ials_data), on
+        the current stream, with no host synchronisation (it can be captured in a CUDA graph): mu <- 0, G = Y^T Y of the item
+        rows, every user row solved exactly against it, G = X^T X of the new user rows, every item row solved against them.
+        Every solved row's bias is set to 0, so the model scores by x . y alone.  reg (lambda) defaults to the engine's.  The
+        Adam slots, the slot maps and the optimizer scalars are left as they were.  -> data.failed, a device int32 [1]: rows
+        of this sweep that kept their previous values because a pivot was not > 0 (0 unless something is badly wrong)."""
+        alpha, reg = self._alpha_reg(alpha, reg)
+        T = self.t
+        with torch.cuda.device(self.device):
+            data.failed.zero_()
+            T["mu"].zero_()
+            self._gram(T["item_feat"], self.I, data.item_gram, data.workspace)
+            self._ials_half(data, alpha, reg, data.by_user, data.user_plan, (T["item_feat"], self.I, data.item_gram),
+                            (T["user_feat"], T["user_bias"]))
+            self._gram(T["user_feat"], self.U, data.user_gram, data.workspace)
+            self._ials_half(data, alpha, reg, data.by_item, data.item_plan, (T["user_feat"], self.U, data.user_gram),
+                            (T["item_feat"], T["item_bias"]))
+        return data.failed
+
+    def implicit_objective(self, data, alpha, reg=None):
+        """The implicit-feedback loss of the current tables over `data` (ials_data), over all U x I pairs without forming
+        them, in float64 on the device: -> dict(loss, observed, all_pairs, penalty, n), loss = all_pairs + observed + penalty,
+        all_pairs = sum_(u,i) s_ui^2 (from the two Grams), observed = sum over the interactions of c (1 - s)^2 - s^2,
+        penalty = lambda (sum |x_u|^2 + sum |y_i|^2), n = number of (merged) interactions."""
+        alpha, reg = self._alpha_reg(alpha, reg)
+        T = self.t
+        with torch.cuda.device(self.device):
+            self._gram(T["user_feat"], self.U, data.user_gram, data.workspace)
+            self._gram(T["item_feat"], self.I, data.item_gram, data.workspace)
+            check(self.L.tfr_ials_objective(
+                T["user_feat"].data_ptr(), T["item_feat"].data_ptr(), self.U, self.I, self.d, self.feat_stride,
+                self.feat_stride, data.user_gram.data_ptr(), data.item_gram.data_ptr(), alpha, reg,
+                data.by_user.indptr.data_ptr(), data.by_user.partner.data_ptr(), data.by_user.weight.data_ptr(),
+                data.objective.data_ptr(), data.workspace.data_ptr(), data.workspace.numel(), self._stream()))
+        o = data.objective.cpu().numpy()
+        return dict(loss=float(o[0]), observed=float(o[1]), all_pairs=float(o[2]), penalty=float(o[3]), n=int(round(o[4])))
+
+    def fold_in_implicit(self, rows, items, weights=None, n=None, *, alpha, reg=None):
+        """iALS user rows for new users (or new interactions of known ones) against the trained item side: for each row
+        label r in [0, n) the x that minimises the implicit-feedback loss (include/tfrecomm.h) over all items with the item
+        rows fixed, from the interactions (rows == r) -- duplicates merged and weights summed as ials_data does, weight 1 each
+        by default.  The user half-sweep's light-row kernel, one CTA per row whatever its length, against G = Y^T Y computed
+        in the call: a training user folded in from its own interactions gets the half-sweep's bits.  n defaults to
+        max(rows) + 1; reg (lambda) defaults to the engine's.  A row without interactions gets x = 0.  -> FoldedUsers with
+        zero biases (rank it with rank_folded, which then ranks by x . y); info 0, or 1 for a row that could not be solved
+        (NaN)."""
+        alpha, reg = self._alpha_reg(alpha, reg)
+        if n is None:
+            r_ = rows if isinstance(rows, torch.Tensor) else np.asarray(rows)
+            n = int(r_.max()) + 1 if (r_.numel() if isinstance(r_, torch.Tensor) else r_.size) else 0
+        n = int(n)
+        r, it, w = self._merge_interactions(rows, items, weights, n, "fold_in_implicit")
+        dev = self.device
+        indptr = torch.zeros(n + 1, dtype=torch.int64, device=dev)
+        indptr[1:] = torch.cumsum(torch.bincount(r, minlength=n), 0)
+        it = it.to(torch.int32).contiguous()
+        feat = torch.full((n, self.d), float("nan"), dtype=torch.float32, device=dev)
+        bias = torch.zeros(n, dtype=torch.float32, device=dev)
+        gram = torch.empty(self.d * (self.d + 1) // 2, dtype=torch.float64, device=dev)
+        ws = torch.empty(check(self.L.tfr_gram_workspace_bytes(self.I, self.d)), dtype=torch.uint8, device=dev)
+        failed = torch.zeros(1, dtype=torch.int32, device=dev)
+        rows_all = torch.arange(n, dtype=torch.int32, device=dev)
+        with torch.cuda.device(dev):
+            self._gram(self.t["item_feat"], self.I, gram, ws)
+            check(self.L.tfr_ials_half_sweep(
+                self.t["item_feat"].data_ptr(), self.I, self.d, self.feat_stride, gram.data_ptr(), alpha, reg,
+                indptr.data_ptr(), it.data_ptr(), w.data_ptr(), rows_all.data_ptr(), n, None, None, 0, None, 0, 1,
+                feat.data_ptr(), self.d, None, failed.data_ptr(), None, 0, self._stream()))
+        info = torch.isnan(feat[:, 0]).to(torch.int32) if n else torch.zeros(0, dtype=torch.int32, device=dev)
+        return FoldedUsers(feat, bias, PairCSR(indptr, it), info)
 
     def _csr_by_user(self, users, items, rates=None, dedup=False, n_rows=None):
         """(user, item[, rate]) pairs -> CSR by user, item ids ascending inside a user: (indptr int64 [U + 1], items int32,
