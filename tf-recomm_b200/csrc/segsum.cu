@@ -22,57 +22,11 @@
 #include <map>
 #include <mutex>
 
-#include "common.cuh"
+#include "segsum.cuh"
 
 namespace tfr {
 
 constexpr int SEG_TILE_MAX = 32;  // tiles of 32, 16 or 8 sorted entries: tfr::seg_tile(B, dim)
-
-struct SegSide {
-  const int32_t* sid;      // sorted ids of this table
-  const int32_t* spos;     // batch positions
-  const int32_t* partner;  // the OTHER id column of the batch (items for the user table)
-  const float* own_feat;   // this table's rows
-  const float* partner_feat;
-  int64_t own_stride, partner_stride;  // floats between consecutive rows (dim, or 3*dim for interleaved tables)
-  const float* own_bias;
-  const float* partner_bias;  // fused forward only
-  float *gsum, *gsum_b, *cont, *cont_b, *tail, *tail_b;
-  uint8_t* kind;  // per tile: TILE_MID | TILE_START (see segsum_fixup_kernel)
-  int32_t* fix_list;     // work list of the fix-up: the TILE_START tiles, in no particular order
-  uint32_t* fix_count;   // its length (zeroed by the id sort and by the fix-up's last CTA)
-  int64_t* slot;  // [rows] row -> (step stamp << 32 | head index of its run, where its gsum lives)
-  int32_t n_rows; // ids >= n_rows mark occurrences owned by another rank (row-sharded mode): skipped
-  // factorization-machine mode (xval != null): the sorted ids are FEATURE ids of the batch's non-zeros, position =
-  // index p of the non-zero; partner row = sums[rowof[p]] (the CSR row's sum_i V_i x_i), and
-  //   g_V = e_r * (x_p * (sums_r - V_f * x_p)) + reg * V_f        (Rendle 2010 eq. 4; forward.py:21-22's model)
-  //   g_W = e_r * x_p (+ reg * W_f if TFR_REG_BIAS)
-  const float* xval;      // [nnz] feature values
-  const int32_t* rowof;   // [nnz] CSR row of every non-zero
-  int is_item;
-};
-
-// The forward fused into the segment sums (FUSED = true): a tile holds, for every occurrence, the own row and the
-// partner row, i.e. everything ops.py:44-47 needs -- each side recomputes logits = ((sum_k u*v' + mu) + b_u) + b_i
-// and d cost/d logits itself (same operands, same order on both sides: bit-identical e), the user side writes
-// logits / infer and the fixed-order partial sums of e and of the float64 squared error.  No forward kernel, no
-// err array, one launch less in front of the table pass.
-struct FwdArgs {
-  const float* mu;
-  const float* rates;
-  float *logits, *infer;       // by batch position; optional
-  float* partials;             // [gridDim.x] per-CTA sums of e (user side)
-  double* se_partials;
-};
-
-// tile classification written by the tiles kernel, read by the fix-up:
-//   TILE_MID   the whole tile is ONE run that began in an earlier tile and goes on into the next
-//   TILE_START the tile's last run begins here and goes on into the next tile (tail[t] is valid)
-constexpr uint8_t TILE_MID = 1, TILE_START = 2;
-
-__device__ __forceinline__ int64_t pack_slot(uint32_t stamp, int64_t k) {
-  return (int64_t)(((uint64_t)stamp << 32) | (uint32_t)k);
-}
 
 template <int VEC>
 struct Acc {
@@ -124,7 +78,6 @@ __device__ __forceinline__ Acc<VEC> lds_units(const float* row, int unit) {
   return a;
 }
 
-constexpr int SEG_THREADS = 128;  // CTA of the tiles kernel
 #ifndef SEG_PBASE
 #define SEG_PBASE 4
 #endif
@@ -722,7 +675,7 @@ int segsum_grid_x(int dim, int64_t B) {  // CTAs per side = number of per-CTA pa
 
 // the tiles kernel stages rows in dynamic shared memory (32 KB per CTA at dim 128, up to 64 KB): opt in once per
 // instantiation
-static int prep_tiles(const void* fn, size_t smem) {
+int tfr::prep_tiles(const void* fn, size_t smem) {
   static std::mutex mu;
   static std::map<const void*, size_t> done;
   std::lock_guard<std::mutex> lock(mu);
@@ -771,7 +724,9 @@ static int launch_segsum(const SegSide& su, const SegSide& si, int n_sides, cons
   if (g.vec == V && g.lanes == LL && units == UU) {                                                               \
     if (int rc = prep_tiles((const void*)segsum_fixup_kernel<V>, fix_smem)) return rc; /* same carve-out as the tiles */ \
     if (fw && generic) TFR_SEG_LAUNCH(V, LL, UU, true, true)                                                       \
-    else if (fw) TFR_SEG_LAUNCH(V, LL, UU, true, false)                                                            \
+    else if (fw && V == 4 && UU == 4 && chain_tiles_supported(LL, tile)) {                                          \
+      if (int rc = launch_chain_tiles(su, si, *fw, opt, B, dim, n_tiles, tile, LL, grid, pdl, st)) return rc;      \
+    } else if (fw) TFR_SEG_LAUNCH(V, LL, UU, true, false)                                                          \
     else if (generic) TFR_SEG_LAUNCH(V, LL, UU, false, true)                                                       \
     else TFR_SEG_LAUNCH(V, LL, UU, false, false)                                                                   \
     TFR_LAUNCH_CHECK();                                                                                            \
