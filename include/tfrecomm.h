@@ -342,6 +342,34 @@ int tfr_svd_train_step_gathered(const tfr_svd_tables* t, tfr_opt_scalars* opt, c
                                 int64_t n, int32_t flags, int32_t var_mask, const float* sum_err, const double* sum_se,
                                 void* workspace, int64_t workspace_bytes, void* stream);
 
+/* ---- serving from row-sharded tables: exact top-k over items spread over n_ranks ranks (item i on rank i mod n_ranks,
+ * local row i / n_ranks).  Every rank runs tfr_rank_users on its item shard against the same n query rows (gathered by
+ * tfr_shard_gather_rows + an all-reduce: one n-row user table, query j = row j), with k = min(k, items over ALL ranks) so
+ * that every rank's list has the same shape; the caller all-gathers the lists (NCCL) and merges them here.
+ *  tfr_shard_excl_indptr / tfr_shard_excl_fill: the per-rank exclusion lists tfr_rank_users takes.  Source: a CSR over
+ *    n_rows rows (indptr int64 [n_rows + 1], items int32 ascending inside a row, GLOBAL item ids, duplicates allowed), e.g.
+ *    the training pairs by user or fold-in ratings.  Output: a CSR over the n QUERY positions, row q = the items of source
+ *    row rows[q] that this rank owns (item mod n_ranks == rank) as LOCAL ids (item / n_ranks), ascending.  Count -> scan ->
+ *    fill: _indptr writes out_indptr [n + 1] (out_indptr[n] = the total, read back to size out_items), _fill writes
+ *    out_items.  A rows[q] outside [0, n_rows) gives an empty list.  The work is the length of the query rows' source
+ *    lists, whatever n_rows.  items / out_items may be null when there are no entries.  workspace (indptr only):
+ *    tfr_shard_excl_workspace_bytes(n).
+ *  tfr_shard_topk_merge: val (float64) / idx (int32) [n_ranks][n][k], the per-rank lists in the layout an all-gather of
+ *    [n][k] blocks produces; list g of query q is sorted (score descending, local id ascending) and padded with id -1.
+ *    out_val / out_idx [n][k] = the top k of the union under (score descending, GLOBAL id ascending), global id = local
+ *    id * n_ranks + g, missing ranks (-inf, -1): the ranking tfr_rank_users gives on the re-assembled item table, ids
+ *    and bits.  One warp per query.
+ * TFR_ERR_INVALID before any CUDA call unless 1 <= n_ranks <= 8, 0 <= rank < n_ranks, 1 <= k <= 1024, 0 <= n < 2^31,
+ * 0 <= n_rows < 2^31, and the pointers are non-null when n > 0. */
+int64_t tfr_shard_excl_workspace_bytes(int64_t n);
+int tfr_shard_excl_indptr(const int64_t* indptr, const int32_t* items, int64_t n_rows, const int32_t* rows, int64_t n,
+                          int32_t n_ranks, int32_t rank, int64_t* out_indptr, void* workspace, int64_t workspace_bytes,
+                          void* stream);
+int tfr_shard_excl_fill(const int64_t* indptr, const int32_t* items, int64_t n_rows, const int32_t* rows, int64_t n,
+                        int32_t n_ranks, int32_t rank, const int64_t* out_indptr, int32_t* out_items, void* stream);
+int tfr_shard_topk_merge(const double* val, const int32_t* idx, int32_t n_ranks, int64_t n, int32_t k, double* out_val,
+                         int32_t* out_idx, void* stream);
+
 /* ---- FM forward: replaces forward.py:21-22 `fma` ---------------------------------------------
  * yhat[r] = w0 + sum_i W_i x_i + 0.5 * sum_f ((sum_i V_if x_i)^2 - sum_i V_if^2 x_i^2) on CSR rows
  * (indptr int64 [n+1], indices int32, data fp32).  sums (optional) receives sum_i V_if x_i [n,dim].

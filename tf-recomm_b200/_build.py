@@ -13,7 +13,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "_obj")
 SO = os.path.join(HERE, os.environ.get("TFR_SO_NAME", "libtfrecomm.so"))
 OBJ = OBJ + os.environ.get("TFR_OBJ_SUFFIX", "")
-SOURCES = ["svd_forward.cu", "dedup_sort.cu", "segsum.cu", "chain.cu", "adam.cu", "adam_ring.cu", "fm.cu", "shard.cu", "allpairs.cu", "metrics.cu", "rank_users.cu", "fold_in.cu", "als.cu", "ials.cu", "capi.cu"]
+SOURCES = ["svd_forward.cu", "dedup_sort.cu", "segsum.cu", "chain.cu", "adam.cu", "adam_ring.cu", "fm.cu", "shard.cu", "shard_rank.cu", "allpairs.cu", "metrics.cu", "rank_users.cu", "fold_in.cu", "als.cu", "ials.cu", "capi.cu"]
 NVCC = os.environ.get("TFR_NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
          "-ccbin", "/usr/bin/g++", "-Xcompiler", "-fPIC,-fopenmp"] + os.environ.get("TFR_EXTRA_NVCC_FLAGS", "").split()

@@ -144,6 +144,10 @@ _PROTOS = {
     "tfr_shard_gather_records": (C.c_int, [C.POINTER(SvdTables), vp, C.POINTER(i32), C.POINTER(i32), i32, vp, vp]),
     "tfr_shard_fwd_records": (C.c_int, [C.POINTER(SvdTables), vp, vp, vp, vp, vp, i64, vp, vp, vp, vp, vp, vp, vp]),
     "tfr_shard_owner_prepare": (C.c_int, [vp, vp, C.POINTER(i32), C.POINTER(i32), i32, i32, i64, i64, vp, vp, vp, vp, vp, vp, vp]),
+    "tfr_shard_excl_workspace_bytes": (i64, [i64]),
+    "tfr_shard_excl_indptr": (C.c_int, [vp, vp, i64, vp, i64, i32, i32, vp, vp, i64, vp]),
+    "tfr_shard_excl_fill": (C.c_int, [vp, vp, i64, vp, i64, i32, i32, vp, vp, vp]),
+    "tfr_shard_topk_merge": (C.c_int, [vp, vp, i32, i64, i32, vp, vp, vp]),
     "tfr_svd_train_step_gathered": (C.c_int, [C.POINTER(SvdTables), vp, vp, vp, i64, i32, i32, vp, vp, vp, i64, vp]),
     "tfr_fm_forward": (C.c_int, [i64, vp, vp, vp, vp, vp, vp, i32, vp, vp, vp]),
     "tfr_fm_segment_grads": (C.c_int, [vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, i64, C.POINTER(StepWs), vp]),

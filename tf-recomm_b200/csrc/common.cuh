@@ -211,4 +211,8 @@ inline RowGeom row_geom(int dim) {
   return g;
 }
 
+// most ranks a row-sharded layout holds (rows of a table live on rank id mod G): the all-to-all's per-rank tables
+// (shard.cu) and the merge of the item shards' rankings (shard_rank.cu, one list head per lane)
+constexpr int SHARD_MAX_RANKS = 8;
+
 }  // namespace tfr

@@ -17,6 +17,7 @@
 #include <string.h>
 
 #include "common.cuh"
+#include "rank_order.cuh"
 
 namespace tfr {
 
@@ -269,13 +270,7 @@ __global__ void __launch_bounds__(RU_SEL_THREADS) rank_users_select_kernel(
 }
 
 // ---- 3. merge of the sorted chunk lists: one warp per query -----------------------------------------------------------
-// (v, i) ranks before (ov, oi): higher score, then lower item id; i = -1 (an exhausted list) ranks last.
-__device__ __forceinline__ bool ru_before(double v, int i, double ov, int oi) {
-  if (oi < 0) return i >= 0;
-  if (i < 0) return false;
-  return v > ov || (v == ov && i < oi);
-}
-
+// (the order and the warp arg-best step: rank_order.cuh, shared with the merge of item shards)
 constexpr int RU_MERGE_WARPS = 4;
 __global__ void __launch_bounds__(32 * RU_MERGE_WARPS) rank_users_merge_kernel(
     const double* __restrict__ part_val, const int32_t* __restrict__ part_idx, int32_t* __restrict__ heads, int n, int n_chunks,
@@ -305,13 +300,7 @@ __global__ void __launch_bounds__(32 * RU_MERGE_WARPS) rank_users_merge_kernel(
   for (int r = 0; r < k; ++r) {
     double wv = bv;
     int wi = bi, wl = lane;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      const double ov = __shfl_xor_sync(0xffffffffu, wv, o);
-      const int oi = __shfl_xor_sync(0xffffffffu, wi, o);
-      const int ol = __shfl_xor_sync(0xffffffffu, wl, o);
-      if (ru_before(ov, oi, wv, wi) || (oi == wi && ol < wl)) { wv = ov; wi = oi; wl = ol; }
-    }
+    ru_warp_best(wv, wi, wl);
     if (wi < 0) {   // every list is exhausted: pad the rest
       for (int rr = r + lane; rr < k; rr += 32) { out_val[(size_t)q * k + rr] = -INFINITY; out_idx[(size_t)q * k + rr] = -1; }
       return;

@@ -51,7 +51,6 @@ __global__ void __launch_bounds__(256) shard_gather_rows_kernel(const float* __r
 // A received buffer is [src 0: user part | item part][src 1: ...]...: ascending position = (source rank, position in
 // the source's slice) = GLOBAL BATCH ORDER, so the stable sort + in-order segment sums add duplicate rows in the order
 // the single-GPU path (and TF's unsorted_segment_sum) does.  Record stride = dim + 4 floats (16-byte aligned rows).
-constexpr int SHARD_MAX_RANKS = 8;
 struct ShardLayout {  // a combined buffer, by source (or destination) rank: [u_begin, i_begin) user part, [i_begin, end) item part
   int32_t n_ranks;
   int32_t u_begin[SHARD_MAX_RANKS], i_begin[SHARD_MAX_RANKS], end[SHARD_MAX_RANKS];

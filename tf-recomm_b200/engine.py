@@ -389,12 +389,13 @@ class SvdEngine:
         if exclude is not None:
             csr = exclude if isinstance(exclude, PairCSR) else self.pair_csr(*exclude)
         q = self._dev_i32(np.atleast_1d(np.asarray(users)) if not isinstance(users, torch.Tensor) else users.reshape(-1))
-        return self._rank_rows(self.t["user_feat"], self.t["user_bias"], self.U, self.feat_stride, q, k, csr)
+        return self._rank_rows(self.t["user_feat"], self.t["user_bias"], self.U, self.feat_stride, q, min(k, self.I), csr)
 
     def _rank_rows(self, user_feat, user_bias, n_users, user_stride, q, k, csr):
         """tfr_rank_users of the query rows q (device int32) of the user table (user_feat, user_bias) against this
-        engine's item side; csr: exclusion CSR indexed by the table's rows, or None."""
-        n, k = int(q.numel()), int(min(k, self.I))
+        engine's item side; csr: exclusion CSR indexed by the table's rows, or None.  k columns, padded with (-inf, -1)
+        past this engine's items (a shard of a row-sharded model ranks the k of the whole item table)."""
+        n, k = int(q.numel()), int(k)
         dev = self.device
         idx = torch.empty(n, k, dtype=torch.int32, device=dev)
         val = torch.empty(n, k, dtype=torch.float64, device=dev)
@@ -453,7 +454,7 @@ class SvdEngine:
         that could not be folded (info != 0, NaN) ranks nothing: (-inf, -1)."""
         n = int(folded.feat.shape[0])
         q = torch.arange(n, dtype=torch.int32, device=self.device)
-        return self._rank_rows(folded.feat, folded.bias, n, 0, q, k, folded.ratings if exclude_rated else None)
+        return self._rank_rows(folded.feat, folded.bias, n, 0, q, min(k, self.I), folded.ratings if exclude_rated else None)
 
     # ---- alternating least squares: exact half-sweeps of the training loss (tfr_als_half_sweep) ---------------------------
     def _als_refuse(self, reg=None):

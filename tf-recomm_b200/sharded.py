@@ -11,6 +11,10 @@ Per step, on every rank (one process per GPU, torch.distributed/NCCL for the plu
      (partner rows from the gathered buffers), one Adam pass over the local shard                     [local kernels]
 The exchange is ~68 MB per step against a 42.6 GB local table pass at G=8, so scaling is governed by the local pass
 (SURVEY 8e).  The reference has no distributed code; this is the B200-native equivalent north_star asks for.
+
+Serving (rank_users, fold_in, rank_folded) gives the single-GPU results, ids and bits, from the same sharded tables:
+query rows (or the rows of the rated items) are gathered to every rank the same way, every rank ranks its own item shard
+with the single-GPU kernel, and the per-rank lists are all-gathered and merged under the ranking's total order.
 """
 import ctypes as C
 
@@ -19,8 +23,8 @@ import torch
 import torch.distributed as dist
 
 from . import _lib, sharding
-from ._lib import OPT_SGD, README_FLAGS, VAR_ALL, OptScalars, SvdTables, check
-from .engine import SvdEngine
+from ._lib import LOSS_SIGMOID_CE, OPT_SGD, README_FLAGS, VAR_ALL, OptScalars, SvdTables, TfrError, check
+from .engine import FoldedUsers, PairCSR, SvdEngine
 
 
 class ShardedSvdEngine:
@@ -289,3 +293,191 @@ class ShardedSvdEngine:
 
     def get_local_tables(self):
         return self.local.get_tables()
+
+    # ---- serving: exact top-k and fold-in from the sharded tables ---------------------------------------------------------
+    # Collective calls: every rank passes the same arguments and gets the same result, the ids and bits SvdEngine gives on
+    # the re-assembled tables.  Ids are checked against the global tables on every rank before any collective, so every
+    # rank raises together.  The phases (gather / exclusion lists / local rank / merge) are separate methods so that tests
+    # can drive G virtual ranks on one GPU with the collectives emulated; the public methods compose them with
+    # torch.distributed, or with nothing at world 1.
+    def _check_ids(self, users, items, n_users=None):
+        SvdEngine._check_ids(self, users, items, n_users)   # against the GLOBAL U and I
+
+    def _dev_i32(self, a):
+        return self.local._dev_i32(a)
+
+    def _dev_f32(self, a):
+        return self.local._dev_f32(a)
+
+    def _all_reduce(self, t):
+        if self.world > 1:
+            dist.all_reduce(t, op=dist.ReduceOp.SUM, group=self.group)
+        return t
+
+    def _all_gather(self, t):
+        """[G, *t.shape]: every rank's t, by rank (all_gather_into_tensor)."""
+        if self.world == 1:
+            return t.unsqueeze(0)
+        out = torch.empty((self.world,) + tuple(t.shape), dtype=t.dtype, device=self.device)
+        dist.all_gather_into_tensor(out, t.contiguous(), group=self.group)
+        return out
+
+    def _gather_rows(self, feat, bias, rows_local, ids):
+        """tfr_shard_gather_rows of a local table: the rows of ids (device int32, global) this rank owns at their
+        positions, zeros elsewhere, as one buffer [m rows of d | m biases]; summed over the ranks it holds every row.
+        An all-reduce adds the +0.0 of the ranks that do not own a row, so an owned -0.0 arrives as +0.0.  No result bit
+        depends on that: the scorer's dot product and the fold-in Gram and right-hand side are float64 sums that start
+        from +0.0, a product with a zero factor is a zero, and in round-to-nearest +0.0 + (-0.0) = +0.0 + (+0.0) = +0.0,
+        so such a sum is never -0.0 and adding either zero to it (or a bias, or mu, after it) gives the same bits."""
+        m, d, e = ids.numel(), self.d, self.local
+        flat = torch.empty(max(m * d + m, 1), dtype=torch.float32, device=self.device)
+        keys = torch.empty(max(m, 1), dtype=torch.int32, device=self.device)
+        check(self.L.tfr_shard_gather_rows(feat.data_ptr(), bias.data_ptr(), rows_local, d, e.feat_stride, ids.data_ptr(),
+                                           m, self.world, self.rank, flat.data_ptr(), flat[m * d:].data_ptr(),
+                                           keys.data_ptr(), e._stream()))
+        return flat
+
+    def pair_csr(self, users, items):
+        """An exclusion set for rank_users from GLOBAL (user, item) pairs, built once per training set: this rank's share,
+        the distinct pairs whose item it owns, as a PairCSR by global user id with global item ids.  Not collective."""
+        self._check_ids(users, items)
+        u, i = self._dev_i32(users).to(torch.int64), self._dev_i32(items).to(torch.int64)
+        keep = i % self.world == self.rank
+        key = torch.unique(u[keep] * self.I + i[keep])   # sorted
+        indptr = torch.zeros(self.U + 1, dtype=torch.int64, device=self.device)
+        indptr[1:] = torch.cumsum(torch.bincount(key // self.I, minlength=self.U), 0)
+        return PairCSR(indptr, (key % self.I).to(torch.int32).contiguous())
+
+    def serve_gather(self, q):
+        """Phase 1 of rank_users: the query users' rows (q device int32, global ids) this rank owns; summed over the ranks
+        (all-reduce) the buffer is the n-row user table [n rows of d | n biases] of the queries, row j = user q[j]."""
+        with torch.cuda.device(self.device):
+            return self._gather_rows(self.local.t["user_feat"], self.local.t["user_bias"], self.U_loc, q)
+
+    def serve_exclusions(self, csr, rows):
+        """This rank's exclusion lists by query position: the items of csr's rows `rows` (device int32) that it owns, as
+        ascending local ids -- a PairCSR over len(rows) rows (tfr_shard_excl_indptr / _fill; one total read back)."""
+        n, dev = rows.numel(), self.device
+        indptr = torch.empty(n + 1, dtype=torch.int64, device=dev)
+        nbytes = check(self.L.tfr_shard_excl_workspace_bytes(n))
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        args = (csr.indptr.data_ptr(), csr.items.data_ptr(), csr.indptr.numel() - 1, rows.data_ptr(), n, self.world,
+                self.rank)
+        with torch.cuda.device(dev):
+            st = self.local._stream()
+            check(self.L.tfr_shard_excl_indptr(*args, indptr.data_ptr(), ws.data_ptr(), nbytes, st))
+            items = torch.empty(int(indptr[n]), dtype=torch.int32, device=dev)
+            check(self.L.tfr_shard_excl_fill(*args, indptr.data_ptr(), items.data_ptr(), st))
+        return PairCSR(indptr, items)
+
+    def serve_rank(self, user_feat, user_bias, k, excl):
+        """Phase 2: tfr_rank_users of every row of an n-row user table (the gathered queries, or folded users) against
+        this rank's item shard -> (local item ids [n, k], scores [n, k]).  k: of the WHOLE item table, so that every
+        rank's list has the same shape (a shard with fewer items pads with (-inf, -1)); excl: serve_exclusions or None."""
+        n = int(user_bias.numel())
+        q = torch.arange(n, dtype=torch.int32, device=self.device)
+        return self.local._rank_rows(user_feat, user_bias, n, 0, q, k, excl)
+
+    def serve_merge(self, val, idx):
+        """Phase 3: the all-gathered lists val / idx [G, n, k] -> (items [n, k] int32 global ids, scores [n, k] float64),
+        the top k of their union (tfr_shard_topk_merge)."""
+        G, n, k = idx.shape
+        if G != self.world:
+            raise TfrError("serve_merge: %d lists for a world of %d" % (G, self.world))
+        out_idx = torch.empty(n, k, dtype=torch.int32, device=self.device)
+        out_val = torch.empty(n, k, dtype=torch.float64, device=self.device)
+        with torch.cuda.device(self.device):
+            check(self.L.tfr_shard_topk_merge(val.data_ptr(), idx.data_ptr(), G, n, k, out_val.data_ptr(),
+                                              out_idx.data_ptr(), self.local._stream()))
+        return out_idx, out_val
+
+    def _rank_table(self, user_feat, user_bias, k, excl):
+        idx, val = self.serve_rank(user_feat, user_bias, k, excl)
+        return self.serve_merge(self._all_gather(val), self._all_gather(idx))
+
+    def rank_users(self, users, k=50, exclude=None):
+        """SvdEngine.rank_users on the sharded model: -> (items [n, k] int32 global ids, scores [n, k] float64) on the
+        device, identical in ids and bits to SvdEngine.rank_users on the re-assembled tables with the same exclude.
+        exclude: global (users, items) pairs, or a PairCSR from pair_csr() (build it once).  Collective: the query rows
+        are gathered to every rank, each ranks its item shard, and the per-rank lists are all-gathered and merged."""
+        self._check_ids(users, [])
+        csr = None
+        if exclude is not None:
+            csr = exclude if isinstance(exclude, PairCSR) else self.pair_csr(*exclude)
+        q = self._dev_i32(np.atleast_1d(np.asarray(users)) if not isinstance(users, torch.Tensor) else users.reshape(-1))
+        n, d, k = q.numel(), self.d, int(min(k, self.I))
+        if n == 0:
+            return (torch.empty(0, k, dtype=torch.int32, device=self.device),
+                    torch.empty(0, k, dtype=torch.float64, device=self.device))
+        with torch.cuda.device(self.device):
+            table = self._all_reduce(self.serve_gather(q))
+            excl = self.serve_exclusions(csr, q) if csr is not None else None
+            return self._rank_table(table[:n * d].view(n, d), table[n * d:n * d + n], k, excl)
+
+    def fold_gather(self, ids):
+        """Phase 1 of fold_in: the rows of the rated items ids (device int32, distinct, ascending) this rank owns; summed
+        over the ranks (all-reduce) the buffer is the compact item table [m rows of d | m biases], row j = item ids[j]."""
+        with torch.cuda.device(self.device):
+            return self._gather_rows(self.local.t["item_feat"], self.local.t["item_bias"], self.I_loc, ids)
+
+    def fold_plan(self, rows, items, rates, n=None, reg=None):
+        """Phase 0 of fold_in, the same on every rank: the refusals of SvdEngine.fold_in, the ratings CSR as SvdEngine
+        builds it (global ids), the distinct rated items (ascending) and each rating's position among them."""
+        e = self.local
+        if e.flags & LOSS_SIGMOID_CE:
+            raise TfrError("fold_in solves the squared-error objective; the sigmoid cross-entropy model is not supported")
+        reg = e.hyper["reg"] if reg is None else float(reg)
+        if not reg >= 0.0:
+            raise TfrError("fold_in: reg must be >= 0, got %r" % reg)
+        sizes = [a.numel() if isinstance(a, torch.Tensor) else np.asarray(a).size for a in (rows, items, rates)]
+        if len(set(sizes)) != 1:
+            raise TfrError("fold_in: rows, items and rates differ in length: %s" % sizes)
+        if n is None:
+            n = int((rows if isinstance(rows, torch.Tensor) else np.asarray(rows)).max()) + 1 if sizes[0] else 0
+        n = int(n)
+        indptr, it, rt = SvdEngine._csr_by_user(self, rows, items, rates, n_rows=n)   # checks ids against n and I
+        ids, pos = torch.unique(it, return_inverse=True)   # sorted: positions keep the CSR's order
+        return dict(n=n, reg=reg, indptr=indptr, items=it, rates=rt, ids=ids.to(torch.int32).contiguous(),
+                    pos=pos.to(torch.int32).contiguous())
+
+    def fold_gather(self, ids):
+        """Phase 1 of fold_in: the rows of the rated items ids (device int32, global) this rank owns; summed over the
+        ranks (all-reduce) the buffer is the compact item table [m rows of d | m biases], row j = item ids[j]."""
+        with torch.cuda.device(self.device):
+            return self._gather_rows(self.local.t["item_feat"], self.local.t["item_bias"], self.I_loc, ids)
+
+    def fold_solve(self, plan, table):
+        """Phase 2 of fold_in: tfr_fold_in_users against the compact item table, ratings by position in it."""
+        e, dev, d, n, m = self.local, self.device, self.d, plan["n"], plan["ids"].numel()
+        feat = torch.empty(n, d, dtype=torch.float32, device=dev)
+        bias = torch.empty(n, dtype=torch.float32, device=dev)
+        info = torch.empty(n, dtype=torch.int32, device=dev)
+        with torch.cuda.device(dev):
+            check(self.L.tfr_fold_in_users(table.data_ptr(), table[m * d:].data_ptr(), e.t["mu"].data_ptr(), m, d, 0,
+                                           e.flags, plan["reg"], plan["indptr"].data_ptr(), plan["pos"].data_ptr(),
+                                           plan["rates"].data_ptr(), n, feat.data_ptr(), bias.data_ptr(), info.data_ptr(),
+                                           e._stream()))
+        return FoldedUsers(feat, bias, PairCSR(plan["indptr"], plan["items"]), info)
+
+    def fold_in(self, rows, items, rates, n=None, reg=None):
+        """SvdEngine.fold_in on the sharded item side, the same FoldedUsers in bits (feat, bias, info; ratings with global
+        item ids).  Collective: the rows of the distinct rated items are gathered to every rank as a compact table, the
+        ratings CSR is built as SvdEngine builds it and its ids replaced by positions in that table, and every rank
+        solves the same systems (tfr_fold_in_users): tiny, redundant work that needs no broadcast.  Refuses what
+        SvdEngine.fold_in refuses, with TfrError."""
+        plan = self.fold_plan(rows, items, rates, n, reg)
+        return self.fold_solve(plan, self._all_reduce(self.fold_gather(plan["ids"])))
+
+    def rank_folded(self, folded, k=50, exclude_rated=True):
+        """SvdEngine.rank_folded on the sharded item side, the same ids and bits.  The folded rows are on every rank
+        already (fold_in solves them everywhere): each rank ranks its item shard, the lists are all-gathered and merged.
+        exclude_rated: never recommend the items the row was folded in from.  Collective."""
+        n, k = int(folded.feat.shape[0]), int(min(k, self.I))
+        if n == 0:
+            return (torch.empty(0, k, dtype=torch.int32, device=self.device),
+                    torch.empty(0, k, dtype=torch.float64, device=self.device))
+        with torch.cuda.device(self.device):
+            excl = None
+            if exclude_rated:
+                excl = self.serve_exclusions(folded.ratings, torch.arange(n, dtype=torch.int32, device=self.device))
+            return self._rank_table(folded.feat, folded.bias, k, excl)
