@@ -100,11 +100,13 @@ typedef struct {
   uint32_t chunk_ctr[4]; /* per-table chunk counters of the table pass's dynamic scheduling; 0 between steps */
   uint64_t* timeline;    /* optional debug buffer [2][TFR_TL_SLOTS] of %globaltimer ns: earliest block entry and
                             latest warp exit of every kernel of the step (there is no nsys on the box); null = off */
+  float lr_t_prev;       /* lr_t of the step that ended last (the end of a step moves lr_t on): the two-step table pass
+                            of tfr_svd_pair_pass applies that step's decay with it */
 } tfr_opt_scalars;
 #define TFR_TL_SLOTS 16
 enum { TFR_TL_ASSEMBLE = 0, TFR_TL_FWD = 1, TFR_TL_SORT = 2, TFR_TL_TILES = 3, TFR_TL_FIXUP = 4, TFR_TL_STREAM_UF = 5,
        TFR_TL_STREAM_IF = 6, TFR_TL_STREAM_UB = 7, TFR_TL_STREAM_IB = 8, TFR_TL_TOUCHED_U = 9, TFR_TL_TOUCHED_I = 10,
-       TFR_TL_FINISH = 11 };
+       TFR_TL_FINISH = 11, TFR_TL_BRING = 12 };
 
 int tfr_opt_init(tfr_opt_scalars* opt_dev, float lr, float reg, float beta1, float beta2, float eps,
                  int32_t flags, int32_t var_mask, void* stream);
@@ -219,6 +221,21 @@ int tfr_svd_train_step(const tfr_svd_tables* t, tfr_opt_scalars* opt, const int3
                        const int32_t* items, const float* rates, int64_t B, float* logits, float* infer,
                        int32_t flags, int32_t var_mask, void* workspace, int64_t workspace_bytes, void* stream,
                        void* const* side_streams, int32_t n_side, void* const* fork_join_events);
+/* Two Adam steps t, t+1 with ONE table pass (Adam, single-table tables only; bit for bit the state two steps leave).
+ * ws_t / ws_next: the workspaces of batches t and t+1, both sorted (tfr_svd_prefetch_batch); B is their batch size.
+ *   1. tfr_svd_train_step_presorted(phases = 1) on batch t                (forward + segment sums of step t)
+ *   2. tfr_svd_pair_bring: brings the rows of batch t+1 (run heads of ws_next's sorted ids, both sides, their bias
+ *      entries) to the end of step t -- step t's summed gradient if the row is in batch t, else step t's decay -- and
+ *      ends step t (bias_global, beta powers, lr_t, counters)
+ *   3. tfr_svd_train_step_presorted(phases = 1) on batch t+1              (reads the tables as step t left them)
+ *   4. tfr_svd_pair_pass: ONE pass over every row of every trained table applies what steps t and t+1 still owe each
+ *      row (the slot-map stamp tells: t+1 = step t+1's gradient; t = step t's gradient then step t+1's decay; else
+ *      both decays), and its last CTA ends step t+1.  Between 2 and 4 nothing may write ws_t's or ws_next's summed
+ *      gradients or partial sums (an id sort into either workspace may run beside step 4). */
+int tfr_svd_pair_bring(const tfr_svd_tables* t, tfr_opt_scalars* opt, int64_t B, int32_t flags, int32_t var_mask,
+                       void* ws_t, int64_t ws_t_bytes, void* ws_next, int64_t ws_next_bytes, void* stream);
+int tfr_svd_pair_pass(const tfr_svd_tables* t, tfr_opt_scalars* opt, int64_t B, int32_t flags, int32_t var_mask,
+                      void* ws_t, int64_t ws_t_bytes, void* ws_next, int64_t ws_next_bytes, void* stream);
 /* cudaEvent_t (timing disabled) on the current device, for callers without CUDA bindings of their own. */
 int tfr_event_create(void** event_out);
 int tfr_event_destroy(void* event);

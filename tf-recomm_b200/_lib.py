@@ -34,7 +34,7 @@ class OptScalars(C.Structure):
                 ("flags", i32), ("var_mask", i32),
                 ("global_step", i64), ("batch_cursor", i64), ("prefetch_cursor", i64), ("se_sum", C.c_double),
                 ("g_mu", f32), ("ticket", C.c_uint32), ("se_ring", vp), ("se_ring_len", i64),
-                ("chunk_ctr", C.c_uint32 * 4), ("timeline", vp)]
+                ("chunk_ctr", C.c_uint32 * 4), ("timeline", vp), ("lr_t_prev", f32)]
 
 
 class SvdTables(C.Structure):
@@ -127,6 +127,8 @@ _PROTOS = {
     "tfr_svd_prefetch_batch": (C.c_int, [C.POINTER(SvdTables), vp, vp, vp, vp, vp, i64, i64, vp, vp, vp, vp, i64, vp]),
     "tfr_svd_train_step_presorted": (C.c_int, [C.POINTER(SvdTables), vp, vp, vp, vp, i64, vp, vp, i32, i32, i32, vp, i64,
                                                vp]),
+    "tfr_svd_pair_bring": (C.c_int, [C.POINTER(SvdTables), vp, i64, i32, i32, vp, i64, vp, i64, vp]),
+    "tfr_svd_pair_pass": (C.c_int, [C.POINTER(SvdTables), vp, i64, i32, i32, vp, i64, vp, i64, vp]),
     "tfr_svd_step_carve": (C.c_int, [vp, i64, i64, i32, C.POINTER(StepWs)]),
     "tfr_svd_fwd_err": (C.c_int, [C.POINTER(SvdTables), vp, vp, vp, vp, i64, vp, vp, C.POINTER(StepWs), vp]),
     "tfr_svd_fwd_segment_grads": (C.c_int, [C.POINTER(SvdTables), vp, vp, vp, vp, i64, vp, vp, i32, C.POINTER(StepWs), vp]),

@@ -47,6 +47,7 @@ struct StreamTab {
   float *var, *m, *v;
   const int64_t* slot;  // (step stamp << 32 | run-head index); valid only if the stamp is this step's
   const float* gsum;
+  const float* gsum0;  // two-step pass: the previous step's summed gradients (rows stamped with that step)
   uint32_t n;        // floats (rows * width)
   uint32_t width;    // floats per row
   uint32_t stride;   // floats between consecutive rows of var (and of m, of v): width, or 3*width when var | m | v of a
@@ -70,13 +71,20 @@ struct StreamArgs {
 
 constexpr uint32_t DYN_TRIPS = 8;
 
-template <int UNROLL, bool DYNAMIC>
+// STEPS = 2: the pass applies two steps, t = global_step - 1 (already ended: tfr_svd_pair_bring) and t+1 = global_step,
+// in registers.  Rows of batch t+1 (stamp t+1) were brought to the end of step t before step t+1's forward and take
+// step t+1's gradient; rows of batch t only (stamp t) take step t's gradient, then step t+1's decay; all others decay
+// twice.  Per element that is the fp32 sequence two one-step passes run, so the state is the same bit for bit.
+template <int UNROLL, bool DYNAMIC, int STEPS>
 __global__ void __launch_bounds__(512, 2) adam_stream_multi_kernel(const __grid_constant__ StreamArgs a,
                                                                 const tfr_opt_scalars* __restrict__ opt, int tl_slot) {
+  static_assert(STEPS == 1 || (STEPS == 2 && !DYNAMIC), "two-step pass: static schedule only");
   pdl_wait();                // the fix-up's summed gradients and slot maps are complete
   pdl_launch_dependents();   // the next step's segment sums may become resident as this grid drains
   TlScope tl_scope(opt, tl_slot, a.tl_every != 0);
   const AdamK k = load_k(opt);
+  AdamK k0 = k;              // STEPS = 2: step t's scalars (only lr_t differs between two steps)
+  if (STEPS == 2) k0.lr_t = opt->lr_t_prev;
   const uint32_t stamp = (uint32_t)opt->global_step;
   uint32_t stride = gridDim.x * blockDim.x;
   uint32_t gtid = blockIdx.x * blockDim.x + threadIdx.x;
@@ -112,7 +120,7 @@ __global__ void __launch_bounds__(512, 2) adam_stream_multi_kernel(const __grid_
       auto trip = [&](uint32_t q0, uint32_t us) {
 
         float4 x[UNROLL], y[UNROLL], z[UNROLL], g[UNROLL];
-        bool has[UNROLL];
+        bool has[UNROLL], has0[UNROLL];  // has: a row of this step's slice; has0 (STEPS = 2): of step t's only
         size_t at[UNROLL];
         uint32_t row[UNROLL];
 #pragma unroll
@@ -130,11 +138,14 @@ __global__ void __launch_bounds__(512, 2) adam_stream_multi_kernel(const __grid_
         for (int u = 0; u < UNROLL; ++u) {
           const uint32_t q = q0 + u * us;
           has[u] = false;
+          has0[u] = false;
           if (q < n4 && t.slot) {
             const int64_t sl = t.slot[row[u]];
             has[u] = (uint32_t)(sl >> 32) == stamp;
-            if (has[u])
-              g[u] = *reinterpret_cast<const float4*>(t.gsum + (size_t)(uint32_t)sl * t.width + ((q - row[u] * upr) << 2));
+            if (STEPS == 2) has0[u] = (uint32_t)(sl >> 32) == stamp - 1u;
+            if (has[u] || has0[u])
+              g[u] = *reinterpret_cast<const float4*>((has[u] ? t.gsum : t.gsum0) + (size_t)(uint32_t)sl * t.width +
+                                                      ((q - row[u] * upr) << 2));
           }
         }
 #pragma unroll
@@ -148,6 +159,19 @@ __global__ void __launch_bounds__(512, 2) adam_stream_multi_kernel(const __grid_
             adam_grad(x[u].z, y[u].z, z[u].z, g[u].z, k);
             adam_grad(x[u].w, y[u].w, z[u].w, g[u].w, k);
           } else {
+            if (STEPS == 2) {
+              if (has0[u]) {
+                adam_grad(x[u].x, y[u].x, z[u].x, g[u].x, k0);
+                adam_grad(x[u].y, y[u].y, z[u].y, g[u].y, k0);
+                adam_grad(x[u].z, y[u].z, z[u].z, g[u].z, k0);
+                adam_grad(x[u].w, y[u].w, z[u].w, g[u].w, k0);
+              } else {
+                adam_decay(x[u].x, y[u].x, z[u].x, k0);
+                adam_decay(x[u].y, y[u].y, z[u].y, k0);
+                adam_decay(x[u].z, y[u].z, z[u].z, k0);
+                adam_decay(x[u].w, y[u].w, z[u].w, k0);
+              }
+            }
             adam_decay(x[u].x, y[u].x, z[u].x, k);
             adam_decay(x[u].y, y[u].y, z[u].y, k);
             adam_decay(x[u].z, y[u].z, z[u].z, k);
@@ -187,14 +211,22 @@ __global__ void __launch_bounds__(512, 2) adam_stream_multi_kernel(const __grid_
         const uint32_t row = t.width == 1u ? e : e / t.width;
         const size_t at = (size_t)row * t.stride + (e - row * t.width);
         float p = ld_stream_f1(t.var + at), q = ld_stream_f1(t.m + at), r = ld_stream_f1(t.v + at);
-        bool hs = false;
+        bool hs = false, hs0 = false;
         float gg = 0.0f;
         if (t.slot) {
           const int64_t sl = t.slot[row];
           hs = (uint32_t)(sl >> 32) == stamp;
-          if (hs) gg = t.gsum[(size_t)(uint32_t)sl * t.width + (e - row * t.width)];
+          if (STEPS == 2) hs0 = (uint32_t)(sl >> 32) == stamp - 1u;
+          if (hs || hs0) gg = (hs ? t.gsum : t.gsum0)[(size_t)(uint32_t)sl * t.width + (e - row * t.width)];
         }
-        if (hs) adam_grad(p, q, r, gg, k); else adam_decay(p, q, r, k);
+        if (hs) {
+          adam_grad(p, q, r, gg, k);
+        } else {
+          if (STEPS == 2) {
+            if (hs0) adam_grad(p, q, r, gg, k0); else adam_decay(p, q, r, k0);
+          }
+          adam_decay(p, q, r, k);
+        }
         st_stream_f1(t.var + at, p);
         st_stream_f1(t.m + at, q);
         st_stream_f1(t.v + at, r);
@@ -322,6 +354,125 @@ __global__ void __launch_bounds__(256) adam_slice_kernel(SliceSide s0, SliceSide
   }
 }
 
+// ---- two steps per table pass: bring the rows of batch t+1 to the end of step t -------------------------------
+// Runs after step t's segment sums and before step t+1's forward, one lane group per SLICE_ENT sorted entries of batch
+// t+1, both sides in one launch (blockIdx.y).  A run head's row (and its bias entry) takes step t's summed gradient if
+// the slot map carries step t's stamp (the row is in both batches), step t's decay otherwise; written back in place.
+// The two-step pass then owes these rows step t+1 only.  The last CTA ends step t.
+struct BringSide {
+  float *var, *m, *v;        // feature table (null = not trained)
+  float *bvar, *bm, *bv;     // bias table sharing the row ids (null = not trained)
+  const int32_t* sid;        // batch t+1's sorted ids
+  const int64_t* slot;       // row -> slot map as step t's fix-up left it
+  const float* gsum;         // step t's summed gradients [n, width], by run head
+  const float* bgsum;        // [n]
+  int64_t stride;            // floats between consecutive rows of var / m / v
+};
+
+template <int VEC, int L>
+__global__ void __launch_bounds__(256) adam_bring_kernel(BringSide s0, BringSide s1, int width, int64_t n,
+                                                         const tfr_opt_scalars* __restrict__ opt, FinishArgs fin) {
+  {
+    TlScope tl_scope(opt, TFR_TL_BRING);
+    const BringSide s = blockIdx.y ? s1 : s0;
+    const AdamK k = load_k(opt);
+    const uint32_t stamp = (uint32_t)opt->global_step;
+    const int lane = threadIdx.x & (L - 1);
+    const int64_t kk0 = (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / L) * SLICE_ENT;
+    if (kk0 < n && (s.var || s.bvar)) {
+      int32_t id[SLICE_ENT];
+      bool head[SLICE_ENT], in[SLICE_ENT];
+      uint32_t gi[SLICE_ENT];
+      int32_t prev = kk0 > 0 ? s.sid[kk0 - 1] : -1;
+#pragma unroll
+      for (int e = 0; e < SLICE_ENT; ++e) {
+        const int64_t kk = kk0 + e;
+        id[e] = kk < n ? s.sid[kk] : -1;
+        head[e] = kk < n && id[e] != prev;
+        prev = id[e];
+        in[e] = false;
+        gi[e] = 0;
+        if (head[e]) {
+          const int64_t sl = s.slot[id[e]];
+          in[e] = (uint32_t)(sl >> 32) == stamp;
+          gi[e] = (uint32_t)sl;
+        }
+      }
+      if (s.bvar && lane == 0) {
+        float a[SLICE_ENT], b[SLICE_ENT], d[SLICE_ENT], g[SLICE_ENT];
+#pragma unroll
+        for (int e = 0; e < SLICE_ENT; ++e)
+          if (head[e]) {
+            a[e] = s.bvar[id[e]]; b[e] = s.bm[id[e]]; d[e] = s.bv[id[e]];
+            if (in[e]) g[e] = s.bgsum[gi[e]];
+          }
+#pragma unroll
+        for (int e = 0; e < SLICE_ENT; ++e)
+          if (head[e]) {
+            if (in[e]) adam_grad(a[e], b[e], d[e], g[e], k); else adam_decay(a[e], b[e], d[e], k);
+            s.bvar[id[e]] = a[e]; s.bm[id[e]] = b[e]; s.bv[id[e]] = d[e];
+          }
+      }
+      if (s.var) {
+        const int n_units = width / VEC;
+        for (int unit = lane; unit < n_units; unit += L) {
+          float a[SLICE_ENT][VEC], b[SLICE_ENT][VEC], d[SLICE_ENT][VEC], g[SLICE_ENT][VEC];
+#pragma unroll
+          for (int e = 0; e < SLICE_ENT; ++e) {
+            if (!head[e]) continue;
+            const size_t off = (size_t)id[e] * s.stride + (size_t)unit * VEC;
+            const size_t goff = (size_t)gi[e] * width + (size_t)unit * VEC;
+            if constexpr (VEC == 4) {
+              const float4 av = *reinterpret_cast<const float4*>(s.var + off);
+              const float4 bv4 = *reinterpret_cast<const float4*>(s.m + off);
+              const float4 dv4 = *reinterpret_cast<const float4*>(s.v + off);
+              a[e][0] = av.x; a[e][1] = av.y; a[e][2] = av.z; a[e][3] = av.w;
+              b[e][0] = bv4.x; b[e][1] = bv4.y; b[e][2] = bv4.z; b[e][3] = bv4.w;
+              d[e][0] = dv4.x; d[e][1] = dv4.y; d[e][2] = dv4.z; d[e][3] = dv4.w;
+              if (in[e]) {
+                const float4 gv = *reinterpret_cast<const float4*>(s.gsum + goff);
+                g[e][0] = gv.x; g[e][1] = gv.y; g[e][2] = gv.z; g[e][3] = gv.w;
+              }
+            } else {
+              a[e][0] = s.var[off]; b[e][0] = s.m[off]; d[e][0] = s.v[off];
+              if (in[e]) g[e][0] = s.gsum[goff];
+            }
+          }
+#pragma unroll
+          for (int e = 0; e < SLICE_ENT; ++e) {
+            if (!head[e]) continue;
+            const size_t off = (size_t)id[e] * s.stride + (size_t)unit * VEC;
+#pragma unroll
+            for (int c = 0; c < VEC; ++c) {
+              if (in[e]) adam_grad(a[e][c], b[e][c], d[e][c], g[e][c], k);
+              else adam_decay(a[e][c], b[e][c], d[e][c], k);
+            }
+            if constexpr (VEC == 4) {
+              *reinterpret_cast<float4*>(s.var + off) = make_float4(a[e][0], a[e][1], a[e][2], a[e][3]);
+              *reinterpret_cast<float4*>(s.m + off) = make_float4(b[e][0], b[e][1], b[e][2], b[e][3]);
+              *reinterpret_cast<float4*>(s.v + off) = make_float4(d[e][0], d[e][1], d[e][2], d[e][3]);
+            } else {
+              s.var[off] = a[e][0]; s.m[off] = b[e][0]; s.v[off] = d[e][0];
+            }
+          }
+        }
+      }
+    }
+  }
+  // the last CTA to get here ends step t (every CTA has read lr_t and the stamp by now)
+  __shared__ int s_last;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    s_last = atomicAdd(&fin.opt->ticket, 1u) == gridDim.x * gridDim.y - 1;
+  }
+  __syncthreads();
+  if (s_last && threadIdx.x < 32) {
+    finish_step_scalars(fin.mu, fin.m_mu, fin.v_mu, fin.opt, fin.partials, fin.se_partials, fin.n_partials);
+    if (threadIdx.x == 0) fin.opt->ticket = 0;
+  }
+}
+
 // ---- end of step (as a launch of its own: SGD mode, no trained table, the piecewise API) ---------------------
 // The row -> slot maps carry the step's stamp, so nothing has to be reset between steps.
 __global__ void __launch_bounds__(32) finish_step_kernel(tfr_svd_tables t, tfr_opt_scalars* opt,
@@ -339,6 +490,7 @@ __global__ void opt_init_kernel(tfr_opt_scalars* opt, float lr, float reg, float
   opt->one_minus_beta2 = sub_rn(1.0f, beta2);
   float tt = sqrt_rn(sub_rn(1.0f, beta2));
   opt->lr_t = div_rn(mul_rn(lr, tt), sub_rn(1.0f, beta1));
+  opt->lr_t_prev = opt->lr_t;
   opt->flags = flags; opt->var_mask = var_mask;
   opt->global_step = 0; opt->batch_cursor = 0; opt->prefetch_cursor = 0;
   opt->se_sum = 0.0; opt->g_mu = 0.0f; opt->ticket = 0u;
@@ -359,7 +511,7 @@ extern "C" int tfr_opt_init(tfr_opt_scalars* opt_dev, float lr, float reg, float
 }
 
 static int launch_stream_chunks(const StreamTab* chunks, int n_chunks, const tfr_opt_scalars* opt, int tl_slot,
-                                cudaStream_t st, const FinishArgs* fin) {
+                                cudaStream_t st, const FinishArgs* fin, int steps) {
   StreamArgs a;
   memset(&a, 0, sizeof(a));
   if (fin) a.fin = *fin;
@@ -372,7 +524,7 @@ static int launch_stream_chunks(const StreamTab* chunks, int n_chunks, const tfr
   a.n_tabs = n_chunks;
   a.total_units = (uint32_t)units;
   a.copy_only = tune(TUNE_STREAM_COPY_ONLY);
-  a.dynamic = (fin && tune(TUNE_STREAM_DYNAMIC)) ? 1 : 0;
+  a.dynamic = (fin && steps == 1 && tune(TUNE_STREAM_DYNAMIC)) ? 1 : 0;
   a.tl_every = tune(TUNE_TL_EVERY_CTA);
   a.ld_hint = tune(TUNE_STREAM_LD);
   a.st_hint = tune(TUNE_STREAM_ST);
@@ -414,15 +566,18 @@ static int launch_stream_chunks(const StreamTab* chunks, int n_chunks, const tfr
     grid = at;
   }
   const bool pdl = tune(TUNE_PDL) != 0;
-  if (a.dynamic) {
-    TFR_PREP((adam_stream_multi_kernel<2, true>));
-    TFR_CUDA(launch_kernel(adam_stream_multi_kernel<2, true>, dim3((unsigned)grid), dim3(cfg_threads), 0, st, pdl, a, opt, tl_slot));
+  if (steps == 2) {  // UNROLL 2 only: at 4 the kernel spills at 64 registers
+    TFR_PREP((adam_stream_multi_kernel<2, false, 2>));
+    TFR_CUDA(launch_kernel(adam_stream_multi_kernel<2, false, 2>, dim3((unsigned)grid), dim3(cfg_threads), 0, st, pdl, a, opt, tl_slot));
+  } else if (a.dynamic) {
+    TFR_PREP((adam_stream_multi_kernel<2, true, 1>));
+    TFR_CUDA(launch_kernel(adam_stream_multi_kernel<2, true, 1>, dim3((unsigned)grid), dim3(cfg_threads), 0, st, pdl, a, opt, tl_slot));
   } else if (cfg_unroll >= 4) {
-    TFR_PREP((adam_stream_multi_kernel<4, false>));
-    TFR_CUDA(launch_kernel(adam_stream_multi_kernel<4, false>, dim3((unsigned)grid), dim3(cfg_threads), 0, st, pdl, a, opt, tl_slot));
+    TFR_PREP((adam_stream_multi_kernel<4, false, 1>));
+    TFR_CUDA(launch_kernel(adam_stream_multi_kernel<4, false, 1>, dim3((unsigned)grid), dim3(cfg_threads), 0, st, pdl, a, opt, tl_slot));
   } else {
-    TFR_PREP((adam_stream_multi_kernel<2, false>));
-    TFR_CUDA(launch_kernel(adam_stream_multi_kernel<2, false>, dim3((unsigned)grid), dim3(cfg_threads), 0, st, pdl, a, opt, tl_slot));
+    TFR_PREP((adam_stream_multi_kernel<2, false, 1>));
+    TFR_CUDA(launch_kernel(adam_stream_multi_kernel<2, false, 1>, dim3((unsigned)grid), dim3(cfg_threads), 0, st, pdl, a, opt, tl_slot));
   }
   return TFR_OK;
 }
@@ -434,8 +589,9 @@ int ring_pass_launch(const tfr_adam_table* tabs, int n, const tfr_opt_scalars* o
                      const FinishArgs* fin);
 // fin != null: the pass's last launch also ends the step (see FinishArgs); returns 1 if it did, 0 if no launch
 // was issued (nothing to stream), negative on error.
+// gsum0 (null: one step): the previous step's summed gradient of every table -- the two-step pass (always the LDG pass)
 int adam_stream_multi_impl(const tfr_adam_table* tables, int32_t n_tables, tfr_opt_scalars* opt, int32_t tl_slot,
-                           void* stream, const FinishArgs* fin);
+                           void* stream, const FinishArgs* fin, const float* const* gsum0 = nullptr);
 }
 
 extern "C" int tfr_adam_stream_multi(const tfr_adam_table* tables, int32_t n_tables, const tfr_opt_scalars* opt,
@@ -445,13 +601,16 @@ extern "C" int tfr_adam_stream_multi(const tfr_adam_table* tables, int32_t n_tab
 }
 
 int tfr::adam_stream_multi_impl(const tfr_adam_table* tables, int32_t n_tables, tfr_opt_scalars* opt, int32_t tl_slot,
-                                void* stream, const FinishArgs* fin) {
+                                void* stream, const FinishArgs* fin, const float* const* gsum0) {
   TFR_CHECK_ARG(tables && n_tables >= 1 && n_tables <= 4 && opt && tl_slot >= 0 && tl_slot < TFR_TL_SLOTS);
   for (int i = 0; i < n_tables; ++i) {
     TFR_CHECK_ARG(tables[i].rows >= 0 && tables[i].width > 0);
     TFR_CHECK_ARG(tables[i].rows == 0 || (tables[i].var && tables[i].m && tables[i].v && (!tables[i].slot || tables[i].gsum)));
   }
-  if (ring_pass_eligible(tables, n_tables)) {
+  const int steps = gsum0 ? 2 : 1;
+  for (int i = 0; gsum0 && i < n_tables; ++i)
+    TFR_CHECK_ARG(tables[i].rows == 0 || (tables[i].slot && gsum0[i] && (tables[i].width % 4 != 0 || (uintptr_t)gsum0[i] % 16 == 0)));
+  if (steps == 1 && ring_pass_eligible(tables, n_tables)) {
     const int rc = ring_pass_launch(tables, n_tables, opt, tl_slot, (cudaStream_t)stream, fin);
     return rc < 0 ? rc : 1;
   }
@@ -483,12 +642,13 @@ int tfr::adam_stream_multi_impl(const tfr_adam_table* tables, int32_t n_tables, 
       c.stride = (uint32_t)rstride;
       c.slot = t.slot ? t.slot + r0 : nullptr;
       c.gsum = t.gsum;
+      c.gsum0 = gsum0 ? gsum0[i] : nullptr;
       c.n = (uint32_t)(nr * (uint64_t)t.width);
       c.width = (uint32_t)t.width;
       c.unit_end = 0;
       const uint64_t cu = ((uint64_t)c.n + 3) / 4;
       if (np == 4 || pending_units + cu >= ((uint64_t)1 << 32)) {
-        int rc = launch_stream_chunks(pending, np, opt, tl_slot, st, nullptr);
+        int rc = launch_stream_chunks(pending, np, opt, tl_slot, st, nullptr, steps);
         if (rc) return rc;
         np = 0;
         pending_units = 0;
@@ -498,7 +658,7 @@ int tfr::adam_stream_multi_impl(const tfr_adam_table* tables, int32_t n_tables, 
     }
   }
   if (np) {
-    const int rc = launch_stream_chunks(pending, np, opt, tl_slot, st, fin);
+    const int rc = launch_stream_chunks(pending, np, opt, tl_slot, st, fin, steps);
     return rc < 0 ? rc : 1;
   }
   return 0;
@@ -577,5 +737,54 @@ int adam_pass_and_finish(const tfr_adam_table* tabs, int nt, const tfr_svd_table
   }
   if (rc == 0) return tfr_svd_finish_step(t, opt, nullptr, nullptr, 0, ws, n_partials, stream);
   return TFR_OK;
+}
+
+// the two-step pass of steps t (ended, summed gradients gsum0[i] of table i) and t+1 (ws), which it ends
+int adam_pair_pass_and_finish(const tfr_adam_table* tabs, const float* const* gsum0, int nt, const tfr_svd_tables* t,
+                              tfr_opt_scalars* opt, const tfr_svd_step_ws* ws, int n_partials, void* stream) {
+  TFR_CHECK_ARG(n_partials > 0 && n_partials <= TFR_MAX_PARTIALS);
+  int rc = 0;
+  if (nt > 0) {
+    const FinishArgs fin{opt, t->mu, t->m_mu, t->v_mu, ws->partials, ws->se_partials, n_partials};
+    rc = adam_stream_multi_impl(tabs, nt, opt, TFR_TL_STREAM_UF, stream, &fin, gsum0);
+    if (rc < 0) return rc;
+  }
+  if (rc == 0) return tfr_svd_finish_step(t, opt, nullptr, nullptr, 0, ws, n_partials, stream);
+  return TFR_OK;
+}
+
+// sides[i].gsum / bgsum: step t's summed gradients; sorted_ids: batch t+1's; slot[i]: the side's row -> slot map
+int adam_bring_and_finish(const tfr_slice_update* sides, const int64_t* const* slot, int32_t width, int64_t n,
+                          const tfr_svd_tables* t, tfr_opt_scalars* opt, const tfr_svd_step_ws* ws, int n_partials,
+                          void* stream) {
+  TFR_CHECK_ARG(sides && slot && width > 0 && n > 0 && opt && n_partials > 0 && n_partials <= TFR_MAX_PARTIALS);
+  BringSide ss[2];
+  for (int i = 0; i < 2; ++i) {
+    const tfr_slice_update& u = sides[i];
+    TFR_CHECK_ARG(u.sorted_ids && slot[i]);
+    TFR_CHECK_ARG(!u.var || (u.gsum && u.m && u.v));
+    TFR_CHECK_ARG(!u.bvar || (u.bgsum && u.bm && u.bv));
+    ss[i] = BringSide{u.var, u.m, u.v, u.bvar, u.bm, u.bv, u.sorted_ids, slot[i], u.gsum, u.bgsum,
+                      u.stride ? u.stride : width};
+  }
+  const FinishArgs fin{opt, t->mu, t->m_mu, t->v_mu, ws->partials, ws->se_partials, n_partials};
+  const RowGeom g = row_geom(width);
+  const int64_t groups = (n + SLICE_ENT - 1) / SLICE_ENT;
+  const int groups_per_cta = 256 / g.lanes;
+  dim3 grid((unsigned)((groups + groups_per_cta - 1) / groups_per_cta), 2u);
+  cudaStream_t st = (cudaStream_t)stream;
+#define TFR_BRING_CASE(V, LL)                                                                        \
+  if (g.vec == V && g.lanes == LL) {                                                                 \
+    TFR_PREP((adam_bring_kernel<V, LL>));                                                            \
+    adam_bring_kernel<V, LL><<<grid, 256, 0, st>>>(ss[0], ss[1], width, n, opt, fin);                \
+    TFR_LAUNCH_CHECK();                                                                               \
+    return TFR_OK;                                                                                    \
+  }
+  TFR_BRING_CASE(4, 1) TFR_BRING_CASE(4, 2) TFR_BRING_CASE(4, 4) TFR_BRING_CASE(4, 8) TFR_BRING_CASE(4, 16)
+  TFR_BRING_CASE(4, 32) TFR_BRING_CASE(1, 1) TFR_BRING_CASE(1, 2) TFR_BRING_CASE(1, 4) TFR_BRING_CASE(1, 8)
+  TFR_BRING_CASE(1, 16) TFR_BRING_CASE(1, 32)
+#undef TFR_BRING_CASE
+  set_error("unsupported width %d", width);
+  return TFR_ERR_INVALID;
 }
 }  // namespace tfr

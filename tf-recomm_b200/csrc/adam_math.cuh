@@ -74,7 +74,8 @@ static __device__ __noinline__ void finish_step_scalars(float* mu, float* m_mu, 
       opt->beta1_power = mul_rn(opt->beta1_power, opt->beta1);
       opt->beta2_power = mul_rn(opt->beta2_power, opt->beta2);
       // lr_t of the NEXT step (TF: _apply_sparse_shared recomputes it from the advanced powers), so that a step
-      // needs no kernel in front of the forward
+      // needs no kernel in front of the forward; this step's stays for the two-step pass
+      opt->lr_t_prev = opt->lr_t;
       float tt = sqrt_rn(sub_rn(1.0f, opt->beta2_power));
       opt->lr_t = div_rn(mul_rn(opt->lr, tt), sub_rn(1.0f, opt->beta1_power));
     }

@@ -78,6 +78,11 @@ int svd_segment_grads_impl(const tfr_svd_tables* t, const tfr_opt_scalars* opt, 
                            const int32_t* items, int64_t B, const tfr_svd_step_ws* ws, int flags_host, void* stream);
 int adam_pass_and_finish(const tfr_adam_table* tabs, int nt, const tfr_svd_tables* t, tfr_opt_scalars* opt,
                          const tfr_svd_step_ws* ws, int n_partials, int tl_slot, void* stream);
+int adam_pair_pass_and_finish(const tfr_adam_table* tabs, const float* const* gsum0, int nt, const tfr_svd_tables* t,
+                              tfr_opt_scalars* opt, const tfr_svd_step_ws* ws, int n_partials, void* stream);
+int adam_bring_and_finish(const tfr_slice_update* sides, const int64_t* const* slot, int32_t width, int64_t n,
+                          const tfr_svd_tables* t, tfr_opt_scalars* opt, const tfr_svd_step_ws* ws, int n_partials,
+                          void* stream);
 
 void prep_kernel(const void* fn) { prep_kernel_carveout(fn, 0); }
 
@@ -320,6 +325,56 @@ extern "C" int tfr_svd_train_step_presorted(const tfr_svd_tables* t, tfr_opt_sca
   TFR_CHECK_ARG(phases >= 1 && phases <= 3);
   return run_step(t, opt, users, items, rates, B, logits, infer, flags, var_mask, workspace, workspace_bytes, stream,
                   nullptr, 0, nullptr, true, phases);
+}
+
+// ---- two steps per table pass (include/tfrecomm.h: tfr_svd_pair_bring / tfr_svd_pair_pass) ----------------------------
+static int pair_args(const tfr_svd_tables* t, tfr_opt_scalars* opt, int64_t B, int32_t flags, void* ws_t,
+                     int64_t ws_t_bytes, void* ws_next, int64_t ws_next_bytes, tfr_svd_step_ws* a, tfr_svd_step_ws* b) {
+  TFR_CHECK_ARG(t && opt && B > 0 && t->dim > 0 && ws_t && ws_next && ws_t != ws_next);
+  // Adam on single-table tables: SGD has no table-wide pass, the row-sharded step folds its partial sums elsewhere
+  TFR_CHECK_ARG(!(flags & TFR_OPT_SGD) && t->g_user_feat == nullptr && t->user_slot && t->item_slot);
+  TFR_CHECK_ARG(t->m_uf && t->v_uf && t->m_if && t->v_if && t->m_ub && t->v_ub && t->m_ib && t->v_ib && t->m_mu && t->v_mu);
+  int rc = tfr_svd_step_carve(ws_t, ws_t_bytes, B, t->dim, a);
+  if (rc) return rc;
+  if ((rc = tfr_svd_step_carve(ws_next, ws_next_bytes, B, t->dim, b))) return rc;
+  // the fused step: its fix-up's last CTA folded the partial sums into [TFR_MAX_PARTIALS]
+  a->partials += TFR_MAX_PARTIALS; a->se_partials += TFR_MAX_PARTIALS;
+  b->partials += TFR_MAX_PARTIALS; b->se_partials += TFR_MAX_PARTIALS;
+  return TFR_OK;
+}
+
+extern "C" int tfr_svd_pair_bring(const tfr_svd_tables* t, tfr_opt_scalars* opt, int64_t B, int32_t flags,
+                                  int32_t var_mask, void* ws_t, int64_t ws_t_bytes, void* ws_next, int64_t ws_next_bytes,
+                                  void* stream) {
+  tfr_svd_step_ws a, b;
+  int rc = pair_args(t, opt, B, flags, ws_t, ws_t_bytes, ws_next, ws_next_bytes, &a, &b);
+  if (rc) return rc;
+  const bool uf = var_mask & TFR_VAR_UF, ub = var_mask & TFR_VAR_UB, itf = var_mask & TFR_VAR_IF, ib = var_mask & TFR_VAR_IB;
+  const tfr_slice_update sides[2] = {
+      {uf ? t->user_feat : nullptr, t->m_uf, t->v_uf, ub ? t->user_bias : nullptr, t->m_ub, t->v_ub, b.su_ids,
+       a.gsum_uf, a.gsum_ub, t->feat_stride},
+      {itf ? t->item_feat : nullptr, t->m_if, t->v_if, ib ? t->item_bias : nullptr, t->m_ib, t->v_ib, b.si_ids,
+       a.gsum_if, a.gsum_ib, t->feat_stride}};
+  const int64_t* slots[2] = {t->user_slot, t->item_slot};
+  return adam_bring_and_finish(sides, slots, t->dim, B, t, opt, &a, 1, stream);
+}
+
+extern "C" int tfr_svd_pair_pass(const tfr_svd_tables* t, tfr_opt_scalars* opt, int64_t B, int32_t flags,
+                                 int32_t var_mask, void* ws_t, int64_t ws_t_bytes, void* ws_next, int64_t ws_next_bytes,
+                                 void* stream) {
+  tfr_svd_step_ws a, b;
+  int rc = pair_args(t, opt, B, flags, ws_t, ws_t_bytes, ws_next, ws_next_bytes, &a, &b);
+  if (rc) return rc;
+  const int dim = t->dim;
+  tfr_adam_table tabs[4];
+  const float* gsum0[4];
+  int nt = 0;
+  // the order of run_step's pass
+  if (var_mask & TFR_VAR_UB) { gsum0[nt] = a.gsum_ub; tabs[nt++] = tfr_adam_table{t->user_bias, t->m_ub, t->v_ub, t->user_num, 1, t->user_slot, b.gsum_ub, 0}; }
+  if (var_mask & TFR_VAR_IB) { gsum0[nt] = a.gsum_ib; tabs[nt++] = tfr_adam_table{t->item_bias, t->m_ib, t->v_ib, t->item_num, 1, t->item_slot, b.gsum_ib, 0}; }
+  if (var_mask & TFR_VAR_IF) { gsum0[nt] = a.gsum_if; tabs[nt++] = tfr_adam_table{t->item_feat, t->m_if, t->v_if, t->item_num, dim, t->item_slot, b.gsum_if, t->feat_stride}; }
+  if (var_mask & TFR_VAR_UF) { gsum0[nt] = a.gsum_uf; tabs[nt++] = tfr_adam_table{t->user_feat, t->m_uf, t->v_uf, t->user_num, dim, t->user_slot, b.gsum_uf, t->feat_stride}; }
+  return adam_pair_pass_and_finish(tabs, gsum0, nt, t, opt, &b, 1, stream);
 }
 
 // The step from the sort on, for the all-to-all sharded exchange: keys and ws.err by arrival position are the caller's

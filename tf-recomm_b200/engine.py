@@ -193,7 +193,10 @@ class SvdEngine:
         self.se_ring = None
         self.overlap = True
         self._primed = None
+        self._ahead = 1        # batches assembled + sorted ahead from set _primed on (2: the next one in the other set)
         self.graph_steps = 8   # steps per captured graph in run_stream_steps (pipelined mode)
+        # two steps per table pass in run_stream_steps (None: where the pass is bandwidth-bound, see _pair_steps)
+        self.pair_steps = None
 
     # ---- plumbing ---------------------------------------------------------------------------------------
     def _n_side(self):
@@ -1074,10 +1077,10 @@ class SvdEngine:
             ri = torch.from_numpy(np.ascontiguousarray(row_index, dtype=np.int64)).to(self.device)
         assert ri.numel() % B == 0
         # captured graphs bake the buffer's address: keep ONE persistent buffer and copy new streams into it
-        # (+ B zero entries of slack: the pipelined step assembles one batch past the end)
+        # (+ 2B zero entries of slack: the pipelined steps assemble up to two batches past the end)
         cap = getattr(self, "_row_index_buf", None)
-        if cap is None or cap.numel() < ri.numel() + B:
-            self._row_index_buf = torch.zeros(ri.numel() + B, dtype=torch.int64, device=self.device)
+        if cap is None or cap.numel() < ri.numel() + 2 * B:
+            self._row_index_buf = torch.zeros(ri.numel() + 2 * B, dtype=torch.int64, device=self.device)
             self._destroy_graphs()
         self._row_index_buf[:ri.numel()].copy_(ri)
         self._row_index_buf[ri.numel():].zero_()
@@ -1097,7 +1100,7 @@ class SvdEngine:
 
     # ---- debug timeline (in-kernel %globaltimer stamps; there is no nsys on the box) ----------------------
     TL_NAMES = ("assemble", "fwd_err", "sort", "seg_tiles", "seg_fixup", "adam_pass", "-", "-", "-", "sgd_slice",
-                "-", "finish")
+                "-", "finish", "bring_rows")
 
     def enable_timeline(self):
         self.timeline = torch.zeros(32, dtype=torch.int64, device=self.device)
@@ -1143,31 +1146,37 @@ class SvdEngine:
                                             bufs["users"].data_ptr(), bufs["items"].data_ptr(),
                                             bufs["rates"].data_ptr(), ws.data_ptr(), ws.numel(), stream_handle))
 
-    def _enqueue_pipelined_step(self, B, slot):
-        """Step on the batch already assembled + sorted in set `slot`, while the NEXT batch is assembled + sorted
-        into the other set on the side stream: the id-only work leaves the critical path (it runs under the
+    def _phase(self, B, slot, p, stream):
+        bufs, ws = self.stream_buffers(B, slot), self.workspace((B, slot))
+        check(self.L.tfr_svd_train_step_presorted(C.byref(self.tables_struct), self.opt.data_ptr(),
+                                                  bufs["users"].data_ptr(), bufs["items"].data_ptr(),
+                                                  bufs["rates"].data_ptr(), B, bufs["logits"].data_ptr(),
+                                                  bufs["infer"].data_ptr(), self.flags, self.var_mask, p,
+                                                  ws.data_ptr(), ws.numel(), stream.cuda_stream))
+
+    def _enqueue_pipelined_step(self, B, slot, ahead=1):
+        """Step on the batch already assembled + sorted in set `slot`, while the batch after the `ahead` sorted ones
+        is assembled + sorted on the side stream (into the other set when ahead = 1, into `slot` itself when the other
+        set already holds the next batch): the id-only work leaves the critical path (it runs under the
         bandwidth-bound table pass, which it barely disturbs)."""
         main = torch.cuda.current_stream(self.device)
         side = self.side_streams[0]
-        bufs, ws = self.stream_buffers(B, slot), self.workspace((B, slot))
+        target = (slot + ahead) & 1
 
         def phase(p):
-            check(self.L.tfr_svd_train_step_presorted(C.byref(self.tables_struct), self.opt.data_ptr(),
-                                                      bufs["users"].data_ptr(), bufs["items"].data_ptr(),
-                                                      bufs["rates"].data_ptr(), B, bufs["logits"].data_ptr(),
-                                                      bufs["infer"].data_ptr(), self.flags, self.var_mask, p,
-                                                      ws.data_ptr(), ws.numel(), main.cuda_stream))
+            self._phase(B, slot, p, main)
         # Where to fork the next batch's assemble + sort: UNDER the table pass when that pass is long (it is
         # bandwidth-bound and barely notices them, while the latency-bound gathers of phase 1 would slow down
         # beside them); at the start of the step when the tables are small and the pass is a few microseconds.
-        small = self._small_tables()
+        # (into `slot` itself only once this step's forward has read the set)
+        small = self._small_tables() and target != slot
         if small:
             side.wait_stream(main)
-            self._prefetch(B, 1 - slot, False, side.cuda_stream)
+            self._prefetch(B, target, False, side.cuda_stream)
         phase(1)                      # forward + segment sums
         if not small:
             side.wait_stream(main)
-            self._prefetch(B, 1 - slot, False, side.cuda_stream)
+            self._prefetch(B, target, False, side.cuda_stream)
         hook = getattr(self, "timing_hook", None)   # bench.py: event-record nodes around the table pass, in situ
         if hook:
             hook("pass_begin", slot, main)
@@ -1175,6 +1184,41 @@ class SvdEngine:
         if hook:
             hook("pass_end", slot, main)
         main.wait_stream(side)
+
+    def _enqueue_pair(self, B, slot):
+        """Steps t and t+1 on the batches sorted in sets `slot` and 1 - slot with ONE table pass (tfr_svd_pair_pass):
+        forward + segment sums of t -> the rows of batch t+1 brought to the end of step t -> forward + segment sums of
+        t+1 -> the two-step pass, under which batches t+2 and t+3 are assembled + sorted into the two sets on the side
+        stream.  Nothing the side stream writes (ids, sorted pairs, sort scratch) is read by the pass (summed
+        gradients, folded partial sums, slot maps), so two buffer sets are enough."""
+        main = torch.cuda.current_stream(self.device)
+        side = self.side_streams[0]
+        ws_t, ws_n = self.workspace((B, slot)), self.workspace((B, 1 - slot))
+        args = (C.byref(self.tables_struct), self.opt.data_ptr(), B, self.flags, self.var_mask,
+                ws_t.data_ptr(), ws_t.numel(), ws_n.data_ptr(), ws_n.numel(), main.cuda_stream)
+        self._phase(B, slot, 1, main)
+        check(self.L.tfr_svd_pair_bring(*args))
+        self._phase(B, 1 - slot, 1, main)
+        side.wait_stream(main)
+        self._prefetch(B, slot, False, side.cuda_stream)
+        self._prefetch(B, 1 - slot, False, side.cuda_stream)
+        hook = getattr(self, "timing_hook", None)
+        if hook:
+            hook("pass_begin", slot, main)
+        check(self.L.tfr_svd_pair_pass(*args))
+        if hook:
+            hook("pass_end", slot, main)
+        main.wait_stream(side)
+
+    def _pair_steps(self):
+        """Two steps per table pass (Adam only): where the pass streams the tables from HBM -- it then costs about one
+        step's pass for two steps.  The knob-selected passes (TMA ring, dynamic scheduling) keep one step per pass."""
+        if self.sgd:
+            return False
+        if self.pair_steps is not None:
+            return bool(self.pair_steps)
+        return (not self._small_tables() and _lib.tune_get("PASS_RING") == 0
+                and _lib.tune_get("STREAM_DYNAMIC") == 0)
 
     def stream_buffers(self, B, slot=0):
         key = ("bufs", B, slot)
@@ -1240,16 +1284,21 @@ class SvdEngine:
         with torch.cuda.device(self.device):
             self._run_pipelined(self.stream_B, n_steps, True, launch=False)
 
-    def _pipe_graph(self, B, slot, K):
-        """Graph of K consecutive pipelined steps beginning on buffer set `slot` (K = 1, or an even count so that the
-        graph ends on the set it began with)."""
-        key = (B, "pipe", slot, K)
+    def _enqueue_steps(self, B, slot, K, pair, ahead):
+        """K consecutive pipelined steps beginning on buffer set `slot`: K / 2 pairs, or K single steps."""
+        if pair:
+            for _ in range(K // 2):
+                self._enqueue_pair(B, slot)
+        else:
+            for i in range(K):
+                self._enqueue_pipelined_step(B, (slot + i) & 1, ahead)
+
+    def _pipe_graph(self, B, slot, K, pair, ahead):
+        """Graph of _enqueue_steps (K = 1, or an even count so that the graph ends on the set it began with)."""
+        key = (B, "pipe", slot, K, pair, ahead)
         g = self._graphs.get(key)
         if g is None:
-            def many():
-                for i in range(K):
-                    self._enqueue_pipelined_step(B, (slot + i) & 1)
-            g = self._graphs[key] = self._capture(many)
+            g = self._graphs[key] = self._capture(lambda: self._enqueue_steps(B, slot, K, pair, ahead))
         return g
 
     def _run_pipelined(self, B, n_steps, use_graph, launch):
@@ -1257,27 +1306,37 @@ class SvdEngine:
             self.stream_buffers(B, slot)
             self.workspace((B, slot))
         slot = getattr(self, "_primed", None)
+        ahead = self._ahead
         if slot is None:  # nothing assembled ahead for the batch at the cursor: prime set 0
-            slot = 0
+            slot, ahead = 0, 1
             if launch:
                 self._prefetch(B, 0, True, self._stream())
+        pair = self._pair_steps() and n_steps >= 2
+        if pair and ahead == 1:  # a pair steps two sorted batches: the one after the cursor into the other set
+            ahead = 2
+            if launch:
+                self._prefetch(B, 1 - slot, False, self._stream())
         # graphs of `self.graph_steps` consecutive steps: one launch per graph_steps steps instead of one per step --
-        # the gap between two graph launches is paid once per graph.  The remainder runs as single-step graphs.
+        # the gap between two graph launches is paid once per graph.  The remainder runs as graphs of one pair and of
+        # one single step.
         K = max(2, int(getattr(self, "graph_steps", 8)) // 2 * 2)
         done = 0
         while done < n_steps:
-            k = K if (use_graph and n_steps - done >= K) else 1
+            left = n_steps - done
+            k = K if (use_graph and left >= K) else (2 if pair and left >= 2 else 1)
+            p = pair and k >= 2
             if use_graph:
-                g = self._pipe_graph(B, slot, k)
+                g = self._pipe_graph(B, slot, k, p, ahead)
                 if launch:
                     check(self.L.tfr_graph_launch(g, self._stream()))
             elif launch:
-                self._enqueue_pipelined_step(B, slot)
+                self._enqueue_steps(B, slot, k, p, ahead)
             if k == 1:
                 slot = 1 - slot
             done += k
         if launch:
             self._primed = slot  # set `slot` now holds the batch at the (advanced) cursor
+            self._ahead = ahead
         return self.stream_buffers(B, 1 - slot)
 
     # ---- state access ------------------------------------------------------------------------------------

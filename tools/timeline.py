@@ -1,5 +1,7 @@
 """Per-kernel start/end times inside ONE graph-replayed train step, from in-kernel %globaltimer stamps
-(tfr_opt_set_timeline).  Usage (GPU box): python tools/timeline.py [workload] [overlap 0..3]"""
+(tfr_opt_set_timeline).  Usage (GPU box): python tools/timeline.py [workload] [overlap 0..3]
+TFR_TL_STEPS=2: one PAIR of steps per record (two steps per table pass): the slots of the forward / segment-sum kernels
+then span both steps' launches."""
 import os
 import sys
 
@@ -28,8 +30,9 @@ def main():
         eng.graph_steps = int(os.environ["TFR_GRAPH_STEPS"])
     eng.set_train_data(*cols)
     B, reps = w["B"], 12
+    per = int(os.environ.get("TFR_TL_STEPS", "1"))
     np.random.seed(1)
-    eng.set_index_stream(np.random.randint(0, len(cols[0]), (reps + 8) * B), B)
+    eng.set_index_stream(np.random.randint(0, len(cols[0]), (per * reps + 8) * B), B)
     eng.enable_timeline()
     eng.run_stream_steps(8, use_graph=use_graph, pipeline=pipeline)
     torch.cuda.synchronize()
@@ -37,11 +40,12 @@ def main():
     for _ in range(reps):
         eng.reset_timeline()
         torch.cuda.synchronize()
-        eng.run_stream_steps(1, use_graph=use_graph, pipeline=pipeline)
+        eng.run_stream_steps(per, use_graph=use_graph, pipeline=pipeline)
         torch.cuda.synchronize()
         for k, (a, b) in eng.read_timeline().items():
             acc.setdefault(k, []).append((a, b))
-    print("workload %s overlap=%d  (us from the step's first kernel entry; median of %d steps)" % (name, overlap, reps))
+    print("workload %s overlap=%d  (us from the first kernel entry of %d step(s); median of %d records)"
+          % (name, overlap, per, reps))
     end_all = 0
     for k in eng.TL_NAMES:
         if k in acc:
