@@ -62,7 +62,8 @@ int tfr_device_sm_count(void);
  * What a knob may change:
  *  - bit for bit the same results: SMEM_CARVEOUT, TILES_CARVEOUT, STREAM_LD, STREAM_ST, STREAM_CTAS_PER_SM,
  *    STREAM_UNROLL, STREAM_THREADS, STREAM_DYNAMIC, TL_EVERY_CTA, PDL, SORT_SPLIT, PASS_RING, RING_STAGES,
- *    RING_STAGE_KB, RING_THREADS, RING_L2_HINT, RING_CTAS_PER_SM, RING_SLOT_MODE 0..2, RANK_CHUNK;
+ *    RING_STAGE_KB, RING_THREADS, RING_L2_HINT, RING_CTAS_PER_SM, RING_SLOT_MODE 0..2, RANK_CHUNK, SEG_CHAIN (0 = the
+ *    fused segment sums of dim % 4 == 0 rows at four units per lane take segsum_tiles_kernel instead of chain.cu's kernel);
  *  - the fp32 rounding of the training step, within the oracle's 1e-5 bar: SEG_TILE (where runs of equal ids are
  *    regrouped into partial sums; its default depends on the batch size, the dim and the device's SM count) and
  *    SEG_MAX_UNITS (lanes per row, hence the order of the fused forward's dot products, and the default tile);

@@ -53,6 +53,9 @@ const TuneEntry kTune[TUNE_COUNT] = {
     // 111.1 / 112.6 / 121.4 ms at 1024 / 2048 / 4096 / 8192 / 16384 ratings per chunk; 4096 ties the fastest with a 224 MB
     // workspace (2048: 491 MB)
     {"ALS_CHUNK", 4096},
+    // 0: the fused segment sums take segsum_tiles_kernel<4, L, 4, true, false> where chain_tiles_kernel<L, T> would run;
+    // the two compute the same bits, and the old kernel is the reference the tests hold the chain kernel to
+    {"SEG_CHAIN", 1},
 };
 std::mutex g_tune_mu;
 int g_tune_val[TUNE_COUNT];

@@ -32,6 +32,7 @@ enum TuneKey {
   TUNE_RANK_CHUNK,        // tfr_rank_users: items per selection chunk (a multiple of 1024, 1024 .. 16384)
   TUNE_RANK_STAGES,       // debug: which kernels of tfr_rank_users run (1 score | 2 select | 4 merge)
   TUNE_ALS_CHUNK,         // ALS half-sweeps: ratings per Gram chunk of a heavy row (tfr_als_chunk: a multiple of 32)
+  TUNE_SEG_CHAIN,         // 0: the fused segment sums of chain geometries take segsum_tiles_kernel (chain.cu's reference)
   TUNE_COUNT
 };
 int tune(TuneKey k);

@@ -724,7 +724,7 @@ static int launch_segsum(const SegSide& su, const SegSide& si, int n_sides, cons
   if (g.vec == V && g.lanes == LL && units == UU) {                                                               \
     if (int rc = prep_tiles((const void*)segsum_fixup_kernel<V>, fix_smem)) return rc; /* same carve-out as the tiles */ \
     if (fw && generic) TFR_SEG_LAUNCH(V, LL, UU, true, true)                                                       \
-    else if (fw && V == 4 && UU == 4 && chain_tiles_supported(LL, tile)) {                                          \
+    else if (fw && V == 4 && UU == 4 && chain_tiles_supported(LL, tile) && tune(TUNE_SEG_CHAIN)) {                  \
       if (int rc = launch_chain_tiles(su, si, *fw, opt, B, dim, n_tiles, tile, LL, grid, pdl, st)) return rc;      \
     } else if (fw) TFR_SEG_LAUNCH(V, LL, UU, true, false)                                                          \
     else if (generic) TFR_SEG_LAUNCH(V, LL, UU, false, true)                                                       \

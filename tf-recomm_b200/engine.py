@@ -98,6 +98,17 @@ class IalsData(NamedTuple):
     objective: torch.Tensor
 
 
+def idle_slot_entry(global_step):
+    """The row -> slot map entry of a row no step has touched since global_step (signed int64): the stamp of the last
+    completed step, (global_step - 1) mod 2^32, with an index of all ones.  A single step and the bring of a pair look for
+    the stamp global_step, a pair's table pass for global_step + 1 and global_step, so no upcoming step matches it for
+    2^32 - 1 steps.  A constant -1 (stamp 0xffffffff) would match as soon as a step or a pair's pass reaches -1 (mod 2^32)
+    -- right after a restore to a step near it -- and every untouched row would read the summed gradient at index
+    0xffffffff, past the end of the workspace.  At step 0 it is -1, a fresh engine's entry."""
+    e = (((global_step - 1) & 0xffffffff) << 32) | 0xffffffff
+    return e - (1 << 64) if e >= 1 << 63 else e
+
+
 def _require_cuda():
     if not torch.cuda.is_available():
         raise TfrError("tf-recomm_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback for this path")
@@ -1392,8 +1403,10 @@ class SvdEngine:
             if not self.sgd and ("m_" + n) in z.files:
                 self.slots["m_" + n].copy_(torch.from_numpy(z["m_" + n].reshape(self.t[n].shape)))
                 self.slots["v_" + n].copy_(torch.from_numpy(z["v_" + n].reshape(self.t[n].shape)))
-        self.user_slot.fill_(-1)  # global_step is about to change: stale stamps must not become valid again
-        self.item_slot.fill_(-1)
+        # global_step is about to change: stale stamps must not become valid again (idle_slot_entry)
+        fill = idle_slot_entry(int(z["__step__"][0]))
+        self.user_slot.fill_(fill)
+        self.item_slot.fill_(fill)
         for field, val, dt in (("beta1_power", z["__opt__"][0], torch.float32), ("beta2_power", z["__opt__"][1], torch.float32),
                                ("global_step", z["__step__"][0], torch.int64)):
             off = getattr(OptScalars, field).offset
