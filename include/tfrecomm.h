@@ -490,6 +490,34 @@ int tfr_rank_users(const float* user_feat, const float* item_feat, const float* 
                    const int32_t* excl_item, double* topk_val, int32_t* topk_idx, void* workspace, int64_t workspace_bytes,
                    void* stream);
 
+/* ---- similar rows: exact float64 cosine top-k neighbours of query rows in their own table (items with items, users with
+ * users).  For a query row q and a candidate row v of the same table, both dim floats:
+ *  - acc = sum over d of (double)q[d] * (double)v[d], in d order from 0.0 (each product is exact in float64, so an FMA
+ *    changes no bit);
+ *  - |x| = __dsqrt_rn(sum over d of (double)x[d]^2), in d order from 0.0;
+ *  - cos(q, v) = __ddiv_rn(acc, __dmul_rn(|q|, |v|)), each step correctly rounded;
+ *  - abs_rows != 0 (items of the fork model, TFR_ABS_ITEM, which scores u.|q_i|): |q| and |v| elementwise are used in acc;
+ *    the norms are unchanged by this;
+ *  - a candidate is never returned if it is the query's own row (skip), if either row has norm 0, or if the score is not
+ *    finite; a zero query row therefore ranks nothing;
+ *  - order: score descending, then lowest id; k columns, padded with (-inf, -1): the rules of tfr_rank_users.
+ * Every score depends only on the two rows, so any chunking and any row sharding give the same bits.
+ * query_feat [n_query_rows] (query_stride floats between rows) is the table the queries are read from: query q is row
+ * query_rows[q] (device; repeats and any order allowed; an id outside [0, n_query_rows) gives a row of (-inf, -1) and is
+ * never read through).  feat [n_rows] (stride) holds the candidates.  skip[q] (device, may be null = none) is the candidate
+ * row never returned for query q, or -1.  On one GPU both are the same table and skip = query_rows; on a shard of a
+ * row-sharded table the query table is the gathered n-row table of the queries and skip is the query's local id on this
+ * rank, or -1.  Strides of 0 mean dim.  The norms of the candidate and query rows are computed on every call.
+ * TFR_ERR_INVALID before any CUDA call unless 1 <= dim <= 512, 1 <= k <= 1024, n_query_rows, n_rows, n_queries in
+ * [0, 2^31), strides >= dim, and query_rows, topk_val, topk_idx non-null when n_queries > 0 (query_feat when
+ * n_query_rows > 0, feat when n_rows > 0).  n_queries = 0 is a no-op.  workspace: tfr_similar_rows_workspace_bytes (a
+ * function of its arguments only; needs no device). */
+int64_t tfr_similar_rows_workspace_bytes(int64_t n_queries, int64_t n_rows, int32_t k);
+int tfr_similar_rows(const float* query_feat, int64_t n_query_rows, int64_t query_stride, const int32_t* query_rows,
+                     const int32_t* skip, int64_t n_queries, const float* feat, int64_t n_rows, int64_t stride, int32_t dim,
+                     int32_t abs_rows, int32_t k, double* topk_val, int32_t* topk_idx, void* workspace,
+                     int64_t workspace_bytes, void* stream);
+
 /* ---- fold-in of users that were not trained: exact least-squares user rows against the fixed item side -----------------
  * With item_feat, item_bias and mu fixed, the training loss (ops.py:81-89,124-126: squared error + reg * L2 on the gathered
  * rows, biases too with TFR_REG_BIAS) restricted to one user is a ridge regression in theta = [p_u ; b_u].  Its per-occurrence

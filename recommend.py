@@ -3,6 +3,7 @@
     python recommend.py --checkpoint fm.ckpt --users 3,17,42 --k 10                  # synthetic ml1m training split
     python recommend.py --checkpoint fm.ckpt --users 3 --dataset mydata --no-exclude
     python recommend.py --checkpoint fm.ckpt --fold-in new_users.csv --k 10            # users not in the checkpoint
+    python recommend.py --checkpoint fm.ckpt --similar-items 3,17,42 --k 10           # items like these items
 
 The model (shape and variant) comes from the checkpoint (SvdEngine.from_checkpoint); the path resolves as
 svd_train_val.py writes it, under config.BASE_DIR.  Unless --no-exclude is given, the items each user rated in the
@@ -16,9 +17,13 @@ against the checkpoint's item side, regularised by --reg, the training default o
 SvdEngine.rank_folded; unless --no-exclude is given, a label's own rated items are never recommended.  No training split is
 read.
 
+--similar-items ITEMS lists, for each given item, the items most like it by cosine of the item rows
+(SvdEngine.similar_items: exact float64, never the item itself).  No training split is read.
+
 stdout: one line per query user, in the order given (--fold-in: per distinct label, in order of first appearance):
 `user<TAB>item:score item:score ...` (scores %.6f; a user with fewer than k rankable items gets fewer pairs, a label that
-could not be folded in gets none and a note on stderr).  Everything else goes to stderr.
+could not be folded in gets none and a note on stderr); --similar-items: `item<TAB>item:score ...`, one line per given
+item.  Everything else goes to stderr.
 """
 import argparse
 import csv
@@ -41,6 +46,8 @@ def main(argv=None, out=None):
     who.add_argument("--users", type=str, help="comma-separated user ids")
     who.add_argument("--fold-in", dest="fold_in", type=str, default=None,
                      help="CSV with header user,item,rating: rank these users, folded into the model from their ratings")
+    who.add_argument("--similar-items", dest="similar_items", type=str, default=None,
+                     help="comma-separated item ids: list the items most like each of them (cosine of the item rows)")
     ap.add_argument("--reg", type=float, default=config.LAMBDA_REG,
                     help="L2 weight of the fold-in (the model's training reg; checkpoints do not record it)")
     ap.add_argument("--k", type=int, default=10)
@@ -52,6 +59,8 @@ def main(argv=None, out=None):
     args = ap.parse_args(argv)
     if args.fold_in is not None:
         return fold_in(args, out)
+    if args.similar_items is not None:
+        return similar_items(args, out)
     users = np.array([int(x) for x in args.users.split(",") if x.strip()], np.int64)
     eng = SvdEngine.from_checkpoint(os.path.join(config.BASE_DIR, args.checkpoint))
     exclude = None
@@ -100,6 +109,16 @@ def fold_in(args, out):
         if st != 0:
             print("user %s: could not be folded in (info %d): no recommendations" % (label, st), file=sys.stderr)
         out.write("%s\t%s\n" % (label, " ".join("%d:%.6f" % (i, v) for i, v in zip(row_i, row_v) if i >= 0)))
+    out.flush()
+
+
+def similar_items(args, out):
+    items = np.array([int(x) for x in args.similar_items.split(",") if x.strip()], np.int64)
+    eng = SvdEngine.from_checkpoint(os.path.join(config.BASE_DIR, args.checkpoint))
+    idx, val = eng.similar_items(items, k=args.k)
+    idx, val = idx.cpu().numpy(), val.cpu().numpy()
+    for i, row_i, row_v in zip(items, idx, val):
+        out.write("%d\t%s\n" % (i, " ".join("%d:%.6f" % (j, v) for j, v in zip(row_i, row_v) if j >= 0)))
     out.flush()
 
 

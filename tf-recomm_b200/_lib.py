@@ -163,6 +163,8 @@ _PROTOS = {
                                               i64, vp]),
     "tfr_rank_users_workspace_bytes": (i64, [i64, i64, i32]),
     "tfr_rank_users": (C.c_int, [vp, vp, vp, vp, vp, i64, i64, i32, i64, i64, i32, vp, i64, i32, vp, vp, vp, vp, vp, i64, vp]),
+    "tfr_similar_rows_workspace_bytes": (i64, [i64, i64, i32]),
+    "tfr_similar_rows": (C.c_int, [vp, i64, i64, vp, vp, i64, vp, i64, i64, i32, i32, i32, vp, vp, vp, i64, vp]),
     "tfr_fold_in_users": (C.c_int, [vp, vp, vp, i64, i32, i64, i32, f32, vp, vp, vp, i64, vp, vp, vp, vp]),
     "tfr_als_chunk": (i32, []),
     "tfr_als_workspace_bytes": (i64, [i64, i32]),

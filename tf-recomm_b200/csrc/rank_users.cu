@@ -13,6 +13,11 @@
 //  3. rank_users_merge_kernel: one warp per query merges the sorted chunk lists into the final k, padding with (-inf, -1).
 //     The chunks hold disjoint items and the order is total, so any chunking gives the same result.
 // Scores of at most RANK_SCORE_BUDGET bytes exist at a time: larger query batches are scored and selected in passes.
+//
+// tfr_similar_rows (the neighbours of query rows in their own table, by float64 cosine) runs the same select and merge
+// after two kernels of its own: row_norms_kernel (the norms of the candidate rows and of the query rows) and
+// similar_rows_score_kernel, the scorer's main loop with a cosine epilogue.  A NaN score is never ranked, so the query's
+// own row and zero rows need no exclusion list.
 #include <math.h>
 #include <string.h>
 
@@ -32,21 +37,26 @@ constexpr int RU_MAX_K = 1024;
 constexpr int64_t RU_SCORE_BUDGET = (int64_t)1 << 30;   // bytes of float64 scores per pass
 
 // ---- 1. scores -----------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(RU_THREADS) rank_users_score_kernel(
-    const float* __restrict__ U, const float* __restrict__ V, const float* __restrict__ ub, const float* __restrict__ ib,
-    const float* __restrict__ mu, int n_users, int n_items, int dim, int64_t us, int64_t is, bool abs_item,
-    const int32_t* __restrict__ query, int nb, double* __restrict__ scores) {
+// The main loop shared by the scorers: acc[x][y] = the in-order float64 dot product of query row ql = qrow + 4x of the
+// CTA's block (s_qid[ql] = its table row, -1 if padding or out of range) and item row i0 + icol + 8y.  kAbsQuery / abs_item:
+// the rows enter as |x|.  The epilogue gets (acc, s_qid, q0, qrow, i0, icol); a warp of padding rows does not call it.
+// tid is threadIdx.x read in the kernel, where __launch_bounds__ bounds it: read here, its range is lost, the loads are
+// unrolled differently, and rank_users_score_kernel would no longer compile to the instructions it had as a plain kernel.
+template <bool kAbsQuery, class Epilogue>
+__device__ __forceinline__ void ru_score_tile(const float* __restrict__ U, const float* __restrict__ V, int n_users,
+                                              int n_items, int dim, int64_t us, int64_t is, bool abs_item,
+                                              const int32_t* __restrict__ query, int nb, int tid, Epilogue epi) {
   __shared__ double sU[RU_DK][RU_QB + 1];
   __shared__ double sV[RU_DK][RU_IT + 1];
   __shared__ int s_qid[RU_QB];
   const int i0 = blockIdx.x * RU_IT, q0 = blockIdx.y * RU_QB;
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int lane = tid & 31, w = tid >> 5;
   const int tx = lane & 7, ty = lane >> 3;
   const int wq = w >> 2, wi = w & 3;
-  if (threadIdx.x < RU_QB) {
-    const int q = q0 + threadIdx.x;
+  if (tid < RU_QB) {
+    const int q = q0 + tid;
     int id = q < nb ? query[q] : -1;
-    s_qid[threadIdx.x] = (id >= 0 && id < n_users) ? id : -1;   // ids are device data: guarded here
+    s_qid[tid] = (id >= 0 && id < n_users) ? id : -1;   // ids are device data: guarded here
   }
   const bool active = q0 + wq * 16 < nb;   // (warp-uniform) a warp whose 16 query rows are all padding computes nothing
   double acc[4][4];
@@ -57,17 +67,17 @@ __global__ void __launch_bounds__(RU_THREADS) rank_users_score_kernel(
   __syncthreads();
   for (int d0 = 0; d0 < dim; d0 += RU_DK) {
     // coalesced: a warp reads 32 consecutive dims of one row
-    for (int e = threadIdx.x; e < RU_IT * RU_DK; e += RU_THREADS) {
+    for (int e = tid; e < RU_IT * RU_DK; e += RU_THREADS) {
       const int r = e / RU_DK, dd = e % RU_DK;
       float x = 0.0f;
       if (i0 + r < n_items && d0 + dd < dim) x = V[(size_t)(i0 + r) * is + d0 + dd];
       sV[dd][r] = (double)(abs_item ? fabsf(x) : x);
     }
-    for (int e = threadIdx.x; e < RU_QB * RU_DK; e += RU_THREADS) {
+    for (int e = tid; e < RU_QB * RU_DK; e += RU_THREADS) {
       const int r = e / RU_DK, dd = e % RU_DK;
       const int id = s_qid[r];
       const float x = (id >= 0 && d0 + dd < dim) ? U[(size_t)id * us + d0 + dd] : 0.0f;
-      sU[dd][r] = (double)x;
+      sU[dd][r] = (double)(kAbsQuery ? fabsf(x) : x);
     }
     __syncthreads();
     if (active) {
@@ -85,19 +95,94 @@ __global__ void __launch_bounds__(RU_THREADS) rank_users_score_kernel(
     __syncthreads();
   }
   if (!active) return;
-  const double m = (double)mu[0];
+  epi(acc, s_qid, q0, wq * 16 + ty, i0, wi * 32 + tx);
+}
+
+__global__ void __launch_bounds__(RU_THREADS) rank_users_score_kernel(
+    const float* __restrict__ U, const float* __restrict__ V, const float* __restrict__ ub, const float* __restrict__ ib,
+    const float* __restrict__ mu, int n_users, int n_items, int dim, int64_t us, int64_t is, bool abs_item,
+    const int32_t* __restrict__ query, int nb, double* __restrict__ scores) {
+  ru_score_tile<false>(U, V, n_users, n_items, dim, us, is, abs_item, query, nb, threadIdx.x,
+                [&](const double (&acc)[4][4], const int* s_qid, int q0, int qrow, int i0, int icol) {
+    const double m = (double)mu[0];
 #pragma unroll
-  for (int x = 0; x < 4; ++x) {
-    const int ql = wq * 16 + ty + 4 * x, q = q0 + ql;
-    const int id = s_qid[ql];
-    if (q >= nb || id < 0) continue;
-    const double bu = (double)ub[id];
+    for (int x = 0; x < 4; ++x) {
+      const int ql = qrow + 4 * x, q = q0 + ql;
+      const int id = s_qid[ql];
+      if (q >= nb || id < 0) continue;
+      const double bu = (double)ub[id];
 #pragma unroll
-    for (int y = 0; y < 4; ++y) {
-      const int it = i0 + wi * 32 + tx + 8 * y;
-      if (it < n_items) scores[(size_t)q * n_items + it] = __dadd_rn(__dadd_rn(__dadd_rn(acc[x][y], bu), (double)ib[it]), m);
+      for (int y = 0; y < 4; ++y) {
+        const int it = i0 + icol + 8 * y;
+        if (it < n_items) scores[(size_t)q * n_items + it] = __dadd_rn(__dadd_rn(__dadd_rn(acc[x][y], bu), (double)ib[it]), m);
+      }
     }
+  });
+}
+
+// tfr_similar_rows: cos = acc / (|q| |v|), each step correctly rounded.  NaN (never ranked, see ru_key) for the skipped
+// row and for a zero denominator.  Every other score is finite or NaN already: the norms of finite float rows are finite
+// and their product neither overflows nor underflows in float64, and an inf or NaN entry makes acc / (|q| |v|) a NaN.
+template <bool kAbs>
+__global__ void __launch_bounds__(RU_THREADS) similar_rows_score_kernel(
+    const float* __restrict__ Q, const float* __restrict__ V, int n_query_rows, int n_rows, int dim, int64_t qs, int64_t vs,
+    const int32_t* __restrict__ query, const int32_t* __restrict__ skip, int nb,
+    const double* __restrict__ qnorm, const double* __restrict__ vnorm, double* __restrict__ scores) {
+  ru_score_tile<kAbs>(Q, V, n_query_rows, n_rows, dim, qs, vs, kAbs, query, nb, threadIdx.x,
+                [&](const double (&acc)[4][4], const int* s_qid, int q0, int qrow, int i0, int icol) {
+    double vn[4];
+#pragma unroll
+    for (int y = 0; y < 4; ++y) vn[y] = i0 + icol + 8 * y < n_rows ? vnorm[i0 + icol + 8 * y] : 0.0;
+#pragma unroll
+    for (int x = 0; x < 4; ++x) {
+      const int ql = qrow + 4 * x, q = q0 + ql;
+      if (q >= nb || s_qid[ql] < 0) continue;
+      const double qn = qnorm[q];
+      const int sk = skip ? skip[q] : -1;
+#pragma unroll
+      for (int y = 0; y < 4; ++y) {
+        const int it = i0 + icol + 8 * y;
+        if (it >= n_rows) continue;
+        const double den = __dmul_rn(qn, vn[y]);
+        scores[(size_t)q * n_rows + it] = (it == sk || den == 0.0) ? __longlong_as_double(0x7ff8000000000000ll)
+                                                                   : __ddiv_rn(acc[x][y], den);
+      }
+    }
+  });
+}
+
+// The float64 norms of tfr_similar_rows: out[r] = sqrt(sum over d in order from 0.0 of (double)x[d]^2), x = table row r
+// (rows == null) or rows[r] (0 for an id outside [0, n_table)).  A CTA stages 32 dims of its 128 rows in shared memory
+// (a warp reads 32 consecutive dims of one row); each thread then sums its own row.
+constexpr int RN_ROWS = 128;
+__global__ void __launch_bounds__(RN_ROWS) row_norms_kernel(const float* __restrict__ X, int n_table, int64_t stride,
+                                                            int dim, const int32_t* __restrict__ rows, int n,
+                                                            double* __restrict__ out) {
+  __shared__ float s[RN_ROWS][RU_DK + 1];
+  __shared__ int s_row[RN_ROWS];
+  const int r0 = blockIdx.x * RN_ROWS;
+  {
+    const int r = r0 + threadIdx.x;
+    int id = r < n ? (rows ? rows[r] : r) : -1;
+    s_row[threadIdx.x] = (id >= 0 && id < n_table) ? id : -1;
   }
+  double acc = 0.0;
+  __syncthreads();
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  for (int d0 = 0; d0 < dim; d0 += RU_DK) {
+    for (int rr = w; rr < RN_ROWS; rr += RN_ROWS / 32) {
+      const int id = s_row[rr];
+      s[rr][lane] = (id >= 0 && d0 + lane < dim) ? X[(size_t)id * stride + d0 + lane] : 0.0f;
+    }
+    __syncthreads();
+    const int kmax = min(RU_DK, dim - d0);
+    for (int kk = 0; kk < kmax; ++kk) {
+      const double x = (double)s[threadIdx.x][kk];
+      acc = __fma_rn(x, x, acc);
+    }
+    __syncthreads();
+  }
+  if (r0 + threadIdx.x < n) out[r0 + threadIdx.x] = s_row[threadIdx.x] >= 0 ? __dsqrt_rn(acc) : 0.0;
 }
 
 // ---- 2. exact top-k of every (query, chunk) ----------------------------------------------------------------------------
@@ -341,6 +426,47 @@ extern "C" int64_t tfr_rank_users_workspace_bytes(int64_t n_queries, int64_t n_i
          align_up(parts * 4, 256) + align_up(n_queries * chunks * 4, 256);
 }
 
+// The passes of both entries: score(q0, nb, scores) scores queries q0 .. q0 + nb - 1 into scores [nb, n_items], then the
+// chunks are selected and merged.  query / n_query_rows: what the select kernel checks the ids against.
+template <class Score>
+static int ru_rank(Score score, const int32_t* query, int64_t n_query_rows, int64_t n_queries, int64_t n_items, int32_t k,
+                   const int64_t* excl_indptr, const int32_t* excl_item, double* topk_val, int32_t* topk_idx, void* workspace,
+                   cudaStream_t st) {
+  const int chunk = ru_chunk_items();
+  const int n_chunks = (int)((n_items + chunk - 1) / chunk);
+  const int64_t max_chunks = (n_items + RU_MIN_CHUNK - 1) / RU_MIN_CHUNK;
+  const int64_t nb_max = ru_pass_queries(n_queries, n_items);
+  char* w = reinterpret_cast<char*>(align_up((int64_t)(uintptr_t)workspace, 256));
+  double* scores = reinterpret_cast<double*>(w); w += align_up(nb_max * n_items * 8, 256);
+  double* part_val = reinterpret_cast<double*>(w); w += align_up(n_queries * max_chunks * k * 8, 256);
+  int32_t* part_idx = reinterpret_cast<int32_t*>(w); w += align_up(n_queries * max_chunks * k * 4, 256);
+  int32_t* heads = reinterpret_cast<int32_t*>(w);
+  const int stages = tune(TUNE_RANK_STAGES);
+  if (n_chunks > 0) {
+    const size_t smem = (size_t)chunk * 8;
+    TFR_CUDA(cudaFuncSetAttribute(rank_users_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    for (int64_t q0 = 0; q0 < n_queries; q0 += nb_max) {
+      const int nb = (int)(n_queries - q0 < nb_max ? n_queries - q0 : nb_max);
+      if (stages & 1) {
+        score(q0, nb, scores);
+        TFR_LAUNCH_CHECK();
+      }
+      if (stages & 2) {
+        rank_users_select_kernel<<<(unsigned)((int64_t)nb * n_chunks), RU_SEL_THREADS, smem, st>>>(
+            scores, (int)n_query_rows, (int)n_items, query, (int)q0, n_chunks, chunk, k, excl_indptr, excl_item, part_val,
+            part_idx);
+        TFR_LAUNCH_CHECK();
+      }
+    }
+  }
+  if (stages & 4) {
+    rank_users_merge_kernel<<<(unsigned)((n_queries + RU_MERGE_WARPS - 1) / RU_MERGE_WARPS), 32 * RU_MERGE_WARPS, 0, st>>>(
+        part_val, part_idx, heads, (int)n_queries, n_chunks, k, topk_val, topk_idx);
+    TFR_LAUNCH_CHECK();
+  }
+  return TFR_OK;
+}
+
 extern "C" int tfr_rank_users(const float* user_feat, const float* item_feat, const float* user_bias, const float* item_bias,
                               const float* mu, int64_t n_users, int64_t n_items, int32_t dim, int64_t user_stride,
                               int64_t item_stride, int32_t flags, const int32_t* query_users, int64_t n_queries, int32_t k,
@@ -362,41 +488,61 @@ extern "C" int tfr_rank_users(const float* user_feat, const float* item_feat, co
     return TFR_ERR_WORKSPACE;
   }
   cudaStream_t st = (cudaStream_t)stream;
-  const int chunk = ru_chunk_items();
-  const int n_chunks = (int)((n_items + chunk - 1) / chunk);
-  const int64_t max_chunks = (n_items + RU_MIN_CHUNK - 1) / RU_MIN_CHUNK;
-  const int64_t nb_max = ru_pass_queries(n_queries, n_items);
-  char* w = reinterpret_cast<char*>(align_up((int64_t)(uintptr_t)workspace, 256));
-  double* scores = reinterpret_cast<double*>(w); w += align_up(nb_max * n_items * 8, 256);
-  double* part_val = reinterpret_cast<double*>(w); w += align_up(n_queries * max_chunks * k * 8, 256);
-  int32_t* part_idx = reinterpret_cast<int32_t*>(w); w += align_up(n_queries * max_chunks * k * 4, 256);
-  int32_t* heads = reinterpret_cast<int32_t*>(w);
-  const int stages = tune(TUNE_RANK_STAGES);
   const bool abs_item = (flags & TFR_ABS_ITEM) != 0;
-  if (n_chunks > 0) {
-    const size_t smem = (size_t)chunk * 8;
-    TFR_CUDA(cudaFuncSetAttribute(rank_users_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    for (int64_t q0 = 0; q0 < n_queries; q0 += nb_max) {
-      const int nb = (int)(n_queries - q0 < nb_max ? n_queries - q0 : nb_max);
-      if (stages & 1) {
-        dim3 grid((unsigned)((n_items + RU_IT - 1) / RU_IT), (unsigned)((nb + RU_QB - 1) / RU_QB));
-        rank_users_score_kernel<<<grid, RU_THREADS, 0, st>>>(user_feat, item_feat, user_bias, item_bias, mu, (int)n_users,
-                                                             (int)n_items, dim, user_stride, item_stride, abs_item,
-                                                             query_users + q0, nb, scores);
-        TFR_LAUNCH_CHECK();
-      }
-      if (stages & 2) {
-        rank_users_select_kernel<<<(unsigned)((int64_t)nb * n_chunks), RU_SEL_THREADS, smem, st>>>(
-            scores, (int)n_users, (int)n_items, query_users, (int)q0, n_chunks, chunk, k, excl_indptr, excl_item, part_val,
-            part_idx);
-        TFR_LAUNCH_CHECK();
-      }
-    }
+  auto score = [&](int64_t q0, int nb, double* scores) {
+    dim3 grid((unsigned)((n_items + RU_IT - 1) / RU_IT), (unsigned)((nb + RU_QB - 1) / RU_QB));
+    rank_users_score_kernel<<<grid, RU_THREADS, 0, st>>>(user_feat, item_feat, user_bias, item_bias, mu, (int)n_users,
+                                                         (int)n_items, dim, user_stride, item_stride, abs_item,
+                                                         query_users + q0, nb, scores);
+  };
+  return ru_rank(score, query_users, n_users, n_queries, n_items, k, excl_indptr, excl_item, topk_val, topk_idx, workspace,
+                 st);
+}
+
+extern "C" int64_t tfr_similar_rows_workspace_bytes(int64_t n_queries, int64_t n_rows, int32_t k) {
+  const int64_t ru = tfr_rank_users_workspace_bytes(n_queries, n_rows, k);
+  if (ru < 0) return ru;
+  return ru + align_up(n_rows * 8, 256) + align_up(n_queries * 8, 256);
+}
+
+extern "C" int tfr_similar_rows(const float* query_feat, int64_t n_query_rows, int64_t query_stride,
+                                const int32_t* query_rows, const int32_t* skip, int64_t n_queries, const float* feat,
+                                int64_t n_rows, int64_t stride, int32_t dim, int32_t abs_rows, int32_t k, double* topk_val,
+                                int32_t* topk_idx, void* workspace, int64_t workspace_bytes, void* stream) {
+  TFR_CHECK_ARG(dim >= 1 && dim <= 512 && k >= 1 && k <= RU_MAX_K);
+  TFR_CHECK_ARG(n_query_rows >= 0 && n_query_rows < ((int64_t)1 << 31) && n_rows >= 0 && n_rows < ((int64_t)1 << 31));
+  TFR_CHECK_ARG(n_queries >= 0 && n_queries < ((int64_t)1 << 31));
+  if (query_stride == 0) query_stride = dim;
+  if (stride == 0) stride = dim;
+  TFR_CHECK_ARG(query_stride >= dim && stride >= dim);
+  if (n_queries == 0) return TFR_OK;
+  TFR_CHECK_ARG(query_rows && topk_val && topk_idx);
+  TFR_CHECK_ARG(n_query_rows == 0 || query_feat);
+  TFR_CHECK_ARG(n_rows == 0 || feat);
+  const int64_t need = tfr_similar_rows_workspace_bytes(n_queries, n_rows, k);
+  if (!workspace || workspace_bytes < need) {
+    set_error("similar_rows workspace too small (%lld bytes, need %lld)", (long long)workspace_bytes, (long long)need);
+    return TFR_ERR_WORKSPACE;
   }
-  if (stages & 4) {
-    rank_users_merge_kernel<<<(unsigned)((n_queries + RU_MERGE_WARPS - 1) / RU_MERGE_WARPS), 32 * RU_MERGE_WARPS, 0, st>>>(
-        part_val, part_idx, heads, (int)n_queries, n_chunks, k, topk_val, topk_idx);
+  cudaStream_t st = (cudaStream_t)stream;
+  // the norms go after the ranking's part of the workspace (ru_rank carves that from the aligned start)
+  char* w = reinterpret_cast<char*>(align_up((int64_t)(uintptr_t)workspace, 256)) +
+            (tfr_rank_users_workspace_bytes(n_queries, n_rows, k) - 256);
+  double* vnorm = reinterpret_cast<double*>(w); w += align_up(n_rows * 8, 256);
+  double* qnorm = reinterpret_cast<double*>(w);
+  if (n_rows > 0 && (tune(TUNE_RANK_STAGES) & 1)) {
+    row_norms_kernel<<<(unsigned)((n_rows + RN_ROWS - 1) / RN_ROWS), RN_ROWS, 0, st>>>(feat, (int)n_rows, stride, dim, nullptr,
+                                                                                       (int)n_rows, vnorm);
+    TFR_LAUNCH_CHECK();
+    row_norms_kernel<<<(unsigned)((n_queries + RN_ROWS - 1) / RN_ROWS), RN_ROWS, 0, st>>>(
+        query_feat, (int)n_query_rows, query_stride, dim, query_rows, (int)n_queries, qnorm);
     TFR_LAUNCH_CHECK();
   }
-  return TFR_OK;
+  auto score = [&](int64_t q0, int nb, double* scores) {
+    dim3 grid((unsigned)((n_rows + RU_IT - 1) / RU_IT), (unsigned)((nb + RU_QB - 1) / RU_QB));
+    auto kern = abs_rows ? similar_rows_score_kernel<true> : similar_rows_score_kernel<false>;
+    kern<<<grid, RU_THREADS, 0, st>>>(query_feat, feat, (int)n_query_rows, (int)n_rows, dim, query_stride, stride,
+                                      query_rows + q0, skip ? skip + q0 : nullptr, nb, qnorm + q0, vnorm, scores);
+  };
+  return ru_rank(score, query_rows, n_query_rows, n_queries, n_rows, k, nullptr, nullptr, topk_val, topk_idx, workspace, st);
 }

@@ -429,6 +429,47 @@ class SvdEngine:
                 val.data_ptr(), idx.data_ptr(), ws.data_ptr(), nbytes, self._stream()))
         return idx, val
 
+    # ---- similar items and users: float64 cosine neighbours in the factor space ------------------------------------------
+    def similar_items(self, items, k=10):
+        """The items most like each of items: -> (ids [n, k] int32, scores [n, k] float64) on the device, row q the
+        neighbours of items[q] by cosine of the item rows, k = min(k, I) (tfr_similar_rows: exact float64, score descending,
+        lowest id on ties, padded with (-inf, -1)).  An item is never its own neighbour, and a zero row has none and is
+        nobody's.  Ids may repeat, in any order; host or device.  The fork model (ABS_ITEM) compares |q_i|, the vectors its
+        score uses."""
+        self._check_ids([], items)
+        return self._similar(self.t["item_feat"], self.I, items, k, bool(self.flags & ABS_ITEM))
+
+    def similar_users(self, users, k=10):
+        """similar_items for users: the users whose rows are most like each of users[q] by cosine, k = min(k, U)."""
+        self._check_ids(users, [])
+        return self._similar(self.t["user_feat"], self.U, users, k, False)
+
+    def _similar(self, feat, n_rows, ids, k, abs_rows):
+        q = self._dev_i32(np.atleast_1d(np.asarray(ids)) if not isinstance(ids, torch.Tensor) else ids.reshape(-1))
+        return self._similar_rows(feat, n_rows, self.feat_stride, q, q, feat, n_rows, abs_rows, min(k, n_rows))
+
+    def _similar_rows(self, query_feat, n_query_rows, query_stride, q, skip, feat, n_rows, abs_rows, k):
+        """tfr_similar_rows of the query rows q (device int32) of query_feat against the candidate rows feat (this
+        engine's layout, feat_stride); skip: the candidate row never returned for each query, or -1 (device int32).  k
+        columns, padded with (-inf, -1) past the candidates (a shard of a row-sharded model ranks the k of the whole
+        table)."""
+        n, k = int(q.numel()), int(k)
+        dev = self.device
+        idx = torch.empty(n, k, dtype=torch.int32, device=dev)
+        val = torch.empty(n, k, dtype=torch.float64, device=dev)
+        if n == 0:
+            return idx, val
+        nbytes = check(self.L.tfr_similar_rows_workspace_bytes(n, n_rows, k))
+        key = ("similar_rows_ws", n, n_rows, k)   # serving calls of one shape reuse their workspace
+        ws = self._stage.get(key)
+        if ws is None:
+            ws = self._stage[key] = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        with torch.cuda.device(dev):
+            check(self.L.tfr_similar_rows(query_feat.data_ptr(), n_query_rows, query_stride, q.data_ptr(), skip.data_ptr(),
+                                          n, feat.data_ptr(), n_rows, self.feat_stride, self.d, int(abs_rows), k,
+                                          val.data_ptr(), idx.data_ptr(), ws.data_ptr(), nbytes, self._stream()))
+        return idx, val
+
     # ---- fold-in: user rows for users the model was not trained on ------------------------------------------------------
     def fold_in(self, rows, items, rates, n=None, reg=None):
         """Least-squares user rows for new users (or new ratings of known ones) against the trained item side: for each

@@ -12,9 +12,10 @@ Per step, on every rank (one process per GPU, torch.distributed/NCCL for the plu
 The exchange is ~68 MB per step against a 42.6 GB local table pass at G=8, so scaling is governed by the local pass
 (SURVEY 8e).  The reference has no distributed code; this is the B200-native equivalent north_star asks for.
 
-Serving (rank_users, fold_in, rank_folded) gives the single-GPU results, ids and bits, from the same sharded tables:
-query rows (or the rows of the rated items) are gathered to every rank the same way, every rank ranks its own item shard
-with the single-GPU kernel, and the per-rank lists are all-gathered and merged under the ranking's total order.
+Serving (rank_users, fold_in, rank_folded, similar_items, similar_users) gives the single-GPU results, ids and bits, from
+the same sharded tables: query rows (or the rows of the rated items) are gathered to every rank the same way, every rank
+ranks its own shard with the single-GPU kernel, and the per-rank lists are all-gathered and merged under the ranking's
+total order.
 """
 import ctypes as C
 
@@ -23,7 +24,7 @@ import torch
 import torch.distributed as dist
 
 from . import _lib, sharding
-from ._lib import LOSS_SIGMOID_CE, OPT_SGD, README_FLAGS, VAR_ALL, OptScalars, SvdTables, TfrError, check
+from ._lib import ABS_ITEM, LOSS_SIGMOID_CE, OPT_SGD, README_FLAGS, VAR_ALL, OptScalars, SvdTables, TfrError, check
 from .engine import FoldedUsers, PairCSR, SvdEngine
 
 
@@ -328,7 +329,8 @@ class ShardedSvdEngine:
         An all-reduce adds the +0.0 of the ranks that do not own a row, so an owned -0.0 arrives as +0.0.  No result bit
         depends on that: the scorer's dot product and the fold-in Gram and right-hand side are float64 sums that start
         from +0.0, a product with a zero factor is a zero, and in round-to-nearest +0.0 + (-0.0) = +0.0 + (+0.0) = +0.0,
-        so such a sum is never -0.0 and adding either zero to it (or a bias, or mu, after it) gives the same bits."""
+        so such a sum is never -0.0 and adding either zero to it (or a bias, or mu, after it) gives the same bits.  The
+        norms of similar_items / similar_users are such sums too: the square of either zero is +0.0."""
         m, d, e = ids.numel(), self.d, self.local
         flat = torch.empty(max(m * d + m, 1), dtype=torch.float32, device=self.device)
         keys = torch.empty(max(m, 1), dtype=torch.int32, device=self.device)
@@ -467,6 +469,48 @@ class ShardedSvdEngine:
         SvdEngine.fold_in refuses, with TfrError."""
         plan = self.fold_plan(rows, items, rates, n, reg)
         return self.fold_solve(plan, self._all_reduce(self.fold_gather(plan["ids"])))
+
+    def similar_gather(self, q, items):
+        """Phase 1 of similar_items / similar_users: the query rows (q device int32, global ids) this rank owns; summed over
+        the ranks (all-reduce) the buffer is the n-row table of the queries [n rows of d | n biases], row j = row q[j]
+        (items: the gather of fold_gather; users: the gather of serve_gather)."""
+        return self.fold_gather(q) if items else self.serve_gather(q)
+
+    def similar_rank(self, table, q, k, items):
+        """Phase 2: tfr_similar_rows of every gathered query row (table: similar_gather's buffer, all-reduced) against this
+        rank's shard of the same table -> (local ids [n, k], scores [n, k]).  The query's own row is skipped where this
+        rank owns it (local id q // G).  k: of the WHOLE table, so that every rank's list has the same shape."""
+        e, n, G = self.local, int(q.numel()), self.world
+        qi = q.to(torch.int64)
+        skip = torch.where(qi % G == self.rank, qi // G, -1).to(torch.int32).contiguous()
+        rows = torch.arange(n, dtype=torch.int32, device=self.device)
+        feat, n_loc = (e.t["item_feat"], self.I_loc) if items else (e.t["user_feat"], self.U_loc)
+        abs_rows = items and bool(e.flags & ABS_ITEM)
+        return e._similar_rows(table[:n * self.d], n, 0, rows, skip, feat, n_loc, abs_rows, k)
+
+    def _similar(self, ids, k, items):
+        if items:
+            self._check_ids([], ids)
+        else:
+            self._check_ids(ids, [])
+        q = self._dev_i32(np.atleast_1d(np.asarray(ids)) if not isinstance(ids, torch.Tensor) else ids.reshape(-1))
+        n, k = q.numel(), int(min(k, self.I if items else self.U))
+        if n == 0:
+            return (torch.empty(0, k, dtype=torch.int32, device=self.device),
+                    torch.empty(0, k, dtype=torch.float64, device=self.device))
+        with torch.cuda.device(self.device):
+            idx, val = self.similar_rank(self._all_reduce(self.similar_gather(q, items)), q, k, items)
+            return self.serve_merge(self._all_gather(val), self._all_gather(idx))
+
+    def similar_items(self, items, k=10):
+        """SvdEngine.similar_items on the sharded model: the same ids and bits as on the re-assembled tables.  Collective:
+        the query rows are gathered to every rank, each ranks its own item shard by cosine, and the per-rank lists are
+        all-gathered and merged (tfr_shard_topk_merge)."""
+        return self._similar(items, k, True)
+
+    def similar_users(self, users, k=10):
+        """SvdEngine.similar_users on the sharded model, as similar_items.  Collective."""
+        return self._similar(users, k, False)
 
     def rank_folded(self, folded, k=50, exclude_rated=True):
         """SvdEngine.rank_folded on the sharded item side, the same ids and bits.  The folded rows are on every rank
