@@ -32,6 +32,7 @@ the items they did not rate in training, and hit rate / precision / recall / NDC
 validation items (rated >= --topk-min-rating; on the DISCRETE branch, an outcome of 1).
 """
 import argparse
+import contextlib
 import os
 import time
 from collections import deque
@@ -54,6 +55,59 @@ def roc_auc(y_true, score):
     return float((r[y].sum() - n_pos * (n_pos + 1) / 2.0) / (n_pos * n_neg))
 
 
+def _graph(args):
+    """The reference's graph (:30-56): -> ((user, item, rate, wins, fails) placeholders, infer, logits, cost, train_op)."""
+    user_batch = ops.placeholder(ops.int32, shape=[None], name="id_user")
+    item_batch = ops.placeholder(ops.int32, shape=[None], name="id_item")
+    rate_batch = ops.placeholder(ops.float32, shape=[None])
+    wins_batch = ops.placeholder(ops.float32, shape=[None], name="nb_wins")
+    fails_batch = ops.placeholder(ops.float32, shape=[None], name="nb_fails")
+    ops.reset_default_graph()
+    infer, logits, regularizer, _, _, _, _ = ops.inference_svd(
+        user_batch, item_batch, wins_batch, fails_batch, user_num=args.user_num, item_num=args.item_num, dim=args.dim,
+        device=config.DEVICE, variant=args.variant)
+    ops.train.get_or_create_global_step()
+    cost, train_op = ops.optimization(infer, logits, regularizer, rate_batch, learning_rate=args.lr, reg=args.reg,
+                                      device=config.DEVICE)
+    return (user_batch, item_batch, rate_batch, wins_batch, fails_batch), infer, logits, cost, train_op
+
+
+@contextlib.contextmanager
+def _session(args, log):
+    """The reference's graph in an initialised session (:30-57): -> (sess, engine, writer, _graph's tuple), writer the
+    TensorBoard FileWriter or None.  When the training loop is done: the writer closed and the checkpoint (:197-198)."""
+    graph = _graph(args)
+    init_op = ops.group(ops.global_variables_initializer(), ops.local_variables_initializer())
+    saver = ops.train.Saver()
+    with ops.Session() as sess:
+        sess.run(init_op)
+        writer = summary.FileWriter(args.logdir) if getattr(args, "logdir", None) else None   # :57
+        yield sess, ops.session.current_model().engine, writer, graph
+        if writer is not None:
+            writer.close()
+        if args.checkpoint:
+            path = os.path.join(config.BASE_DIR, args.checkpoint)
+            log(path)
+            saver.save(sess, path)
+
+
+def _topk(engine, k, test, min_rating, exclude, rec, log):
+    """A report's TOPK line: top-k quality on the validation split (SvdEngine.ranking_metrics), kept in rec["topk"].
+    -> the seconds it took, which the next report's elapsed time leaves out."""
+    t_topk = time.time()
+    rm = engine.ranking_metrics(k, test["user"], test["item"], rates=test["outcome"], min_rating=min_rating,
+                                exclude=exclude)
+    rec["topk"] = rm
+    log("TOPK(k={:d}, users={:d}, hr={:f}, precision={:f}, recall={:f}, ndcg={:f})".format(
+        k, rm["n_users"], rm["hr"], rm["precision"], rm["recall"], rm["ndcg"]))
+    return time.time() - t_topk
+
+
+def _topk_summaries(writer, rm, step):
+    for tag, key in (("hr_at_k", "hr"), ("precision_at_k", "precision"), ("recall_at_k", "recall"), ("ndcg_at_k", "ndcg")):
+        writer.add_summary(summary.make_scalar_summary(tag, rm[key]), step)
+
+
 def svd(train, test, args, log=print):
     BATCH_SIZE = args.batch
     nb_batches = len(train["user"]) // BATCH_SIZE
@@ -62,27 +116,9 @@ def svd(train, test, args, log=print):
     cols = ["user", "item", "outcome", "wins", "fails"]
     iter_train = dataio.ShuffleIterator([train[c] for c in cols], batch_size=BATCH_SIZE)
     iter_test = dataio.OneEpochIterator([test[c] for c in cols], batch_size=-1)
-
-    user_batch = ops.placeholder(ops.int32, shape=[None], name="id_user")
-    item_batch = ops.placeholder(ops.int32, shape=[None], name="id_item")
-    rate_batch = ops.placeholder(ops.float32, shape=[None])
-    wins_batch = ops.placeholder(ops.float32, shape=[None], name="nb_wins")
-    fails_batch = ops.placeholder(ops.float32, shape=[None], name="nb_fails")
-
-    ops.reset_default_graph()
-    infer, logits, regularizer, user_bias, user_features, item_bias, item_features = ops.inference_svd(
-        user_batch, item_batch, wins_batch, fails_batch, user_num=args.user_num, item_num=args.item_num, dim=args.dim,
-        device=config.DEVICE, variant=args.variant)
-    ops.train.get_or_create_global_step()
-    cost, train_op = ops.optimization(infer, logits, regularizer, rate_batch, learning_rate=args.lr, reg=args.reg,
-                                      device=config.DEVICE)
-    init_op = ops.group(ops.global_variables_initializer(), ops.local_variables_initializer())
-    saver = ops.train.Saver()
     history = []
-    with ops.Session() as sess:
-        sess.run(init_op)
-        engine = ops.session.current_model().engine
-        writer = summary.FileWriter(args.logdir) if getattr(args, "logdir", None) else None   # :57
+    with _session(args, log) as (sess, engine, writer, graph):
+        (user_batch, item_batch, rate_batch, wins_batch, fails_batch), infer, logits, cost, train_op = graph
         log("{} {} {} {}".format("epoch", "train_error", "val_error", "elapsed_time"))
         train_se = deque(maxlen=nb_batches)
         train_nll = deque(maxlen=nb_batches)
@@ -194,13 +230,7 @@ def svd(train, test, args, log=print):
                 log("{:3d} TRAIN(size={:d}/{:d}, rmse={:f}) TEST(size={:d}, rmse={:f}) {:f}(s)".format(
                     epoch, last_batch, len(train["user"]), train_rmse, len(test["user"]), test_rmse, end - start))
             if topk:
-                t_topk = time.time()
-                rm = engine.ranking_metrics(topk, test["user"], test["item"], rates=test["outcome"],
-                                            min_rating=topk_min_rating, exclude=topk_exclude)
-                rec["topk"] = rm
-                log("TOPK(k={:d}, users={:d}, hr={:f}, precision={:f}, recall={:f}, ndcg={:f})".format(
-                    topk, rm["n_users"], rm["hr"], rm["precision"], rm["recall"], rm["ndcg"]))
-                end += time.time() - t_topk   # the next report's elapsed time is the training's alone
+                end += _topk(engine, topk, test, topk_min_rating, topk_exclude, rec, log)
             history.append(rec)
             if writer is not None:
                 # svd_train_val.py:189-192: train_rmse / test_rmse under these two tags (NaN on the DISCRETE branch, where
@@ -211,42 +241,19 @@ def svd(train, test, args, log=print):
                     for tag in ("train_macc", "train_mauc", "train_mnll", "test_macc", "test_auc", "test_mnll"):
                         writer.add_summary(summary.make_scalar_summary(tag, rec[tag]), report_at)
                 if topk:
-                    for tag, key in (("hr_at_k", "hr"), ("precision_at_k", "precision"), ("recall_at_k", "recall"),
-                                     ("ndcg_at_k", "ndcg")):
-                        writer.add_summary(summary.make_scalar_summary(tag, rec["topk"][key]), report_at)
+                    _topk_summaries(writer, rec["topk"], report_at)
                 writer.flush()
             start = end
-        if writer is not None:
-            writer.close()
-        if args.checkpoint:
-            path = os.path.join(config.BASE_DIR, args.checkpoint)
-            log(path)
-            saver.save(sess, path)
     return history
 
 
 def svd_als(train, test, args, log=print):
     """--solver als: the same model, initialisation, report lines, --topk, summaries and checkpoint as svd(), trained by one
     ALS sweep per epoch.  TRAIN(size=N/N) is the RMSE over every training rating (tfr_svd_objective), TEST the forward's."""
-    user_batch = ops.placeholder(ops.int32, shape=[None], name="id_user")
-    item_batch = ops.placeholder(ops.int32, shape=[None], name="id_item")
-    rate_batch = ops.placeholder(ops.float32, shape=[None])
-    wins_batch = ops.placeholder(ops.float32, shape=[None], name="nb_wins")
-    fails_batch = ops.placeholder(ops.float32, shape=[None], name="nb_fails")
-    ops.reset_default_graph()
-    infer, logits, regularizer, _, _, _, _ = ops.inference_svd(
-        user_batch, item_batch, wins_batch, fails_batch, user_num=args.user_num, item_num=args.item_num, dim=args.dim,
-        device=config.DEVICE, variant=args.variant)
-    ops.train.get_or_create_global_step()
-    ops.optimization(infer, logits, regularizer, rate_batch, learning_rate=args.lr, reg=args.reg, device=config.DEVICE)
-    init_op = ops.group(ops.global_variables_initializer(), ops.local_variables_initializer())
-    saver = ops.train.Saver()
     history = []
     n_train, n_test = len(train["user"]), len(test["user"])
-    with ops.Session() as sess:
-        sess.run(init_op)
-        engine = ops.session.current_model().engine
-        writer = summary.FileWriter(args.logdir) if getattr(args, "logdir", None) else None
+    with _session(args, log) as (sess, engine, writer, graph):
+        (user_batch, item_batch, _, wins_batch, fails_batch), infer, logits, _, _ = graph
         data = engine.als_data(train["user"], train["item"], train["outcome"])
         topk = int(getattr(args, "topk", 0) or 0)
         if topk:
@@ -271,53 +278,23 @@ def svd_als(train, test, args, log=print):
             log("{:3d} TRAIN(size={:d}/{:d}, rmse={:f}) TEST(size={:d}, rmse={:f}) {:f}(s)".format(
                 epoch, n_train, n_train, train_rmse, n_test, test_rmse, end - start))
             if topk:
-                t_topk = time.time()
-                rm = engine.ranking_metrics(topk, test["user"], test["item"], rates=test["outcome"],
-                                            min_rating=float(args.topk_min_rating), exclude=topk_exclude)
-                rec["topk"] = rm
-                log("TOPK(k={:d}, users={:d}, hr={:f}, precision={:f}, recall={:f}, ndcg={:f})".format(
-                    topk, rm["n_users"], rm["hr"], rm["precision"], rm["recall"], rm["ndcg"]))
-                end += time.time() - t_topk
+                end += _topk(engine, topk, test, float(args.topk_min_rating), topk_exclude, rec, log)
             history.append(rec)
             if writer is not None:
                 writer.add_summary(summary.make_scalar_summary("training_error", train_rmse), epoch)
                 writer.add_summary(summary.make_scalar_summary("test_error", test_rmse), epoch)
                 if topk:
-                    for tag, key in (("hr_at_k", "hr"), ("precision_at_k", "precision"), ("recall_at_k", "recall"),
-                                     ("ndcg_at_k", "ndcg")):
-                        writer.add_summary(summary.make_scalar_summary(tag, rec["topk"][key]), epoch)
+                    _topk_summaries(writer, rec["topk"], epoch)
                 writer.flush()
             start = end
-        if writer is not None:
-            writer.close()
-        if args.checkpoint:
-            path = os.path.join(config.BASE_DIR, args.checkpoint)
-            log(path)
-            saver.save(sess, path)
     return history
 
 
 def svd_ials(train, test, args, log=print):
     """--solver ials: the same model, initialisation, --topk lines, summaries and checkpoint as svd(), trained by one iALS
     sweep per epoch from the training pairs as implicit feedback.  IMPLICIT(...) is the loss after the sweep."""
-    user_batch = ops.placeholder(ops.int32, shape=[None], name="id_user")
-    item_batch = ops.placeholder(ops.int32, shape=[None], name="id_item")
-    rate_batch = ops.placeholder(ops.float32, shape=[None])
-    wins_batch = ops.placeholder(ops.float32, shape=[None], name="nb_wins")
-    fails_batch = ops.placeholder(ops.float32, shape=[None], name="nb_fails")
-    ops.reset_default_graph()
-    infer, logits, regularizer, _, _, _, _ = ops.inference_svd(
-        user_batch, item_batch, wins_batch, fails_batch, user_num=args.user_num, item_num=args.item_num, dim=args.dim,
-        device=config.DEVICE, variant=args.variant)
-    ops.train.get_or_create_global_step()
-    ops.optimization(infer, logits, regularizer, rate_batch, learning_rate=args.lr, reg=args.reg, device=config.DEVICE)
-    init_op = ops.group(ops.global_variables_initializer(), ops.local_variables_initializer())
-    saver = ops.train.Saver()
     history = []
-    with ops.Session() as sess:
-        sess.run(init_op)
-        engine = ops.session.current_model().engine
-        writer = summary.FileWriter(args.logdir) if getattr(args, "logdir", None) else None
+    with _session(args, log) as (sess, engine, writer, _):
         data = engine.ials_data(train["user"], train["item"])
         topk_exclude = engine.pair_csr(train["user"], train["item"])
         log("{} {} {}".format("epoch", "implicit_loss", "elapsed_time"))
@@ -332,27 +309,13 @@ def svd_ials(train, test, args, log=print):
             rec = dict(epoch=epoch, implicit_loss=obj["loss"], elapsed=end - start)
             log("{:3d} IMPLICIT(pairs={:d}, loss={:.10g}, observed={:.10g}, all_pairs={:.10g}, penalty={:.10g}) {:f}(s)"
                 .format(epoch, obj["n"], obj["loss"], obj["observed"], obj["all_pairs"], obj["penalty"], end - start))
-            t_topk = time.time()
-            rm = engine.ranking_metrics(args.topk, test["user"], test["item"], rates=test["outcome"],
-                                        min_rating=float(args.topk_min_rating), exclude=topk_exclude)
-            rec["topk"] = rm
-            log("TOPK(k={:d}, users={:d}, hr={:f}, precision={:f}, recall={:f}, ndcg={:f})".format(
-                args.topk, rm["n_users"], rm["hr"], rm["precision"], rm["recall"], rm["ndcg"]))
-            end += time.time() - t_topk
+            end += _topk(engine, args.topk, test, float(args.topk_min_rating), topk_exclude, rec, log)
             history.append(rec)
             if writer is not None:
                 writer.add_summary(summary.make_scalar_summary("implicit_loss", obj["loss"]), epoch)
-                for tag, key in (("hr_at_k", "hr"), ("precision_at_k", "precision"), ("recall_at_k", "recall"),
-                                 ("ndcg_at_k", "ndcg")):
-                    writer.add_summary(summary.make_scalar_summary(tag, rm[key]), epoch)
+                _topk_summaries(writer, rec["topk"], epoch)
                 writer.flush()
             start = end
-        if writer is not None:
-            writer.close()
-        if args.checkpoint:
-            path = os.path.join(config.BASE_DIR, args.checkpoint)
-            log(path)
-            saver.save(sess, path)
     return history
 
 

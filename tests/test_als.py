@@ -142,13 +142,14 @@ def test_als_kernels_compile_without_spills(tmp_path):
                                    os.path.join(ROOT, "tf-recomm_b200", "csrc", src), "-o", obj],
                                   stdout=f, stderr=subprocess.STDOUT)
         info.update(_ptxas_lines(log))
-    names = {"tfr::als_rows_kernel", "tfr::als_chunk_gram_kernel", "tfr::als_heavy_solve_kernel",
-             "tfr::als_objective_rows_kernel", "tfr::als_objective_finish_kernel", "tfr::fold_in_kernel"}
+    half_sweep = ["void tfr::half_sweep_%s_kernel<tfr::FiForm<true, false, true> >" % k   # FiRatings
+                  for k in ("rows", "chunk_gram", "heavy_solve")]
+    names = {*half_sweep, "tfr::als_objective_rows_kernel", "tfr::als_objective_finish_kernel", "tfr::fold_in_kernel"}
     assert names <= set(info), sorted(info)
     for name in names:
         regs, stack, st, ld = info[name]
         assert (stack, st, ld) == (0, 0, 0), (name, info[name])
-    for name in ("tfr::als_rows_kernel", "tfr::als_chunk_gram_kernel", "tfr::als_heavy_solve_kernel", "tfr::fold_in_kernel"):
+    for name in (*half_sweep, "tfr::fold_in_kernel"):
         assert info[name][0] <= 128, (name, info[name])   # __launch_bounds__(256, 2): two CTAs per SM
 
 

@@ -149,20 +149,23 @@ def test_workspace_sizes():
 @pytest.mark.skipif(not os.path.exists(NVCC), reason="needs the CUDA toolkit")
 def test_ials_kernels_compile_without_spills(tmp_path):
     from test_rank_users import _ptxas_lines
-    obj, log = str(tmp_path / "ials.o"), str(tmp_path / "ptxas.txt")
-    with open(log, "w") as f:
-        subprocess.check_call([NVCC, "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-ccbin",
-                               "/usr/bin/g++", "-Xcompiler", "-fPIC", "-Xptxas", "-v", "-c",
-                               os.path.join(ROOT, "tf-recomm_b200", "csrc", "ials.cu"), "-o", obj],
-                              stdout=f, stderr=subprocess.STDOUT)
-    info = _ptxas_lines(log)
-    names = {"tfr::gram_rows_kernel", "tfr::gram_combine_kernel", "tfr::ials_rows_kernel", "tfr::ials_chunk_gram_kernel",
-             "tfr::ials_heavy_solve_kernel", "tfr::ials_objective_rows_kernel", "tfr::ials_objective_finish_kernel"}
+    info = {}
+    for src in ("ials.cu", "als.cu"):   # als.cu: the half-sweep kernels, one template with ALS's
+        obj, log = str(tmp_path / (src + ".o")), str(tmp_path / (src + ".txt"))
+        with open(log, "w") as f:
+            subprocess.check_call([NVCC, "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-ccbin",
+                                   "/usr/bin/g++", "-Xcompiler", "-fPIC", "-Xptxas", "-v", "-c",
+                                   os.path.join(ROOT, "tf-recomm_b200", "csrc", src), "-o", obj],
+                                  stdout=f, stderr=subprocess.STDOUT)
+        info.update(_ptxas_lines(log))
+    half_sweep = ["void tfr::half_sweep_%s_kernel<tfr::FiForm<false, true, false> >" % k   # FiImplicit
+                  for k in ("rows", "chunk_gram", "heavy_solve")]
+    names = {"tfr::gram_rows_kernel", "tfr::gram_combine_kernel", *half_sweep, "tfr::ials_objective_rows_kernel",
+             "tfr::ials_objective_finish_kernel"}
     assert names <= set(info), sorted(info)
     for name in names:
         assert tuple(info[name][1:]) == (0, 0, 0), (name, info[name])
-    for name in ("tfr::gram_rows_kernel", "tfr::ials_rows_kernel", "tfr::ials_chunk_gram_kernel",
-                 "tfr::ials_heavy_solve_kernel"):
+    for name in ("tfr::gram_rows_kernel", *half_sweep):
         assert info[name][0] <= 128, (name, info[name])   # __launch_bounds__(256, 2): two CTAs per SM
 
 

@@ -1,4 +1,4 @@
-// Device code shared by fold-in (fold_in.cu), the ALS half-sweeps (als.cu) and the iALS half-sweeps (ials.cu): the float64
+// Device code shared by fold-in (fold_in.cu), the ALS and iALS half-sweeps (als.cu) and the iALS Gram (ials.cu): the float64
 // normal equations of one row of the model with the other side fixed, built in shared memory, factored and solved by one
 // CTA.  The form of the system is a compile-time parameter (FiForm).  Explicit ratings (FiRatings, fold-in and ALS):
 //     (sum_j x_j x_j^T + reg * n * D) theta = sum_j (r_j - mu - b_{k_j}) x_j,   x_j = [v~_{k_j} ; 1],
@@ -15,6 +15,7 @@
 //    (a warp per trailing row).
 //  - fi_solve: forward / back substitution by one warp with the right-hand side in registers.
 #pragma once
+#include <float.h>
 #include <math.h>
 
 #include "common.cuh"
@@ -235,5 +236,16 @@ __device__ __forceinline__ void fi_solve(const double* tri, const double* rhs, i
     }
   }
 }
+
+// ---- host helpers of the ALS and iALS entry points (als.cu, ials.cu) --------------------------------------------------
+constexpr int OBJ_WARPS = 8, OBJ_MAX_BLOCKS = 1024;   // the objectives' row kernels: warps per block, blocks at most
+
+inline int objective_blocks(int64_t n_rows) {
+  const int64_t b = (n_rows + OBJ_WARPS - 1) / OBJ_WARPS;
+  return (int)(b < 1 ? 1 : (b < OBJ_MAX_BLOCKS ? b : OBJ_MAX_BLOCKS));
+}
+
+inline bool reg_ok(float reg) { return reg > 0.0f && reg <= FLT_MAX; }          // refuses 0, negative, NaN and infinite
+inline bool alpha_ok(float alpha) { return alpha >= 0.0f && alpha <= FLT_MAX; }   // refuses negative, NaN and infinite
 
 }  // namespace tfr

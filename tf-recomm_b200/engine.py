@@ -9,6 +9,7 @@ import contextlib
 import ctypes as C
 import os
 import time
+from types import SimpleNamespace
 from typing import NamedTuple
 
 import numpy as np
@@ -107,6 +108,25 @@ def idle_slot_entry(global_step):
     0xffffffff, past the end of the workspace.  At step 0 it is -1, a fresh engine's entry."""
     e = (((global_step - 1) & 0xffffffff) << 32) | 0xffffffff
     return e - (1 << 64) if e >= 1 << 63 else e
+
+
+def csr_of(rows, cols, n_rows, n_cols, vals=None):
+    """Entries (rows, cols[, vals]) -- int64 device tensors, ids in range -- as CSR over n_rows rows, entries in stable
+    (row, col) order: -> (indptr int64 [n_rows + 1], partner int32, vals in that order | None).  Entries already in that
+    order keep it."""
+    order = torch.argsort(rows * n_cols + cols, stable=True)
+    indptr = torch.zeros(n_rows + 1, dtype=torch.int64, device=rows.device)
+    indptr[1:] = torch.cumsum(torch.bincount(rows, minlength=n_rows), 0)
+    return indptr, cols[order].to(torch.int32).contiguous(), None if vals is None else vals[order].contiguous()
+
+
+def check_lengths(name, what, *arrays):
+    """The sizes of host or device arrays of one entry each -> their common size; TfrError '<name>: <what> differ in
+    length' when they differ."""
+    sizes = [a.numel() if isinstance(a, torch.Tensor) else np.asarray(a).size for a in arrays]
+    if len(set(sizes)) != 1:
+        raise TfrError("%s: %s differ in length: %s" % (name, what, sizes))
+    return sizes[0]
 
 
 def _require_cuda():
@@ -484,11 +504,9 @@ class SvdEngine:
         reg = self.hyper["reg"] if reg is None else float(reg)
         if not reg >= 0.0:
             raise TfrError("fold_in: reg must be >= 0, got %r" % reg)
-        sizes = [a.numel() if isinstance(a, torch.Tensor) else np.asarray(a).size for a in (rows, items, rates)]
-        if len(set(sizes)) != 1:
-            raise TfrError("fold_in: rows, items and rates differ in length: %s" % sizes)
+        size = check_lengths("fold_in", "rows, items and rates", rows, items, rates)
         if n is None:
-            n = int((rows if isinstance(rows, torch.Tensor) else np.asarray(rows)).max()) + 1 if sizes[0] else 0
+            n = int((rows if isinstance(rows, torch.Tensor) else np.asarray(rows)).max()) + 1 if size else 0
         n = int(n)
         indptr, it, rt = self._csr_by_user(rows, items, rates, n_rows=n)
         dev = self.device
@@ -537,29 +555,27 @@ class SvdEngine:
         chunk_heavy = torch.repeat_interleave(torch.arange(heavy.numel(), dtype=torch.int32, device=self.device), n_chunk)
         return AlsPlan(light, heavy.to(torch.int32), heavy_ptr, chunk_heavy)
 
+    def _plans(self, u, i, vals, csr_type, ws_bytes, *other_bytes):
+        """Both CSRs of the entries (u, i, vals) (int64 user / item ids on the device) as csr_type, the plan of each
+        half-sweep at the ALS_CHUNK knob as it is now, and one workspace for both half-sweeps (ws_bytes(n_chunks, d)) and
+        the other calls' byte counts: -> (by_user, by_item, user_plan, item_plan, chunk, workspace)."""
+        by_user, by_item = csr_type(*csr_of(u, i, self.U, self.I, vals)), csr_type(*csr_of(i, u, self.I, self.U, vals))
+        chunk = int(self.L.tfr_als_chunk())
+        up, ip = self._als_plan(by_user.indptr, chunk), self._als_plan(by_item.indptr, chunk)
+        nbytes = max(*(check(ws_bytes(p.chunk_heavy.numel(), self.d)) for p in (up, ip)), *other_bytes)
+        return by_user, by_item, up, ip, chunk, torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+
     def als_data(self, users, items, rates):
         """A training set (one rating per entry, duplicates count; host or device arrays) prepared for als_sweep and
         training_objective: both CSRs and the plan of each half-sweep, built once on the device.  The heavy-row threshold is
         the ALS_CHUNK knob (tfr_als_chunk) as it is now; the plan keeps it."""
         self._als_refuse()
-        sizes = [a.numel() if isinstance(a, torch.Tensor) else np.asarray(a).size for a in (users, items, rates)]
-        if len(set(sizes)) != 1:
-            raise TfrError("als_data: users, items and rates differ in length: %s" % sizes)
+        check_lengths("als_data", "users, items and rates", users, items, rates)
         self._check_ids(users, items)
         u, i = self._dev_i32(users).to(torch.int64), self._dev_i32(items).to(torch.int64)
-        r = self._dev_f32(rates)
-        by = {}
-        for name, rows, cols, n_rows, n_cols in (("user", u, i, self.U, self.I), ("item", i, u, self.I, self.U)):
-            order = torch.argsort(rows * n_cols + cols, stable=True)
-            indptr = torch.zeros(n_rows + 1, dtype=torch.int64, device=self.device)
-            indptr[1:] = torch.cumsum(torch.bincount(rows, minlength=n_rows), 0)
-            by[name] = RatingCSR(indptr, cols[order].to(torch.int32).contiguous(), r[order].contiguous())
-        chunk = int(self.L.tfr_als_chunk())
-        up, ip = self._als_plan(by["user"].indptr, chunk), self._als_plan(by["item"].indptr, chunk)
-        nbytes = max(check(self.L.tfr_als_workspace_bytes(p.chunk_heavy.numel(), self.d)) for p in (up, ip))
-        nbytes = max(nbytes, check(self.L.tfr_svd_objective_workspace_bytes(self.U, self.I)))
         dev = self.device
-        return AlsData(by["user"], by["item"], up, ip, chunk, torch.empty(nbytes, dtype=torch.uint8, device=dev),
+        return AlsData(*self._plans(u, i, self._dev_f32(rates), RatingCSR, self.L.tfr_als_workspace_bytes,
+                                    check(self.L.tfr_svd_objective_workspace_bytes(self.U, self.I))),
                        torch.zeros(1, dtype=torch.int32, device=dev), torch.zeros(6, dtype=torch.float64, device=dev))
 
     def _half_sweep(self, data, reg, csr, plan, fixed, solved):
@@ -618,10 +634,7 @@ class SvdEngine:
         """(row, item[, weight]) entries -> the distinct pairs sorted by (row, item): (row int64, item int64, weight float32),
         each pair's weight the sum of its entries' weights (1 each by default), summed in float64 in the entries' order
         (torch.segment_reduce: one sequential sum per pair, so the same entries give the same bits)."""
-        sizes = [a.numel() if isinstance(a, torch.Tensor) else np.asarray(a).size
-                 for a in ((rows, items) if weights is None else (rows, items, weights))]
-        if len(set(sizes)) != 1:
-            raise TfrError("%s: rows, items and weights differ in length: %s" % (name, sizes))
+        check_lengths(name, "rows, items and weights", *((rows, items) if weights is None else (rows, items, weights)))
         self._check_ids(rows, items, n_rows)
         r, i = self._dev_i32(rows).to(torch.int64), self._dev_i32(items).to(torch.int64)
         w = torch.ones(r.numel(), dtype=torch.float32, device=self.device) if weights is None else self._dev_f32(weights)
@@ -648,35 +661,28 @@ class SvdEngine:
         self._als_refuse()
         u, i, w = self._merge_interactions(users, items, weights, self.U, "ials_data")
         dev = self.device
-        by = {}
-        for name, rows, cols, n_rows, n_cols in (("user", u, i, self.U, self.I), ("item", i, u, self.I, self.U)):
-            order = torch.argsort(rows * n_cols + cols, stable=True) if name == "item" else None
-            indptr = torch.zeros(n_rows + 1, dtype=torch.int64, device=dev)
-            indptr[1:] = torch.cumsum(torch.bincount(rows, minlength=n_rows), 0)
-            cols_s, w_s = (cols, w) if order is None else (cols[order], w[order])
-            by[name] = InteractionCSR(indptr, cols_s.to(torch.int32).contiguous(), w_s.contiguous())
-        chunk = int(self.L.tfr_als_chunk())
-        up, ip = self._als_plan(by["user"].indptr, chunk), self._als_plan(by["item"].indptr, chunk)
-        nbytes = max(check(self.L.tfr_ials_workspace_bytes(p.chunk_heavy.numel(), self.d)) for p in (up, ip))
-        nbytes = max(nbytes, check(self.L.tfr_gram_workspace_bytes(max(self.U, self.I), self.d)),
-                     check(self.L.tfr_ials_objective_workspace_bytes(self.U)))
+        by_user, by_item, up, ip, chunk, ws = self._plans(
+            u, i, w, InteractionCSR, self.L.tfr_ials_workspace_bytes,
+            check(self.L.tfr_gram_workspace_bytes(max(self.U, self.I), self.d)),
+            check(self.L.tfr_ials_objective_workspace_bytes(self.U)))
         n_tri = self.d * (self.d + 1) // 2
-        return IalsData(by["user"], by["item"], up, ip, chunk, torch.zeros(n_tri, dtype=torch.float64, device=dev),
-                        torch.zeros(n_tri, dtype=torch.float64, device=dev),
-                        torch.empty(nbytes, dtype=torch.uint8, device=dev), torch.zeros(1, dtype=torch.int32, device=dev),
-                        torch.zeros(5, dtype=torch.float64, device=dev))
+        return IalsData(by_user, by_item, up, ip, chunk, torch.zeros(n_tri, dtype=torch.float64, device=dev),
+                        torch.zeros(n_tri, dtype=torch.float64, device=dev), ws,
+                        torch.zeros(1, dtype=torch.int32, device=dev), torch.zeros(5, dtype=torch.float64, device=dev))
 
     def _gram(self, feat, n_rows, gram, ws):
         check(self.L.tfr_gram_rows(feat.data_ptr(), n_rows, self.d, self.feat_stride, gram.data_ptr(), ws.data_ptr(),
                                    ws.numel(), self._stream()))
 
     def _ials_half(self, data, alpha, reg, csr, plan, fixed, solved):
+        """tfr_ials_half_sweep of the rows of `plan` into the rows of `solved` (feat, bias or None), with data's chunk,
+        failed counter and workspace; row strides are the tensors' own."""
         (ff, n_fixed, gram), (of, ob) = fixed, solved
         check(self.L.tfr_ials_half_sweep(
-            ff.data_ptr(), n_fixed, self.d, self.feat_stride, gram.data_ptr(), alpha, reg, csr.indptr.data_ptr(),
+            ff.data_ptr(), n_fixed, self.d, ff.stride(0), gram.data_ptr(), alpha, reg, csr.indptr.data_ptr(),
             csr.partner.data_ptr(), csr.weight.data_ptr(), plan.light.data_ptr(), plan.light.numel(),
             plan.heavy.data_ptr(), plan.heavy_ptr.data_ptr(), plan.heavy.numel(), plan.chunk_heavy.data_ptr(),
-            plan.chunk_heavy.numel(), data.chunk, of.data_ptr(), self.feat_stride, ob.data_ptr() if ob is not None else None,
+            plan.chunk_heavy.numel(), data.chunk, of.data_ptr(), of.stride(0), ob.data_ptr() if ob is not None else None,
             data.failed.data_ptr(), data.workspace.data_ptr(), data.workspace.numel(), self._stream()))
 
     def ials_sweep(self, data, alpha, reg=None):
@@ -731,25 +737,22 @@ class SvdEngine:
             r_ = rows if isinstance(rows, torch.Tensor) else np.asarray(rows)
             n = int(r_.max()) + 1 if (r_.numel() if isinstance(r_, torch.Tensor) else r_.size) else 0
         n = int(n)
-        r, it, w = self._merge_interactions(rows, items, weights, n, "fold_in_implicit")
+        r, i, w = self._merge_interactions(rows, items, weights, n, "fold_in_implicit")
         dev = self.device
-        indptr = torch.zeros(n + 1, dtype=torch.int64, device=dev)
-        indptr[1:] = torch.cumsum(torch.bincount(r, minlength=n), 0)
-        it = it.to(torch.int32).contiguous()
+        csr = InteractionCSR(*csr_of(r, i, n, self.I, w))
+        none32 = torch.empty(0, dtype=torch.int32, device=dev)
+        plan = AlsPlan(torch.arange(n, dtype=torch.int32, device=dev), none32, torch.zeros(1, dtype=torch.int64, device=dev),
+                       none32)   # every row light: one CTA each, whatever its length
         feat = torch.full((n, self.d), float("nan"), dtype=torch.float32, device=dev)
         bias = torch.zeros(n, dtype=torch.float32, device=dev)
         gram = torch.empty(self.d * (self.d + 1) // 2, dtype=torch.float64, device=dev)
         ws = torch.empty(check(self.L.tfr_gram_workspace_bytes(self.I, self.d)), dtype=torch.uint8, device=dev)
-        failed = torch.zeros(1, dtype=torch.int32, device=dev)
-        rows_all = torch.arange(n, dtype=torch.int32, device=dev)
+        half = SimpleNamespace(chunk=1, failed=torch.zeros(1, dtype=torch.int32, device=dev), workspace=ws)
         with torch.cuda.device(dev):
             self._gram(self.t["item_feat"], self.I, gram, ws)
-            check(self.L.tfr_ials_half_sweep(
-                self.t["item_feat"].data_ptr(), self.I, self.d, self.feat_stride, gram.data_ptr(), alpha, reg,
-                indptr.data_ptr(), it.data_ptr(), w.data_ptr(), rows_all.data_ptr(), n, None, None, 0, None, 0, 1,
-                feat.data_ptr(), self.d, None, failed.data_ptr(), None, 0, self._stream()))
+            self._ials_half(half, alpha, reg, csr, plan, (self.t["item_feat"], self.I, gram), (feat, None))
         info = torch.isnan(feat[:, 0]).to(torch.int32) if n else torch.zeros(0, dtype=torch.int32, device=dev)
-        return FoldedUsers(feat, bias, PairCSR(indptr, it), info)
+        return FoldedUsers(feat, bias, PairCSR(csr.indptr, csr.partner), info)
 
     def _csr_by_user(self, users, items, rates=None, dedup=False, n_rows=None):
         """(user, item[, rate]) pairs -> CSR by user, item ids ascending inside a user: (indptr int64 [U + 1], items int32,
@@ -757,20 +760,11 @@ class SvdEngine:
         given, duplicates included, in a stable order.  n_rows: rows of the CSR (user ids in [0, n_rows)), default U."""
         self._check_ids(users, items, n_rows)
         n_rows = self.U if n_rows is None else n_rows
-        dev = self.device
         u, i = self._dev_i32(users).to(torch.int64), self._dev_i32(items).to(torch.int64)
-        rt = None
         if dedup:
             key = torch.unique(u * self.I + i)   # sorted
-            u, it = key // self.I, (key % self.I).to(torch.int32).contiguous()
-        else:
-            r = self._dev_f32(rates) if rates is not None else None
-            order = torch.argsort(u * self.I + i, stable=True)
-            it = i[order].to(torch.int32).contiguous()
-            rt = r[order].contiguous() if r is not None else None
-        indptr = torch.zeros(n_rows + 1, dtype=torch.int64, device=dev)
-        indptr[1:] = torch.cumsum(torch.bincount(u, minlength=n_rows), 0)
-        return indptr, it, rt
+            return csr_of(key // self.I, key % self.I, n_rows, self.I)
+        return csr_of(u, i, n_rows, self.I, self._dev_f32(rates) if rates is not None else None)
 
     def pair_csr(self, users, items):
         """The distinct (user, item) pairs as a PairCSR: build an exclusion set once, pass it to rank_all_users /
@@ -799,9 +793,7 @@ class SvdEngine:
             ex_key = ex_user * self.I + excl.items.to(torch.int64)   # sorted: CSR order
             pos = torch.searchsorted(ex_key, key).clamp_(max=ex_key.numel() - 1)
             key = key[ex_key[pos] != key]
-        rel_indptr = torch.zeros(self.U + 1, dtype=torch.int64, device=dev)
-        rel_indptr[1:] = torch.cumsum(torch.bincount(key // self.I, minlength=self.U), 0)
-        rel_item = (key % self.I).to(torch.int32).contiguous()
+        rel_indptr, rel_item, _ = csr_of(key // self.I, key % self.I, self.U, self.I)
         idx, _, n_unc = self._rank_excluding(k, n_cand, excl)
         s = self.ranking_sums(idx, PairCSR(rel_indptr, rel_item)).cpu().numpy()
         n = int(round(s[4]))

@@ -25,7 +25,7 @@ import torch.distributed as dist
 
 from . import _lib, sharding
 from ._lib import ABS_ITEM, LOSS_SIGMOID_CE, OPT_SGD, README_FLAGS, VAR_ALL, OptScalars, SvdTables, TfrError, check
-from .engine import FoldedUsers, PairCSR, SvdEngine
+from .engine import FoldedUsers, PairCSR, SvdEngine, check_lengths, csr_of
 
 
 class ShardedSvdEngine:
@@ -346,9 +346,8 @@ class ShardedSvdEngine:
         u, i = self._dev_i32(users).to(torch.int64), self._dev_i32(items).to(torch.int64)
         keep = i % self.world == self.rank
         key = torch.unique(u[keep] * self.I + i[keep])   # sorted
-        indptr = torch.zeros(self.U + 1, dtype=torch.int64, device=self.device)
-        indptr[1:] = torch.cumsum(torch.bincount(key // self.I, minlength=self.U), 0)
-        return PairCSR(indptr, (key % self.I).to(torch.int32).contiguous())
+        indptr, items, _ = csr_of(key // self.I, key % self.I, self.U, self.I)
+        return PairCSR(indptr, items)
 
     def serve_gather(self, q):
         """Phase 1 of rank_users: the query users' rows (q device int32, global ids) this rank owns; summed over the ranks
@@ -431,11 +430,9 @@ class ShardedSvdEngine:
         reg = e.hyper["reg"] if reg is None else float(reg)
         if not reg >= 0.0:
             raise TfrError("fold_in: reg must be >= 0, got %r" % reg)
-        sizes = [a.numel() if isinstance(a, torch.Tensor) else np.asarray(a).size for a in (rows, items, rates)]
-        if len(set(sizes)) != 1:
-            raise TfrError("fold_in: rows, items and rates differ in length: %s" % sizes)
+        size = check_lengths("fold_in", "rows, items and rates", rows, items, rates)
         if n is None:
-            n = int((rows if isinstance(rows, torch.Tensor) else np.asarray(rows)).max()) + 1 if sizes[0] else 0
+            n = int((rows if isinstance(rows, torch.Tensor) else np.asarray(rows)).max()) + 1 if size else 0
         n = int(n)
         indptr, it, rt = SvdEngine._csr_by_user(self, rows, items, rates, n_rows=n)   # checks ids against n and I
         ids, pos = torch.unique(it, return_inverse=True)   # sorted: positions keep the CSR's order

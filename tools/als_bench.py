@@ -30,6 +30,17 @@ from tf_recomm_b200.engine import SvdEngine  # noqa: E402
 from recommend_bench import FP64_DATASHEET, gpu_info, timed  # noqa: E402
 
 CHUNKS = (1024, 2048, 4096, 8192, 16384)
+# the half-sweep kernels are one template for ALS and iALS: their profiler names carry the form of the system
+FORMS = (("FiForm<true, false, true> >", "FiRatings>"), ("FiForm<false, true, false> >", "FiImplicit>"))
+
+
+def kernel_label(key):
+    """A profiler event's kernel name without its parameters: 'als_objective_rows_kernel',
+    'half_sweep_rows_kernel<FiRatings>', 'half_sweep_rows_kernel<FiImplicit>', ..."""
+    name = key.split("(")[0].replace("void ", "").replace("tfr::", "")
+    for form, label in FORMS:
+        name = name.replace(form, label)
+    return name
 
 
 def flops(counts, dim):
@@ -67,8 +78,8 @@ def kernel_times(eng, data, reg, reps=3):
                 fn()
             torch.cuda.synchronize()
         for ev in prof.key_averages():
-            if "als_" in ev.key:
-                name = ev.key.split("(")[0].replace("tfr::", "")
+            if "als_" in ev.key or "half_sweep_" in ev.key:
+                name = kernel_label(ev.key)
                 dt = getattr(ev, "device_time_total", None)
                 if dt is None:
                     dt = ev.cuda_time_total

@@ -27,6 +27,7 @@ import tf_recomm_b200  # noqa: E402,F401
 from tf_recomm_b200 import config, synthetic  # noqa: E402
 from tf_recomm_b200._lib import check  # noqa: E402
 from tf_recomm_b200.engine import SvdEngine  # noqa: E402
+from als_bench import kernel_label  # noqa: E402
 from recommend_bench import FP64_DATASHEET, gpu_info, timed  # noqa: E402
 
 K = 50
@@ -76,8 +77,8 @@ def kernel_times(fns, reps=3):
                 fns[label]()
             torch.cuda.synchronize()
         for ev in prof.key_averages():
-            if "gram_" in ev.key or "ials_" in ev.key:
-                name = ev.key.split("(")[0].replace("tfr::", "")
+            if "gram_" in ev.key or "ials_" in ev.key or "half_sweep_" in ev.key:
+                name = kernel_label(ev.key)
                 dt = getattr(ev, "device_time_total", None)
                 if dt is None:
                     dt = ev.cuda_time_total
