@@ -324,11 +324,12 @@ class SvdEngine:
         bi = torch.empty(self.U, dtype=torch.int32, device=dev) if want_best else None
         nbytes = check(self.L.tfr_allpairs_workspace_bytes(self.U, self.I, self.d, int(use_tensor_cores)))
         ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        item_feat, item_stride = self._scored_item_feat()
         with torch.cuda.device(dev):
-            check(self.L.tfr_allpairs(self.t["user_feat"].data_ptr(), self.t["item_feat"].data_ptr(),
+            check(self.L.tfr_allpairs(self.t["user_feat"].data_ptr(), item_feat.data_ptr(),
                                       self.t["user_bias"].data_ptr(), self.t["item_bias"].data_ptr(),
                                       self.t["mu"].data_ptr(), self.U, self.I, self.d, self.feat_stride,
-                                      self.feat_stride, int(use_tensor_cores),
+                                      item_stride, int(use_tensor_cores),
                                       scores.data_ptr() if want_scores else None, bs.data_ptr() if want_best else None,
                                       bi.data_ptr() if want_best else None, ws.data_ptr(), nbytes, self._stream()))
         return dict(scores=scores, best_score=bs, best_item=bi)
@@ -377,32 +378,30 @@ class SvdEngine:
     def rank_all_users(self, k=50, n_cand=None, exclude=None):
         """forward.py:47-61 for EVERY user in one sweep of the tcgen05 GEMM: -> (items [U, k] int32, scores [U, k]
         float64, n_uncertified).  Identical to ranking the float64 score matrix of als3.py:112 (score descending, lowest
-        item id on ties): tensor-core candidates, float64 rescore, certificate, exact fallback (tfr_allpairs_consume).
+        item id on ties): tensor-core candidates, float64 rescore, certificate, exact fallback
+        (tfr_allpairs_rank_excluding).
 
         exclude: items each user must not be recommended (usually the training pairs): a (users, items) pair of id arrays
         (host or device) or a PairCSR from pair_csr().  The ranking is then over each user's remaining items
-        (tfr_allpairs_rank_excluding); a user with fewer than k of them gets (-inf, -1) past the last one.  With exclude,
-        any dim <= 512 is accepted (dims the tensor cores cannot take rank every row exactly on CUDA cores), and an
-        engine whose model scores u.|v| (ABS_ITEM, the fork variant) is ranked by that score."""
-        if exclude is None:
-            k, n_cand, idx, val, n_unc, ws, nbytes = self._topk_setup(k, n_cand)
-            with torch.cuda.device(self.device):
-                check(self.L.tfr_allpairs_consume(self.t["user_feat"].data_ptr(), self.t["item_feat"].data_ptr(),
-                                                  self.t["user_bias"].data_ptr(), self.t["item_bias"].data_ptr(),
-                                                  self.t["mu"].data_ptr(), self.U, self.I, self.d, self.feat_stride,
-                                                  self.feat_stride, k, n_cand, val.data_ptr(), idx.data_ptr(),
-                                                  n_unc.data_ptr(), None, None, None, None, ws.data_ptr(), nbytes,
-                                                  self._stream()))
-            return idx, val, int(n_unc.item())
-        csr = exclude if isinstance(exclude, PairCSR) else self.pair_csr(*exclude)
+        (tfr_allpairs_rank_excluding); a user with fewer than k of them gets (-inf, -1) past the last one.  With or
+        without exclude, any dim <= 512 is accepted (dims the tensor cores cannot take rank every row exactly on CUDA
+        cores), and an engine whose model scores u.|v| (ABS_ITEM, the fork variant) is ranked by that score."""
+        csr = None
+        if exclude is not None:
+            csr = exclude if isinstance(exclude, PairCSR) else self.pair_csr(*exclude)
         return self._rank_excluding(k, n_cand, csr)
+
+    def _scored_item_feat(self):
+        """(item table, row stride) the all-pairs sweeps score against: item_feat, or under ABS_ITEM (the model's score is
+        u.|v|, ops.py:44) a contiguous copy of |item_feat|."""
+        if self.flags & ABS_ITEM:
+            return torch.abs(self.t["item_feat"]).contiguous(), 0
+        return self.t["item_feat"], self.feat_stride
 
     def _rank_excluding(self, k, n_cand, csr):
         """tfr_allpairs_rank_excluding; csr = None: nothing excluded."""
         k, n_cand, idx, val, n_unc, ws, nbytes = self._topk_setup(k, n_cand)
-        item_feat, item_stride = self.t["item_feat"], self.feat_stride
-        if self.flags & ABS_ITEM:   # the model's score is u.|v| (ops.py:44): rank on a copy of |item_feat|
-            item_feat, item_stride = torch.abs(item_feat).contiguous(), 0
+        item_feat, item_stride = self._scored_item_feat()
         with torch.cuda.device(self.device):
             check(self.L.tfr_allpairs_rank_excluding(
                 self.t["user_feat"].data_ptr(), item_feat.data_ptr(), self.t["user_bias"].data_ptr(),
@@ -823,11 +822,12 @@ class SvdEngine:
         dev = self.device
         indptr, it, rt = self._csr_by_user(users, items, rates)
         row_se = torch.empty(self.U, dtype=torch.float64, device=dev)
+        item_feat, item_stride = self._scored_item_feat()
         with torch.cuda.device(dev):
-            check(self.L.tfr_allpairs_consume(self.t["user_feat"].data_ptr(), self.t["item_feat"].data_ptr(),
+            check(self.L.tfr_allpairs_consume(self.t["user_feat"].data_ptr(), item_feat.data_ptr(),
                                               self.t["user_bias"].data_ptr(), self.t["item_bias"].data_ptr(),
                                               self.t["mu"].data_ptr(), self.U, self.I, self.d, self.feat_stride,
-                                              self.feat_stride, 0, 0, None, None, None, indptr.data_ptr(), it.data_ptr(),
+                                              item_stride, 0, 0, None, None, None, indptr.data_ptr(), it.data_ptr(),
                                               rt.data_ptr(), row_se.data_ptr(), None, 0, self._stream()))
         n = max(int(it.numel()), 1)
         return float(torch.sqrt(row_se.sum() / n)), row_se
